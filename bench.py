@@ -2,6 +2,7 @@
 """bench.py - Bellman backups/s of the sweep hot path (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload large|ar1|pv]
+                    [--dump-outputs DIR]
 
 A "step" is one full Bellman sweep (value_iteration's hot path) over the
 configured state grid.  Workload: BASELINE.json configs[4], the storage-AR1
@@ -30,6 +31,9 @@ oracle/_ref/py with its Cython routine compiled from its own source) on bounded 
 same workload, 1 core, and prints the same line (kind "reference"; the oracle port when the
 staged copy is absent).
 --workload pv: BASELINE configs[1], the time-dependent recursion (see run_pv).
+--dump-outputs DIR: after the timed steps, what the timed path computed in its last step is
+written as DIR/<name>.npy (float64), so that two builds can be compared output for output on
+the same seeded inputs (see write_outputs).
 """
 import argparse
 import json
@@ -40,6 +44,9 @@ import threading
 import time
 
 import numpy as np
+
+# the benchmark runs from a tree that may be read-only and leaves nothing in it
+sys.dont_write_bytecode = True
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
@@ -121,6 +128,32 @@ def workload_config(name, dims, W):
             "l2": "GPU arm: every sweep streams its shard of the tables once (4.3 GB on one GPU, "
                   "0.54 GB per GPU on eight; 126 MB of L2), so nothing is flushed between timed "
                   "sweeps; CPU arm: not applicable"}
+
+
+DUMP_LIMIT_BYTES = 60 * 10 ** 6        # under 64 MB in all, .npy headers included
+
+
+def write_outputs(out_dir, arrays, seed=0):
+    """--dump-outputs: each of `arrays` (name -> array) as out_dir/<name>.npy in float64.
+    Above DUMP_LIMIT_BYTES in all, every array keeps the same rows (leading axis) of one
+    sample seeded by `seed`, in ascending order."""
+    arrays = {k: np.asarray(a, dtype=np.float64) for k, a in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        n = len(next(iter(arrays.values())))
+        rows = np.sort(np.random.default_rng(seed).choice(
+            n, size=n * DUMP_LIMIT_BYTES // total, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+
+
+def last_sweep_results(eng, T, J_out):
+    """host (J, pol) of the last sweep over the tables T, whose J is the device array J_out:
+    one row per state in the grid's C order, as value_iteration returns them.  T holds that
+    sweep's argmin until the next sweep over T; K3 maps it to control values."""
+    return eng.to_host(J_out, eng.policy_values(T, eng.gather_argmin(T)))
 
 
 def make_problem(api, args, **solver_kw):
@@ -467,6 +500,13 @@ def run_ours(args):
 
     peak, peak_src = read_peaks()
     J_keep = J_prev.clone()
+    if args.dump_outputs:
+        # (before the e2e calls below sweep over T again)
+        J_last, pol_last = last_sweep_results(eng, T, J_keep)
+        if rank == 0:
+            write_outputs(args.dump_outputs, {"J": J_last.reshape(n_grid),
+                                              "pol": pol_last.reshape(n_grid, -1)})
+        del J_last, pol_last
 
     # end-to-end through the public API, host arrays in and out
     n_e2e = max(3, min(K, 10))
@@ -669,6 +709,8 @@ def run_pv(args):
         sweeps.append(info.get("sweeps_s", float("nan")))
         tabs.append(info.get("tabulate_s", float("nan")) + info.get("upload_build_s", float("nan")))
     launches = _cabi.launch_count() - launches0
+    if args.dump_outputs:
+        write_outputs(args.dump_outputs, {"J": J, "pol": pol})
     from oracle import build as ob
     ob.build()
     from oracle.ref_port import port_api
@@ -749,7 +791,13 @@ def main():
     ap.add_argument("--verify-states", dest="verify_states", type=int, default=1000,
                     help="states of the final sweep checked against the oracle port (0: skip)")
     ap.add_argument("--no-extra", action="store_true")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", metavar="DIR", default=None,
+                    help="write the timed path's results of its last step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm times samples of states, not whole results")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.cpu_sample is None:

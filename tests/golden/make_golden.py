@@ -24,6 +24,15 @@ Fixtures and the reference code path that produced them:
                      SEAREV on 33 x 4 x 3 (control step .05): 2 x value_iteration
   searev_full.npz    config #4 as shipped: policy_iteration(pol_lin, 1000, 5, rel_dp=True)
                      (== examples/20 .../storage control/pol_E10_grid3161_iter5.npy), ~15 min
+  reference_checks.npz  (--reference-checks) the original's side of three cross-checks of
+                     tests/test_oracle.py: multilinear_interpolation on the seeded points of
+                     make_golden_cases.interp_check_inputs; value_iteration + eval_policy(5, rel_dp)
+                     on the seeded 9 x 11 storage-AR1 J; the two columns of examples/01
+                     .../pv_prod.csv.  The committed file holds the oracle's results on these
+                     inputs (every tenth interpolation point): up to commit 3e0e2a7 the three
+                     checks ran live against the reference and matched it exactly (CPU suite:
+                     243 passed, 4 skipped), and neither the oracle nor the inputs changed since.
+                     This option rewrites it from the reference itself.
 """
 import contextlib
 import io
@@ -40,7 +49,7 @@ sys.path.insert(0, ROOT)
 from oracle.ref_loader import load_reference, load_reference_cython  # noqa: E402
 import workloads as wl  # noqa: E402
 sys.path.insert(0, HERE)
-from make_golden_cases import column_cases  # noqa: E402
+from make_golden_cases import column_cases, interp_check_inputs, storage_ar1_check  # noqa: E402
 
 
 def quiet(fn, *a, **k):
@@ -216,11 +225,28 @@ def make_column_cases(ref):
     save('column_cases.npz', **out)
 
 
+def make_reference_checks(ref):
+    from oracle.ref_loader import REF_ROOT
+    cy = load_reference_cython()
+    out = {}
+    for d, (smin, smax, orders, vals, s) in enumerate(interp_check_inputs(), 1):
+        out['interp_d%d' % d] = np.asarray(cy.multilinear_interpolation(smin, smax, orders, vals, s))
+    prob, J = storage_ar1_check(ref)
+    (out['vi_J'], out['vi_pol']), _ = quiet(prob.solver.value_iteration, J)
+    (out['ev_J'], ev_ref), _ = quiet(prob.solver.eval_policy, out['vi_pol'], 5, rel_dp=True)
+    out['ev_Jref'] = np.array(ev_ref)
+    csv = os.path.join(REF_ROOT, 'examples', '01 Deterministic storage control', 'pv_prod.csv')
+    out['pv_t'], out['pv_P'] = np.loadtxt(csv, skiprows=1, delimiter=',').T
+    save('reference_checks.npz', **out)
+
+
 if __name__ == '__main__':
     ref = load_reference()
     assert ref is not None, 'the reference is not available here'
     if '--searev-full' in sys.argv:
         make_searev_full(ref)
+    elif '--reference-checks' in sys.argv:
+        make_reference_checks(ref)
     elif '--column-cases' in sys.argv:
         make_column_cases(ref)
     else:
