@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define SDP_ABI_VERSION 8
+#define SDP_ABI_VERSION 9
 #define SDP_MAX_D 4 /* the reference dispatches d = 1..4 (multilinear_cython.pyx:36-47) */
 
 /* error codes */
@@ -409,6 +409,63 @@ int sdp_policy_eval_p2p(const SdpGrid* grid, int32_t W, int32_t g_per_w, const d
                         const double* J_in, const SdpPeers* peers, const int32_t* ref_cell,
                         const double* ref_lam, const double* ref_g, double* J_ref_out,
                         void* stream);
+
+/* K1'' - forward (adjoint) application of a fixed policy: propagation of a state distribution.
+ * New feature, no reference counterpart: the reference estimates what a policy does to the
+ * system by simulating one trajectory point at a time (examples/20 .../storage_control.py:217,246).
+ * The fixed-policy backup of sdp_policy_eval is J <- g_bar + P J with the interpolated Markov
+ * chain P of the policy tables (same [w][n] planes: cell, lam, g, p); these entry points apply
+ * the transpose, mu <- P^T mu:
+ *   (P^T mu)(y) = sum over (x, w, eps in {0,1}^d) with cell[w*n + x] + sum_k eps_k*M_k = y of
+ *                 mu(x) * coef(x, w, eps)
+ *   coef(x, w, eps) = p_w * f_0 * f_1 * ... * f_{d-1}, multiplied left to right,
+ *                     f_k = eps_k ? lam_k : (1 - lam_k),  lam_k = lam[k*lam_plane + w*n + x]
+ * (bit k of eps is the corner along axis k, M_k the C-order strides).  Weights are not clamped:
+ * outside the grid box the coefficients extrapolate and may be negative, exactly as the backup.
+ * The operator is stored as CSR by DESTINATION y, every (x, w, eps) kept (nnz = n*W*2^d, known up
+ * front; n*W*2^d < 2^31), entries of a row ordered by the source key (x*W + w)*2^d + eps, so the
+ * build is deterministic.  Rows longer than SDP_FWD_PIECE entries (extrapolated next states all
+ * land in the first or last cell) are cut into pieces of SDP_FWD_PIECE entries, summed
+ * separately and combined in piece order: every sum has a fixed association, independent of the
+ * launch shape, and there are no floating-point atomics - results are bit-identical run to run.
+ * All buffers are caller-owned device memory (the struct itself is a host pointer). */
+#define SDP_FWD_PIECE 1024
+typedef struct SdpForwardOp {
+    int64_t n;              /* states (the whole grid: one rank) */
+    int64_t nnz;            /* n * W * 2^d */
+    int64_t* row_ptr;       /* [n+1] entries of row y: row_ptr[y] .. row_ptr[y+1]-1 */
+    int32_t* src;           /* [nnz] source state x of each entry */
+    double* coef;           /* [nnz] coefficient of each entry */
+    double* gbar;           /* [n] expected stage cost g_bar(x) = sum_w p_w*g(x,w), summed in w order */
+    int64_t* piece_first;   /* [n+1] pieces of row y: piece_first[y] .. piece_first[y+1]-1 (none for short rows) */
+    int32_t* piece_row;     /* [max_pieces] row of each piece */
+    int64_t max_pieces;     /* from sdp_forward_sizes */
+    int64_t n_pieces;       /* piece_first[n]: read back by the caller after the build, used by the steps */
+} SdpForwardOp;
+
+/* Sizes of the buffers of a forward operator on a grid of n states, W nodes, d axes: nnz,
+ * max_pieces, the bytes of build scratch and the doubles of step scratch.  Needs the device
+ * current (the scratch of the library's sort is sized for it). */
+int sdp_forward_sizes(int32_t d, int32_t W, int64_t n, int64_t* nnz, int64_t* max_pieces,
+                      int64_t* build_scratch_bytes, int64_t* step_scratch_doubles);
+/* Build op (row_ptr, src, coef, gbar, piece_first, piece_row) from the policy tables of the
+ * whole grid, in the layout sdp_policy_eval takes (g_per_w as there).  Count per destination
+ * (integer atomics), exclusive scan, fill through per-row cursors, sort of every row by source
+ * key, coefficients; then the piece index of the long rows.  scratch: device, scratch_bytes >=
+ * build_scratch_bytes, 256-byte aligned; nothing of it is needed afterwards. */
+int sdp_forward_build(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p,
+                      const int32_t* cell, const double* lam, int64_t lam_plane, const double* g,
+                      const SdpForwardOp* op, void* scratch, int64_t scratch_bytes, void* stream);
+/* n_steps applications of P^T, ping-pong between mu_a (holds mu_0) and mu_b: step k reads mu_k
+ * and writes mu_{k+1}; on return mu_n is in mu_a if n_steps is even, mu_b if odd.
+ * cost_out: device [n_steps], cost_out[k] = <mu_k, g_bar> (expected stage cost of step k);
+ * resid_out: device [1] or NULL, sum_y |mu_n(y) - mu_{n-1}(y)| of the last step;
+ * hist: device [(n_steps+1)*n] or NULL, hist[k*n + y] = mu_k(y);
+ * scratch: device [step_scratch_doubles].  Launches per step: a piece pass (when n_pieces > 0),
+ * the row pass (a team of 8 lanes per row, 256 rows per CTA, per-CTA partial sums of the cost
+ * and the residual), a one-CTA reduction of those partials. */
+int sdp_forward_steps(const SdpForwardOp* op, double* mu_a, double* mu_b, int32_t n_steps,
+                      double* cost_out, double* resid_out, double* hist, double* scratch, void* stream);
 
 /* K3 - argmin index -> control values, the `u_grids[i].flatten()[ind_opt[i]]` of
  * stodynprog.py:686-689 for every state at once.  lo/hi: device [n][nc] box

@@ -12,7 +12,7 @@ import numpy as np
 
 SDP_MAX_D = 4
 SDP_MAX_C = 4
-SDP_ABI_VERSION = 8
+SDP_ABI_VERSION = 9
 LAYOUT_CONTROL_MINOR = 0   # "A": [state][w][u]
 LAYOUT_STATE_MINOR = 1     # "B": [tile of 32 states][u][w][lane]
 LAYOUT_CONTROL_MINOR_FACTORED = 2   # "AF": (x,u) part [state][Upad] + (x,w) part [state][W]
@@ -93,6 +93,23 @@ class SdpPeers(ctypes.Structure):
                 ("A", ctypes.c_void_p * SDP_MAX_PEERS)]
 
 
+class SdpForwardOp(ctypes.Structure):
+    """forward (adjoint) operator of a fixed policy: CSR by destination (sdp_forward_*)"""
+    _fields_ = [("n", ctypes.c_int64),
+                ("nnz", ctypes.c_int64),
+                ("row_ptr", ctypes.c_void_p),
+                ("src", ctypes.c_void_p),
+                ("coef", ctypes.c_void_p),
+                ("gbar", ctypes.c_void_p),
+                ("piece_first", ctypes.c_void_p),
+                ("piece_row", ctypes.c_void_p),
+                ("max_pieces", ctypes.c_int64),
+                ("n_pieces", ctypes.c_int64)]
+
+
+FWD_PIECE = 1024   # SDP_FWD_PIECE: entries per piece of a long row of the forward operator
+
+
 # numpy mirrors of the per-state descriptor and the work item (host-built arrays
 # uploaded verbatim; layouts must match the C structs, checked by the tests)
 STATE_DESC_DTYPE = np.dtype([("entry_off", np.int64),
@@ -150,6 +167,11 @@ SIGNATURES = {
                                        _vp, _vp, _i32, _i32, _i64, _vp, _vp]),
     "sdp_policy_eval_p2p": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64,
                                            _vp, ctypes.POINTER(SdpPeers), _vp, _vp, _vp, _vp, _vp]),
+    "sdp_forward_sizes": (ctypes.c_int, [_i32, _i32, _i64, _vp, _vp, _vp, _vp]),
+    "sdp_forward_build": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _vp, _i64, _vp,
+                                         ctypes.POINTER(SdpForwardOp), _vp, _i64, _vp]),
+    "sdp_forward_steps": (ctypes.c_int, [ctypes.POINTER(SdpForwardOp), _vp, _vp, _i32, _vp, _vp, _vp, _vp,
+                                         _vp]),
     "sdp_policy_values": (ctypes.c_int, [_i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sdp_sweep_finalize_cols": (ctypes.c_int, [ctypes.POINTER(SdpTables), _vp, _vp, _vp, _vp, _i64, _i64,
                                                _i32, _vp, _vp, _vp, _vp, _i32, _vp]),

@@ -6,6 +6,8 @@
 //   * the per-state backup _value_at_state_vect (stodynprog/stodynprog.py:639-691)
 //     looped over the state grid by value_iteration (:511-515)
 //   * the policy-evaluation iteration of eval_policy (:743-763)
+// and adds the forward (transposed) application of a fixed policy's chain, which the
+// reference has no counterpart for (K1'', distribution propagation).
 //
 // This is a gather-reduce, not a contraction: no tensor cores.  The sweep kernel
 // streams the dense (cell, lambda, g) tables once from HBM with 128-bit
@@ -31,6 +33,9 @@
 #include <limits.h>
 #include <math.h>
 #include <atomic>
+
+#include <cub/device/device_scan.cuh>
+#include <cub/device/device_segmented_sort.cuh>
 
 #include "sdp_b200.h"
 
@@ -3375,6 +3380,350 @@ extern "C" int sdp_policy_eval_p2p(const SdpGrid* grid, int32_t W, int32_t g_per
         }
     }
     SDP_LAUNCH_CHECK();
+    return SDP_OK;
+}
+
+// ---------------------------------------------------------------------------
+// K1'': forward (adjoint) operator of a fixed policy, mu <- P^T mu (include/sdp_b200.h).
+// New feature: the reference only simulates trajectories (storage_control.py:217,246).
+// Build: CSR by destination from the [w][n] policy-table planes of K1'.  Steps: a gather, one
+// warp per destination row; no floating-point atomics, every sum in a fixed association.
+// ---------------------------------------------------------------------------
+#define SDP_FWD_ROWS_PER_CTA 256   // one tile of the cost / residual partial sums
+
+static inline int64_t align256(int64_t b) { return (b + 255) & ~(int64_t)255; }
+
+// destination of corner eps of base cell b: bit k of eps is the corner along axis k
+__device__ __forceinline__ int fwd_dest(const GridT<double>& G, int d, int b, int eps) {
+    int y = b;
+#pragma unroll
+    for (int k = 0; k < SDP_MAX_D; ++k)
+        if (k < d && ((eps >> k) & 1)) y += G.stride[k];
+    return y;
+}
+
+// one thread per (x, w) table entry e = w*n + x: count the 2^d destinations
+__global__ void __launch_bounds__(256)
+k_fwd_count(GridT<double> G, int d, int64_t nw, const int32_t* __restrict__ cell, int32_t* __restrict__ counts) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= nw) return;
+    const int b = cell[e];
+    for (int eps = 0; eps < (1 << d); ++eps) atomicAdd(counts + fwd_dest(G, d, b, eps), 1);
+}
+
+// same walk: every entry lands at row_ptr[y] + (a cursor of row y) with its source key
+// (x*W + w)*2^d + eps; the order inside a row is fixed afterwards by sorting the keys
+__global__ void __launch_bounds__(256)
+k_fwd_fill(GridT<double> G, int d, int W, int64_t n, const int32_t* __restrict__ cell,
+           const int64_t* __restrict__ row_ptr, int32_t* __restrict__ cursor, int32_t* __restrict__ keys) {
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n * W) return;
+    const int64_t w = e / n, x = e - w * n;
+    const int b = cell[e];
+    const int key0 = (int)((x * W + w) << d);
+    for (int eps = 0; eps < (1 << d); ++eps) {
+        const int y = fwd_dest(G, d, b, eps);
+        keys[row_ptr[y] + atomicAdd(cursor + y, 1)] = key0 + eps;
+    }
+}
+
+// key -> (source state, coefficient p_w * f_0 * ... * f_{d-1}, left to right); in place on src
+__global__ void __launch_bounds__(256)
+k_fwd_coef(int d, int W, int64_t n, int64_t nnz, const double* __restrict__ p, const double* __restrict__ lam,
+           int64_t lam_plane, int32_t* __restrict__ src, double* __restrict__ coef) {
+    const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (j >= nnz) return;
+    const int key = src[j];
+    const int eps = key & ((1 << d) - 1);
+    const int xw = key >> d;
+    const int x = xw / W, w = xw - x * W;
+    const int64_t e = (int64_t)w * n + x;
+    double c = p[w];
+#pragma unroll
+    for (int k = 0; k < SDP_MAX_D; ++k) {
+        if (k < d) {
+            const double l = lam[(int64_t)k * lam_plane + e];
+            c = mul_(c, ((eps >> k) & 1) ? l : sub_(1.0, l));
+        }
+    }
+    src[j] = x;
+    coef[j] = c;
+}
+
+// g_bar(x) = sum_w p_w * g(x, w), accumulated in w order from 0
+__global__ void __launch_bounds__(256)
+k_fwd_gbar(int W, int g_per_w, int64_t n, const double* __restrict__ p, const double* __restrict__ g,
+           double* __restrict__ gbar) {
+    const int64_t x = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (x >= n) return;
+    double acc = 0.0;
+    for (int w = 0; w < W; ++w) acc = add_(acc, mul_(p[w], g[g_per_w ? (int64_t)w * n + x : x]));
+    gbar[x] = acc;
+}
+
+// pieces per row: ceil(len / SDP_FWD_PIECE) for rows longer than one piece, 0 otherwise
+__global__ void __launch_bounds__(256)
+k_fwd_piece_count(int64_t n, const int64_t* __restrict__ row_ptr, int32_t* __restrict__ counts) {
+    const int64_t y = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (y > n) return;
+    if (y == n) { counts[n] = 0; return; }
+    const int64_t len = row_ptr[y + 1] - row_ptr[y];
+    counts[y] = len > SDP_FWD_PIECE ? (int32_t)((len + SDP_FWD_PIECE - 1) / SDP_FWD_PIECE) : 0;
+}
+
+__global__ void __launch_bounds__(256)
+k_fwd_piece_fill(int64_t n, const int64_t* __restrict__ piece_first, int32_t* __restrict__ piece_row) {
+    const int64_t y = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (y >= n) return;
+    for (int64_t q = piece_first[y]; q < piece_first[y + 1]; ++q) piece_row[q] = (int32_t)y;
+}
+
+// sum of coef[e] * mu[src[e]] over [begin, end) by a team of TEAM lanes: lane-strided in index
+// order, then a butterfly inside the team (every lane of the team ends with the same bits: IEEE
+// addition is commutative).  TEAM is a constant of the operator, not of the launch.
+template <int TEAM>
+__device__ __forceinline__ double fwd_segment(const int32_t* __restrict__ src, const double* __restrict__ coef,
+                                              const double* __restrict__ mu, int64_t begin, int64_t end,
+                                              int tl) {
+    double acc = 0.0;
+#pragma unroll 4
+    for (int64_t e = begin + tl; e < end; e += TEAM)
+        acc = add_(acc, mul_(__ldcs(coef + e), __ldg(mu + __ldcs(src + e))));
+#pragma unroll
+    for (int o = TEAM / 2; o >= 1; o >>= 1) acc = add_(acc, __shfl_xor_sync(0xffffffffu, acc, o));
+    return acc;
+}
+
+// one warp per piece of a long row
+__global__ void __launch_bounds__(256)
+k_fwd_pieces(const int64_t* __restrict__ row_ptr, const int32_t* __restrict__ src, const double* __restrict__ coef,
+             const int64_t* __restrict__ piece_first, const int32_t* __restrict__ piece_row, int64_t n_pieces,
+             const double* __restrict__ mu, double* __restrict__ piece_val) {
+    const int lane = threadIdx.x & 31;
+    const int64_t q = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    if (q >= n_pieces) return;
+    const int y = piece_row[q];
+    const int64_t begin = row_ptr[y] + (q - piece_first[y]) * SDP_FWD_PIECE;
+    const int64_t end = min(begin + SDP_FWD_PIECE, row_ptr[y + 1]);
+    const double v = fwd_segment<32>(src, coef, mu, begin, end, lane);
+    if (lane == 0) piece_val[q] = v;
+}
+
+// the row pass: CTA t owns rows [256t, 256t+256), warp i rows 256t + 32i + j, j = 0..31.  The
+// warp loads the bounds of its 32 rows once (lane j: row j), then sums them SDP_FWD_TEAMS rows at
+// a time, a team of 32/SDP_FWD_TEAMS lanes per row (rows hold n*W*2^d/n entries on average: 36 for
+// W = 9, d = 2), so that several rows' loads are in flight per warp.  Lane j collects row j's value,
+// stores it (coalesced) and forms the cost / residual terms of its row; partials of the tile:
+// part[t] = sum mu_in*g_bar, part[n_tiles + t] = sum |mu_out - mu_in|
+#define SDP_FWD_TEAMS 4
+__global__ void __launch_bounds__(SDP_FWD_ROWS_PER_CTA)
+k_fwd_rows(int64_t n, const int64_t* __restrict__ row_ptr, const int32_t* __restrict__ src,
+           const double* __restrict__ coef, const int64_t* __restrict__ piece_first,
+           const double* __restrict__ piece_val, const double* __restrict__ gbar,
+           const double* __restrict__ mu_in, double* __restrict__ mu_out, double* __restrict__ hist_out,
+           double* __restrict__ part, int64_t n_tiles) {
+    constexpr int TEAM = 32 / SDP_FWD_TEAMS;
+    __shared__ double sh[2][SDP_FWD_ROWS_PER_CTA / 32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int team = lane / TEAM, tl = lane % TEAM;
+    const int64_t base = (int64_t)blockIdx.x * SDP_FWD_ROWS_PER_CTA + warp * 32;
+    const int64_t y = base + lane;
+    int64_t r0 = 0, r1 = 0, q0 = 0, q1 = 0;
+    if (y < n) { r0 = row_ptr[y]; r1 = row_ptr[y + 1]; q0 = piece_first[y]; q1 = piece_first[y + 1]; }
+    double mine = 0.0;
+#pragma unroll 1
+    for (int j0 = 0; j0 < 32; j0 += SDP_FWD_TEAMS) {
+        const int j = j0 + team;
+        const int64_t b = __shfl_sync(0xffffffffu, r0, j), e = __shfl_sync(0xffffffffu, r1, j);
+        const int64_t p0 = __shfl_sync(0xffffffffu, q0, j), p1 = __shfl_sync(0xffffffffu, q1, j);
+        double v;
+        if (p0 == p1) {
+            v = fwd_segment<TEAM>(src, coef, mu_in, b, e, tl);          // empty beyond n: b == e == 0
+        } else {
+            double acc = 0.0;                 // pieces of a long row, in piece order
+            for (int64_t q = p0 + tl; q < p1; q += TEAM) acc = add_(acc, piece_val[q]);
+#pragma unroll
+            for (int o = TEAM / 2; o >= 1; o >>= 1) acc = add_(acc, __shfl_xor_sync(0xffffffffu, acc, o));
+            v = acc;
+        }
+        const double got = __shfl_sync(0xffffffffu, v, ((lane - j0) & (SDP_FWD_TEAMS - 1)) * TEAM);
+        if (lane >= j0 && lane < j0 + SDP_FWD_TEAMS) mine = got;
+    }
+    double c = 0.0, r = 0.0;
+    if (y < n) {
+        mu_out[y] = mine;
+        if (hist_out) hist_out[y] = mine;
+        const double m = mu_in[y];
+        c = mul_(m, gbar[y]);
+        r = fabs(sub_(mine, m));
+    }
+#pragma unroll
+    for (int o = 16; o >= 1; o >>= 1) {
+        c = add_(c, __shfl_xor_sync(0xffffffffu, c, o));
+        r = add_(r, __shfl_xor_sync(0xffffffffu, r, o));
+    }
+    if (lane == 0) { sh[0][warp] = c; sh[1][warp] = r; }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        double cs = 0.0, rs = 0.0;
+        for (int i = 0; i < SDP_FWD_ROWS_PER_CTA / 32; ++i) { cs = add_(cs, sh[0][i]); rs = add_(rs, sh[1][i]); }
+        part[blockIdx.x] = cs;
+        part[n_tiles + blockIdx.x] = rs;
+    }
+}
+
+// one CTA: thread t sums the tiles t, t+256, ... in order, then a fixed tree over the threads
+__global__ void __launch_bounds__(256)
+k_fwd_reduce(const double* __restrict__ part, int64_t n_tiles, double* __restrict__ cost_out,
+             double* __restrict__ resid_out) {
+    __shared__ double sc[256], sr[256];
+    double c = 0.0, r = 0.0;
+    for (int64_t t = threadIdx.x; t < n_tiles; t += 256) {
+        c = add_(c, part[t]);
+        r = add_(r, part[n_tiles + t]);
+    }
+    sc[threadIdx.x] = c;
+    sr[threadIdx.x] = r;
+    __syncthreads();
+    for (int s = 128; s >= 1; s >>= 1) {
+        if (threadIdx.x < s) {
+            sc[threadIdx.x] = add_(sc[threadIdx.x], sc[threadIdx.x + s]);
+            sr[threadIdx.x] = add_(sr[threadIdx.x], sr[threadIdx.x + s]);
+        }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        cost_out[0] = sc[0];
+        if (resid_out) resid_out[0] = sr[0];
+    }
+}
+
+// byte offsets inside the build scratch: counts / cursors int32 [n+1], keys int32 [nnz], cub's
+// temporary storage (the larger of the scans' and the segmented sort's)
+struct FwdScratch {
+    int64_t keys_off, temp_off, temp_bytes, total;
+};
+
+static int fwd_sizes(int d, int W, int64_t n, int64_t* nnz, FwdScratch* S) {
+    if (d < 1 || d > SDP_MAX_D || W < 1 || n < 1) return fail(SDP_EINVAL, "%s", "sdp_forward: bad sizes");
+    const int64_t z = n * (int64_t)W << d;
+    if (z >= (int64_t)INT_MAX || n >= (int64_t)INT_MAX)
+        return fail(SDP_EINVAL, "%s", "sdp_forward: n*W*2^d must stay below 2^31");
+    size_t scan_b = 0, sort_b = 0;
+    SDP_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(nullptr, scan_b, (const int32_t*)nullptr, (int64_t*)nullptr,
+                                                 (int)(n + 1)));
+    SDP_CUDA_CHECK(cub::DeviceSegmentedSort::SortKeys(nullptr, sort_b, (const int32_t*)nullptr, (int32_t*)nullptr,
+                                                      z, n, (const int64_t*)nullptr, (const int64_t*)nullptr));
+    *nnz = z;
+    S->keys_off = align256(4 * (n + 1));
+    S->temp_off = S->keys_off + align256(4 * z);
+    S->temp_bytes = (int64_t)(scan_b > sort_b ? scan_b : sort_b);
+    S->total = S->temp_off + align256(S->temp_bytes);
+    return SDP_OK;
+}
+
+static int64_t fwd_max_pieces(int64_t nnz) { return 2 * (nnz / SDP_FWD_PIECE) + 1; }
+
+extern "C" int sdp_forward_sizes(int32_t d, int32_t W, int64_t n, int64_t* nnz, int64_t* max_pieces,
+                                 int64_t* build_scratch_bytes, int64_t* step_scratch_doubles) {
+    if (!nnz || !max_pieces || !build_scratch_bytes || !step_scratch_doubles)
+        return fail(SDP_EINVAL, "%s", "sdp_forward_sizes: NULL pointer");
+    FwdScratch S;
+    int rc = fwd_sizes(d, W, n, nnz, &S);
+    if (rc) return rc;
+    *max_pieces = fwd_max_pieces(*nnz);
+    *build_scratch_bytes = S.total;
+    *step_scratch_doubles = *max_pieces + 2 * ((n + SDP_FWD_ROWS_PER_CTA - 1) / SDP_FWD_ROWS_PER_CTA);
+    return SDP_OK;
+}
+
+extern "C" int sdp_forward_build(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p,
+                                 const int32_t* cell, const double* lam, int64_t lam_plane, const double* g,
+                                 const SdpForwardOp* op, void* scratch, int64_t scratch_bytes, void* stream) {
+    GridT<double> G;
+    int64_t ng = 0;
+    int rc = make_grid<double>(grid, &G, &ng);
+    if (rc) return rc;
+    if (!op) return fail(SDP_EINVAL, "%s", "sdp_forward_build: NULL op");
+    const int d = grid->d;
+    const int64_t n = op->n;
+    int64_t nnz = 0;
+    FwdScratch S;
+    if (n != ng) return fail(SDP_EINVAL, "%s", "sdp_forward_build: op->n is not the grid size");
+    rc = fwd_sizes(d, W, n, &nnz, &S);
+    if (rc) return rc;
+    if (op->nnz != nnz || op->max_pieces < fwd_max_pieces(nnz) || lam_plane < W * n || scratch_bytes < S.total)
+        return fail(SDP_EINVAL, "%s", "sdp_forward_build: buffer sizes do not match sdp_forward_sizes");
+    if (!p || !cell || !lam || !g || !scratch || !op->row_ptr || !op->src || !op->coef || !op->gbar ||
+        !op->piece_first || !op->piece_row)
+        return fail(SDP_EINVAL, "%s", "sdp_forward_build: NULL pointer");
+    if (((uintptr_t)scratch) & 255) return fail(SDP_EINVAL, "%s", "sdp_forward_build: scratch not 256-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    char* sb = (char*)scratch;
+    int32_t* counts = (int32_t*)sb;
+    int32_t* keys = (int32_t*)(sb + S.keys_off);
+    void* temp = sb + S.temp_off;
+    size_t temp_bytes = (size_t)S.temp_bytes;
+    const int64_t nw = n * W;
+    const unsigned bw = (unsigned)((nw + 255) / 256);
+    SDP_CUDA_CHECK(cudaMemsetAsync(counts, 0, 4 * (n + 1), st));
+    k_fwd_count<<<bw, 256, 0, st>>>(G, d, nw, cell, counts);
+    SDP_LAUNCH_CHECK();
+    SDP_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, (const int32_t*)counts, op->row_ptr,
+                                                 (int)(n + 1), st));
+    SDP_CUDA_CHECK(cudaMemsetAsync(counts, 0, 4 * (n + 1), st));
+    k_fwd_fill<<<bw, 256, 0, st>>>(G, d, W, n, cell, op->row_ptr, counts, keys);
+    SDP_LAUNCH_CHECK();
+    temp_bytes = (size_t)S.temp_bytes;
+    SDP_CUDA_CHECK(cub::DeviceSegmentedSort::SortKeys(temp, temp_bytes, (const int32_t*)keys, op->src, nnz, n,
+                                                      (const int64_t*)op->row_ptr, (const int64_t*)op->row_ptr + 1, st));
+    k_fwd_coef<<<(unsigned)((nnz + 255) / 256), 256, 0, st>>>(d, W, n, nnz, p, lam, lam_plane, op->src, op->coef);
+    SDP_LAUNCH_CHECK();
+    const unsigned bn = (unsigned)((n + 256) / 256);
+    k_fwd_gbar<<<bn, 256, 0, st>>>(W, g_per_w, n, p, g, op->gbar);
+    SDP_LAUNCH_CHECK();
+    k_fwd_piece_count<<<bn, 256, 0, st>>>(n, op->row_ptr, counts);
+    SDP_LAUNCH_CHECK();
+    temp_bytes = (size_t)S.temp_bytes;
+    SDP_CUDA_CHECK(cub::DeviceScan::ExclusiveSum(temp, temp_bytes, (const int32_t*)counts, op->piece_first,
+                                                 (int)(n + 1), st));
+    k_fwd_piece_fill<<<bn, 256, 0, st>>>(n, op->piece_first, op->piece_row);
+    SDP_LAUNCH_CHECK();
+    return SDP_OK;
+}
+
+extern "C" int sdp_forward_steps(const SdpForwardOp* op, double* mu_a, double* mu_b, int32_t n_steps,
+                                 double* cost_out, double* resid_out, double* hist, double* scratch,
+                                 void* stream) {
+    if (!op || n_steps < 0 || op->n < 1 || op->n_pieces < 0 || op->n_pieces > op->max_pieces)
+        return fail(SDP_EINVAL, "%s", "sdp_forward_steps: bad sizes");
+    if (!mu_a || !mu_b || (n_steps > 0 && (!cost_out || !scratch || !op->row_ptr || !op->src || !op->coef ||
+                                           !op->gbar || !op->piece_first || (op->n_pieces && !op->piece_row))))
+        return fail(SDP_EINVAL, "%s", "sdp_forward_steps: NULL pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int64_t n = op->n;
+    if (hist) SDP_CUDA_CHECK(cudaMemcpyAsync(hist, mu_a, 8 * n, cudaMemcpyDeviceToDevice, st));
+    const int64_t n_tiles = (n + SDP_FWD_ROWS_PER_CTA - 1) / SDP_FWD_ROWS_PER_CTA;
+    double* piece_val = scratch;
+    double* part = scratch + op->max_pieces;
+    const double* in = mu_a;
+    double* out = mu_b;
+    for (int k = 0; k < n_steps; ++k) {
+        if (op->n_pieces > 0) {
+            k_fwd_pieces<<<(unsigned)((op->n_pieces + 7) / 8), 256, 0, st>>>(
+                op->row_ptr, op->src, op->coef, op->piece_first, op->piece_row, op->n_pieces, in, piece_val);
+            SDP_LAUNCH_CHECK();
+        }
+        k_fwd_rows<<<(unsigned)n_tiles, SDP_FWD_ROWS_PER_CTA, 0, st>>>(
+            n, op->row_ptr, op->src, op->coef, op->piece_first, piece_val, op->gbar, in, out,
+            hist ? hist + (int64_t)(k + 1) * n : nullptr, part, n_tiles);
+        SDP_LAUNCH_CHECK();
+        k_fwd_reduce<<<1, 256, 0, st>>>(part, n_tiles, cost_out + k, k + 1 == n_steps ? resid_out : nullptr);
+        SDP_LAUNCH_CHECK();
+        const double* t = in;
+        in = out;
+        out = const_cast<double*>(t);
+    }
     return SDP_OK;
 }
 

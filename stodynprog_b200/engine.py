@@ -1386,11 +1386,15 @@ class Engine(object):
                 "instants": n_T, "tables": T}
 
     # -- policy tables ----------------------------------------------------
-    def build_policy_tables(self, solver, pol):
+    def build_policy_tables(self, solver, pol, t_k=None, deterministic=False):
         """Evaluate dyn/cost for the fixed policy on the whole grid exactly as
         eval_policy does (one broadcast call, stodynprog.py:731-755), expand on the
         host to dense [d][W][N] coordinates and run the cell search (K0a) for this
-        rank's equal-count slab."""
+        rank's equal-count slab.
+
+        t_k: the instant, passed first to dyn/cost (as bellman_recursion does).
+        deterministic: accept a system without perturbation (W = 1, p = [1]); eval_policy
+        leaves it False and raises IndexError there, like the reference (:726)."""
         torch = _torch()
         sys = solver.sys
         state_grid_1d = [np.asarray(g, dtype=float) for g in solver.state_grid]
@@ -1399,17 +1403,22 @@ class Engine(object):
         nb_control = len(sys.control)
         grid = _cabi.make_grid(state_grid_1d)
         n_grid = int(np.prod(state_dims))
-        solver.perturb_grid[0]                        # IndexError if deterministic, like :726
+        if not deterministic:
+            solver.perturb_grid[0]                    # IndexError if deterministic, like :726
         w_args, w_shape, W = tb.perturb_layout(solver.perturb_grid)
         w_proba = tb.joint_proba(solver.perturb_proba)
         n_w_axes = len(w_shape)
         state_grid = tuple(np.reshape(g, (1,) * i + (-1,) + (1,) * (nb_state - 1 - i + n_w_axes))
                            for i, g in enumerate(solver.state_grid))
         u_k = [pol[..., i].reshape(state_dims + (1,) * n_w_axes) for i in range(nb_control)]
-        args = state_grid + tuple(u_k) + w_args
+        args = ((t_k,) if t_k is not None else ()) + state_grid + tuple(u_k) + w_args
         x_next = sys.dyn(*args, **sys.params)
         g_k = sys.cost(*args, **sys.params)
-        if n_w_axes > 1:
+        if n_w_axes == 0:
+            # no perturbation: outputs broadcast to the state grid; one node of probability 1
+            x_next = tuple(self._as_full(c, state_dims)[..., None] for c in x_next)
+            g_k = self._as_full(g_k, state_dims)[..., None]
+        elif n_w_axes > 1:
             # one trailing axis: the C-order flattened product of the perturbation axes
             x_next = tuple(tb._fold_w(self._as_full(c, state_dims + w_shape), nb_state, w_shape, "dyn")
                            for c in x_next)
@@ -1527,6 +1536,77 @@ class Engine(object):
                 _cabi.check(rc, "sdp_rel_shift")
             cur, nxt = nxt, cur
         return cur
+
+    # -- forward operator (distribution propagation) ----------------------
+    def build_forward(self, P):
+        """The transposed operator mu <- P^T mu of the policy tables `P` (sdp_forward_build):
+        CSR by destination, g_bar, piece index of the long rows.  One rank only."""
+        torch = _torch()
+        if self.coll.world > 1 or P.n_states != int(np.prod(P.grid.order[:P.grid.d])):
+            raise NotImplementedError(
+                "distribution propagation runs on one rank: the transposed operator of a slab needs "
+                "the sources of the other slabs (not implemented)")
+        n = P.n_states
+        nnz, max_pieces, build_b, step_d = (ctypes.c_int64(), ctypes.c_int64(), ctypes.c_int64(),
+                                            ctypes.c_int64())
+        rc = self.lib.sdp_forward_sizes(P.grid.d, P.W, n, ctypes.byref(nnz), ctypes.byref(max_pieces),
+                                        ctypes.byref(build_b), ctypes.byref(step_d))
+        _cabi.check(rc, "sdp_forward_sizes")
+        F = _cabi.SdpForwardOp()
+        F.n, F.nnz, F.max_pieces = n, nnz.value, max_pieces.value
+        dev = self.device
+        bufs = {"row_ptr": torch.empty(n + 1, dtype=torch.int64, device=dev),
+                "src": torch.empty(nnz.value, dtype=torch.int32, device=dev),
+                "coef": torch.empty(nnz.value, dtype=torch.float64, device=dev),
+                "gbar": torch.empty(n, dtype=torch.float64, device=dev),
+                "piece_first": torch.empty(n + 1, dtype=torch.int64, device=dev),
+                "piece_row": torch.empty(max_pieces.value, dtype=torch.int32, device=dev)}
+        for name, t in bufs.items():
+            setattr(F, name, t.data_ptr())
+        # torch's caching allocator hands out 512-byte aligned blocks
+        scratch = torch.empty(build_b.value, dtype=torch.uint8, device=dev)
+        rc = self.lib.sdp_forward_build(ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.p), self._ptr(P.cell),
+                                        self._ptr(P.lam), P.lam_plane, self._ptr(P.g), ctypes.byref(F),
+                                        self._ptr(scratch), build_b.value, self.stream)
+        _cabi.check(rc, "sdp_forward_build")
+        F.n_pieces = int(bufs["piece_first"][n].item())      # sizes the piece pass of every step
+        del scratch
+        F.bufs = bufs
+        F.step_scratch = torch.empty(step_d.value, dtype=torch.float64, device=dev)
+        return F
+
+    def forward_steps(self, F, mu_a, mu_b, n_steps, cost_out, resid_out=None, hist=None):
+        """n_steps applications of P^T, ping-pong between mu_a (mu_0) and mu_b (device fp64 [n]);
+        cost_out[k] = <mu_k, g_bar>, resid_out[0] = sum |mu_n - mu_{n-1}|, hist[k] = mu_k
+        (device [(n_steps+1)*n]) when given.  Returns the tensor holding mu_n."""
+        rc = self.lib.sdp_forward_steps(ctypes.byref(F), self._ptr(mu_a), self._ptr(mu_b), int(n_steps),
+                                        self._ptr(cost_out), self._ptr(resid_out), self._ptr(hist),
+                                        self._ptr(F.step_scratch), self.stream)
+        _cabi.check(rc, "sdp_forward_steps")
+        return mu_a if n_steps % 2 == 0 else mu_b
+
+    def stationary(self, F, mu0, tol, max_iter, check_every):
+        """Power iteration mu <- P^T mu from the host array mu0: launches of `check_every` steps
+        (fewer for the last), one residual read back after each.  Returns (pi device tensor,
+        steps done, residuals, converged)."""
+        torch = _torch()
+        mu_a = self.to_device(np.ascontiguousarray(mu0, dtype=np.float64).reshape(-1))
+        mu_b = torch.empty_like(mu_a)
+        cost = torch.empty(max(check_every, 1), dtype=torch.float64, device=self.device)
+        resid = torch.zeros(1, dtype=torch.float64, device=self.device)
+        residuals, done, converged = [], 0, False
+        while done < max_iter:
+            k = min(check_every, max_iter - done)
+            mu_n = self.forward_steps(F, mu_a, mu_b, k, cost, resid)
+            if mu_n is mu_b:
+                mu_a, mu_b = mu_b, mu_a
+            done += k
+            r = float(resid.cpu().numpy()[0])
+            residuals.append(r)
+            if r <= tol:
+                converged = True
+                break
+        return mu_a, done, residuals, converged
 
     # -- interpolation ----------------------------------------------------
     def interp(self, grid, values, s):

@@ -548,6 +548,135 @@ class DPSolver(object):
         return J, pol, info
 
     # ------------------------------------------------------------------
+    # new: what a policy does to the system (forward / adjoint application)
+    # ------------------------------------------------------------------
+    @staticmethod
+    def _check_shape(name, A, expect_shape):
+        # same wording as interp_on_state (reference :413-415)
+        if A.shape != expect_shape:
+            raise ValueError('array `{:s}` should be of shape {:s}, not {:s}'.format(
+                name, str(expect_shape), str(A.shape)))
+
+    def _check_mu0(self, mu0):
+        mu0 = np.array(mu0, dtype=float)      # a copy: the caller's array is never written
+        self._check_shape('mu0', mu0, self._state_grid_shape)
+        if not np.all(np.isfinite(mu0)):
+            raise ValueError('`mu0` must be finite')
+        return mu0
+
+    def _forward_operator(self, pol, t_k=None):
+        eng = self.engine
+        P = eng.build_policy_tables(self, np.asarray(pol, dtype=float), t_k=t_k, deterministic=True)
+        return eng.build_forward(P)
+
+    def propagate_distribution(self, pol, mu0, n_steps=None, history=False, report_time=True):
+        """distribution of the state after `n_steps` steps under the policy `pol`, starting
+        from the distribution `mu0` on the state grid, and the expected stage cost of every
+        step.  Not in the reference (which simulates trajectories one point at a time).
+
+        The chain is the one the value function is computed with: the next state of a grid
+        point is spread over the corners of its cell with the interpolation weights (the
+        exact transpose of eval_policy's backup).  Next states outside the grid box
+        extrapolate, which can give negative mass near the boundary.  The operator is
+        linear, so `mu0` need not be normalised.
+
+        Stationary systems: `pol` of shape state_dims + (nb_control,), `n_steps` required.
+        Time-dependent systems: `pol` of shape (T,) + state_dims + (nb_control,) as returned
+        by bellman_recursion; step k applies pol[k] at instant k; `n_steps` defaults to T.
+
+        Returns (mu, expected_cost): mu_n of shape state_dims (or the history mu_0 .. mu_n,
+        shape (n_steps+1,) + state_dims, with `history`), and expected_cost[k] =
+        sum_x mu_k(x) * sum_w p_w g(x, pol(x), w), k < n_steps.
+        """
+        import torch
+        t_start = datetime.now()
+        state_dims = self._state_grid_shape
+        nb_control = len(self.sys.control)
+        pol = np.asarray(pol)
+        if self.sys.stationnary:
+            self._check_shape('pol', pol, state_dims + (nb_control,))
+            if n_steps is None:
+                raise ValueError('n_steps is required for a stationary system')
+        else:
+            T = pol.shape[0] if pol.ndim == len(state_dims) + 2 else 0
+            self._check_shape('pol', pol, (max(T, 1),) + state_dims + (nb_control,))
+            if n_steps is None:
+                n_steps = T
+            if n_steps > T:
+                raise ValueError('n_steps = {:d} exceeds the horizon of `pol` ({:d} instants)'.format(
+                    int(n_steps), T))
+        n_steps = int(n_steps)
+        if n_steps < 0:
+            raise ValueError('n_steps must be >= 0')
+        mu0 = self._check_mu0(mu0)
+        eng = self.engine
+        n = int(np.prod(state_dims))
+        if report_time:
+            print('distribution propagation...', end='')
+        mu_a = eng.to_device(mu0.reshape(-1))
+        mu_b = torch.empty_like(mu_a)
+        cost = torch.zeros(max(n_steps, 1), dtype=torch.float64, device=eng.device)
+        hist = torch.empty((n_steps + 1) * n, dtype=torch.float64, device=eng.device) if history else None
+        if self.sys.stationnary:
+            F = self._forward_operator(pol)
+            mu_n = eng.forward_steps(F, mu_a, mu_b, n_steps, cost, hist=hist)
+        else:
+            # the chain changes with the instant: tables and operator rebuilt per step
+            mu_n = mu_a
+            for k in range(n_steps):
+                F = self._forward_operator(pol[k], t_k=k)
+                nxt = mu_b if mu_n is mu_a else mu_a
+                eng.forward_steps(F, mu_n, nxt, 1, cost[k:k + 1],
+                                  hist=hist[k * n:(k + 2) * n] if history else None)
+                mu_n = nxt
+                del F
+        mu, cost_h = eng.to_host(hist if history else mu_n, cost)
+        exec_time = (datetime.now() - t_start).total_seconds()
+        if report_time:
+            print('\rdistribution propagation run in {:.2f} s'.format(exec_time))
+        shape = ((n_steps + 1,) if history else ()) + state_dims
+        return mu.reshape(shape), cost_h[:n_steps].copy()
+
+    def stationary_distribution(self, pol, mu0=None, tol=1e-12, max_iter=100_000, check_every=50,
+                                report_time=True):
+        """stationary distribution pi = P^T pi of the chain of the stationary policy `pol`
+        (see propagate_distribution), by power iteration from `mu0` (default: uniform 1/N).
+        Stops when sum |mu_{k+1} - mu_k| <= tol, checked every `check_every` steps, or after
+        `max_iter` steps; a chain that does not converge returns converged=False.  The
+        operator is linear, so `mu0` need not be normalised (tol is then relative to its mass).
+        Not in the reference.
+
+        Returns (pi, info): pi of shape state_dims, info = {'n_steps', 'converged',
+        'residuals' (one per check), 'average_cost' = sum_x pi(x) g_bar(x), 'mass' = sum pi,
+        'negative_mass' = sum min(pi, 0)} - negative mass means the grid is too small for the
+        policy's next states (they extrapolate out of the grid box).
+        """
+        t_start = datetime.now()
+        if not self.sys.stationnary:
+            raise ValueError('stationary_distribution needs a stationary system')
+        state_dims = self._state_grid_shape
+        pol = np.asarray(pol)
+        self._check_shape('pol', pol, state_dims + (len(self.sys.control),))
+        n = int(np.prod(state_dims))
+        mu0 = np.full(state_dims, 1.0 / n) if mu0 is None else self._check_mu0(mu0)
+        if int(max_iter) < 0 or int(check_every) < 1:
+            raise ValueError('max_iter must be >= 0 and check_every >= 1')
+        if report_time:
+            print('stationary distribution...', end='')
+        eng = self.engine
+        F = self._forward_operator(pol)
+        pi_dev, n_done, residuals, converged = eng.stationary(F, mu0, tol, int(max_iter), int(check_every))
+        pi, gbar = eng.to_host(pi_dev, F.bufs["gbar"])
+        pi = pi.reshape(state_dims)
+        info = {'n_steps': n_done, 'converged': converged, 'residuals': residuals,
+                'average_cost': float(np.dot(pi.reshape(-1), gbar)),
+                'mass': float(pi.sum()), 'negative_mass': float(np.minimum(pi, 0).sum())}
+        exec_time = (datetime.now() - t_start).total_seconds()
+        if report_time:
+            print('\rstationary distribution run in {:.2f} s ({:d} steps)'.format(exec_time, n_done))
+        return pi, info
+
+    # ------------------------------------------------------------------
     def print_summary(self):
         """summary of the discretisation (reference stodynprog.py:814-875)"""
         print('SDP solver for system "{}"'.format(self.sys.name))
