@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define SDP_ABI_VERSION 9
+#define SDP_ABI_VERSION 10
 #define SDP_MAX_D 4 /* the reference dispatches d = 1..4 (multilinear_cython.pyx:36-47) */
 
 /* error codes */
@@ -227,6 +227,17 @@ typedef struct SdpTables {
      * q*(W|1) + (q >> 1), SDP_COLUMN_PITCH2 doubles per column.
      * Combine pass: pos_row advanced to the band's first position. */
     const int32_t* pos_row;
+    /* Layout CF, optional scratch written with col_table (caller-owned, 16-byte aligned, NULL: no
+     * pruning): [n_cols][order[0]] pairs of doubles, for table row q of a column
+     *   m(q) = sum_w p_w * min(R[q][w], R[q+1][w])      (w in order, rounded as written)
+     *   A(q) = max_w max(|R[q][w]|, |R[q+1][w]|)        (NaN when one of them is NaN)
+     * and (0, NaN) for the last row.  m(q) + g*sum(p) bounds from below the value of every
+     * control whose axis-0 weight is in [0, 1] and that interpolates between rows q and q+1:
+     * the streaming pass skips a control when that bound, less a rounding margin, is already
+     * worse than the best value of the lane (DESIGN.md section 4; option "col_prune").  Used
+     * only with one row per lane, expect == 1 or W == 1, p_w in [0, 1], and when table and
+     * bound together fit SDP_COLUMN_MAX_SMEM_BYTES; ignored otherwise. */
+    double* col_bound;
 } SdpTables;
 
 /* ABI / build identification. */
@@ -245,14 +256,22 @@ const char* sdp_last_kernel(void);
  * "tma_rows" (4|8), "tma_stages" (2..16), "tma_warps" (1..16), "hoist" (layout AF
  * with u_mask == 1: per-item table of inner interpolations, 0|1), "hoist_upl" (2|4),
  * "hoist_const" (0|1: constant-W variant of that kernel for W <= 9),
- * "col_threads" (layout CF: threads per CTA, 128..768), "col_ub" (controls per iteration, 1|2),
+ * "col_threads" (layout CF: threads per CTA, 128..768; 0 = default, 768, or 640 when pruning), "col_ub" (controls per iteration, 1|2),
  * "col_pf" (groups of col_ub controls in flight, 1|2), "col_dynamic" (0|1: the warps of a CTA
  * take the items of a column round-robin / first come first served), "col_prepass" (column tables
  * from the coalesced pre-pass, copied into shared memory by the TMA engine = 2, default, or by
  * vector loads = 1; 0: every CTA gathers its own from J_prev),
+ * "col_prune" (layout CF with col_bound: skip the controls that provably lose, 1 = default, or
+ * evaluate every control, 0; the results are the same),
+ * "col_prune_stats" (0|1: count the warp steps of the pruning sweep and those skipped, read and
+ * reset by sdp_col_prune_counts; off by default, for measurements only),
  * "p2p_timeout_s" (bound of the peer-flag waits, default 600 s, then the kernel traps).
  * Not thread-safe against concurrent launches. */
 int sdp_set_option(const char* name, int value);
+/* With "col_prune_stats" on: the warp steps (groups of col_ub controls of one item) that the
+ * pruning column sweeps have met, and how many of them skipped the evaluation, since the previous
+ * call.  Synchronizes the device.  Both are 0 when nothing was counted. */
+int sdp_col_prune_counts(int64_t* steps, int64_t* skipped);
 
 /* K0a - cell search on explicit points.
  * Replaces the cell-search half of multilinear_interpolation_{1..4}d

@@ -12,7 +12,7 @@ import numpy as np
 
 SDP_MAX_D = 4
 SDP_MAX_C = 4
-SDP_ABI_VERSION = 9
+SDP_ABI_VERSION = 10
 LAYOUT_CONTROL_MINOR = 0   # "A": [state][w][u]
 LAYOUT_STATE_MINOR = 1     # "B": [tile of 32 states][u][w][lane]
 LAYOUT_CONTROL_MINOR_FACTORED = 2   # "AF": (x,u) part [state][Upad] + (x,w) part [state][W]
@@ -77,7 +77,8 @@ class SdpTables(ctypes.Structure):
                 ("col_table_ready", ctypes.c_int32),
                 ("col_launch_hint", ctypes.c_int32),
                 ("item_order", ctypes.c_void_p),
-                ("pos_row", ctypes.c_void_p)]
+                ("pos_row", ctypes.c_void_p),
+                ("col_bound", ctypes.c_void_p)]
 
 
 SDP_MAX_PEERS = 8
@@ -141,6 +142,7 @@ SIGNATURES = {
     "sdp_launch_count": (_i64, []),
     "sdp_last_kernel": (ctypes.c_char_p, []),
     "sdp_set_option": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_int]),
+    "sdp_col_prune_counts": (ctypes.c_int, [ctypes.POINTER(_i64), ctypes.POINTER(_i64)]),
     "sdp_cell_setup": (ctypes.c_int, [_gp, _i64, _vp, _vp, _vp, _vp]),
     "sdp_build_tables": (ctypes.c_int, [_gp, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _i64, _vp,
                                         _i32, _vp]),

@@ -1070,6 +1070,8 @@ struct Tuning {
     int col_pf;        // layout CF: groups of col_ub controls in flight per lane (1|2)
     int col_dynamic;   // layout CF: warps take the items of a column first come first served (1) or round-robin (0)
     int col_prepass;   // layout CF: column tables from the coalesced pre-pass, copied by vector loads (1) or by the TMA engine (2); 0: gathered by every CTA
+    int col_prune;     // layout CF with SdpTables.col_bound: skip the controls that provably lose (1) or evaluate all (0)
+    int col_prune_stats; // layout CF pruning sweep: count warp steps and skipped ones (measurements only)
     int pdl;           // programmatic dependent launch of pre-pass / column sweep / combine (1) or plain launches (0)
     int small_combine; // sdp_sweep_finalize_cols: the 128-thread combine that fits next to a streaming CTA (1) or the 1024-thread one (0)
     int carveout;      // layout CF: streaming kernel and small combine ask for the largest shared-memory carve-out (1) or leave it to the driver (0)
@@ -1109,11 +1111,14 @@ static Tuning& tuning() {
         // round 2 (profiles/r2_emu_variants.txt, one band / one shard of eight): 640 threads round-robin
         // 1.180 / 0.1788 ms, 640 first-come-first-served 1.168 / 0.1729, 768 round-robin 1.158 / 0.1746,
         // 768 first-come-first-served 1.148 / 0.1726 -> 768 threads, items handed out dynamically
-        x.col_threads = clampi(env_int("SDP_COL_THREADS", 768), 128, 768) / 32 * 32;
+        // 0 = by kernel: 768, or 640 for the pruning sweep (column_threads)
+        x.col_threads = env_int("SDP_COL_THREADS", 0) ? clampi(env_int("SDP_COL_THREADS", 0), 128, 768) / 32 * 32 : 0;
         x.col_ub = env_int("SDP_COL_UB", 2) == 1 ? 1 : 2;
         x.col_pf = env_int("SDP_COL_PF", 2) == 1 ? 1 : 2;
         x.col_prepass = clampi(env_int("SDP_COL_PREPASS", 3), 0, 3);
         x.col_dynamic = env_int("SDP_COL_DYNAMIC", 1) != 0;
+        x.col_prune = env_int("SDP_COL_PRUNE", 1) != 0;
+        x.col_prune_stats = 0;
         x.dbg_exchange = 0;
         x.pdl = env_int("SDP_PDL", 1) != 0;
         x.small_combine = env_int("SDP_SMALL_COMBINE", 1) != 0;
@@ -1136,11 +1141,13 @@ extern "C" int sdp_set_option(const char* name, int value) {
     else if (!strcmp(name, "hoist_upl")) t.hoist_upl = (value == 4) ? 4 : 2;
     else if (!strcmp(name, "p2p_timeout_s")) t.p2p_timeout_s = clampi(value, 1, 86400);
     else if (!strcmp(name, "hoist_const")) t.hoist_const = value != 0;
-    else if (!strcmp(name, "col_threads")) t.col_threads = clampi(value, 128, 768) / 32 * 32;
+    else if (!strcmp(name, "col_threads")) t.col_threads = value ? clampi(value, 128, 768) / 32 * 32 : 0;
     else if (!strcmp(name, "col_ub")) t.col_ub = (value == 1) ? 1 : 2;
     else if (!strcmp(name, "col_pf")) t.col_pf = (value == 1) ? 1 : 2;
     else if (!strcmp(name, "col_prepass")) t.col_prepass = clampi(value, 0, 3);
     else if (!strcmp(name, "col_dynamic")) t.col_dynamic = value != 0;
+    else if (!strcmp(name, "col_prune")) t.col_prune = value != 0;
+    else if (!strcmp(name, "col_prune_stats")) t.col_prune_stats = value != 0;
     else if (!strcmp(name, "dbg_exchange")) t.dbg_exchange = value;
     else if (!strcmp(name, "pdl")) t.pdl = value != 0;
     else if (!strcmp(name, "small_combine")) t.small_combine = value != 0;
@@ -1862,6 +1869,40 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 // the first kernel that reads J_prev must perform (consumed by launch_column_table)
 static thread_local const PeersDev* g_wait_peers = nullptr;
 
+// Column pruning (SdpTables.col_bound, DESIGN.md section 4).  With 0 <= l <= 1 and p_w >= 0 the
+// value of a control, sum_w p_w*(g + (1-l)*R[q][w] + l*R[q+1][w]), is at least
+//     g*sum(p) + m(q),   m(q) = sum_w p_w*min(R[q][w], R[q+1][w]),
+// and the value the sweep computes (oml = 1-l, the two products, the add, + g, * p_w, the sum in
+// w order, all rounded to nearest, no FMA) lies within (W+4)*u*(|g| + A)*sum(p) of the exact one
+// (u = 2^-53, A = max_w max(|R[q][w]|, |R[q+1][w]|)).  Computing m(q), g*sum(p), their sum and
+// the subtraction of the margin rounds by at most (W+2)*u*(|g| + A)*sum(p) more, so with W <= 9
+// a margin of 32*u*(|g| + A)*sum(p) (24*u needed, the rest covers O(u^2) terms and the rounding
+// of the margin itself) plus 2^-1000 (underflow in the products) makes `lb` a lower bound of the
+// computed value: lb > best means the control computes a value strictly greater than best, which
+// is neither the minimum nor, at a tie, the argmin.  |g| + A <= 2^1000 and p_w <= 1 rule out
+// overflow (and NaN) in the computed value; a NaN or inf in R or g fails that test, so such a
+// control is never skipped.  Twin: tablebuild.column_prune_skip.
+__device__ __forceinline__ double2 column_bound(const double* r, int P, int W, const PVals& PV) {
+    double m = 0.0, a = 0.0;
+    bool nan = false;
+#pragma unroll
+    for (int w = 0; w < SDP_FACTORED_MAX_W_REG; ++w) {
+        if (w < W) {
+            const double x = r[w], y = r[P + w];
+            m = add_(m, mul_(PV.v[w], fmin(x, y)));
+            a = fmax(a, fmax(fabs(x), fabs(y)));
+            nan |= (x != x) | (y != y);
+        }
+    }
+    return make_double2(m, nan ? CUDART_NAN : a);
+}
+__device__ __forceinline__ bool column_skip(double2 b, double g, double l, double sum_p, double best) {
+    const double ga = add_(fabs(g), b.y);
+    const double margin = add_(mul_(mul_(ga, sum_p), 0x1p-48), 0x1p-1000);
+    const double lb = sub_(add_(mul_(g, sum_p), b.x), margin);
+    return (l >= 0.0) & (l <= 1.0) & (ga <= 0x1p1000) & (lb > best);
+}
+
 #define SDP_CT_ROWS 16
 // `WAIT`: every CTA first waits (lanes 0..world-1, ld.acquire.sys on the local flags) until all
 // ranks have published the current epoch, i.e. until the J slabs of the previous sweep have
@@ -1869,7 +1910,7 @@ static thread_local const PeersDev* g_wait_peers = nullptr;
 template <int D, bool WAIT>
 __global__ void __launch_bounds__(256)
 k_column_table(GridT<double> G, SdpTables T, const double* __restrict__ Jprev, int64_t pitch,
-               PeersDev PW, unsigned long long timeout_ns, int TR) {
+               PeersDev PW, unsigned long long timeout_ns, int TR, PVals PV, int bound) {
     constexpr int NW = D - 1;
     extern __shared__ __align__(16) unsigned char tsm[];
     cudaGridDependencySynchronize();       // (programmatic dependent launch: the previous kernel's writes)
@@ -1879,7 +1920,8 @@ k_column_table(GridT<double> G, SdpTables T, const double* __restrict__ Jprev, i
     }
     const int W = T.W;
     const int P = W | 1;
-    const int CP = TR * P + 1;                    // odd tile pitch per column: conflict-free both ways
+    const int TRc = TR + (bound ? 1 : 0);         // (the bound of row r0+TR-1 also needs row r0+TR)
+    const int CP = (TRc * P) | 1;                 // odd tile pitch per column: conflict-free both ways
     double* tile = reinterpret_cast<double*>(tsm);             // [32][CP]
     double* lw_s = tile + 32 * CP;                             // [NW][32][W]
     int* cw_s = reinterpret_cast<int*>(lw_s + NW * 32 * W);    // [32][W]
@@ -1896,7 +1938,7 @@ k_column_table(GridT<double> G, SdpTables T, const double* __restrict__ Jprev, i
     __syncthreads();
     // (independent iterations: unrolled so that the gathers of several elements are in flight)
 #pragma unroll 6
-    for (int k = threadIdx.x; k < TR * W * 32; k += blockDim.x) {
+    for (int k = threadIdx.x; k < TRc * W * 32; k += blockDim.x) {
         const int lc = k & 31;
         const int rw = k >> 5;
         const int lr = rw / W, w = rw - lr * W;
@@ -1923,6 +1965,35 @@ k_column_table(GridT<double> G, SdpTables T, const double* __restrict__ Jprev, i
             for (int k = threadIdx.x & 31; k < nr * P; k += 32) dst[k] = tile[lc * CP + k];
         }
     }
+    if (bound) {
+        // (threads along the rows of a column: the 16-byte stores of a warp are contiguous)
+        double2* dstb = reinterpret_cast<double2*>(T.col_bound);
+        for (int k = threadIdx.x; k < 32 * nr; k += blockDim.x) {
+            const int lc = k / nr, lr = k - lc * nr, q = r0 + lr;
+            if (c0 + lc >= T.n_cols) break;
+            dstb[(int64_t)(c0 + lc) * rows + q] =
+                q < rows - 1 ? column_bound(tile + lc * CP + lr * P, P, W, PV) : make_double2(0.0, CUDART_NAN);
+        }
+    }
+}
+
+// probabilities of the column kernels as launch constants (1 for a deterministic system)
+static PVals column_pvals(const SdpTables& T) {
+    PVals pv;
+    for (int w = 0; w < SDP_FACTORED_MAX_W_REG; ++w)
+        pv.v[w] = (w < T.W) ? (T.expect ? T.p_host[w] : 1.0) : 0.0;
+    return pv;
+}
+// whether the pre-pass writes SdpTables.col_bound (and the sweep may prune): depends on the
+// tables and the grid only, so that a separate pre-pass (sdp_column_table) and the sweep agree
+static bool column_bound_on(const GridT<double>& G, const SdpTables& T) {
+    if (!T.col_bound || ((uintptr_t)T.col_bound & 15) || T.col_pairs || !(T.expect || T.W == 1))
+        return false;
+    if (SDP_COLUMN_PITCH(G.order[0], T.W) * 8 + (int64_t)G.order[0] * 16 > SDP_COLUMN_MAX_SMEM_BYTES) return false;
+    const PVals pv = column_pvals(T);
+    for (int w = 0; w < T.W; ++w)
+        if (!(pv.v[w] >= 0.0 && pv.v[w] <= 1.0)) return false;
+    return true;
 }
 
 template <int D>
@@ -1934,7 +2005,9 @@ static int launch_column_table(const GridT<double>& G, const SdpTables& T, const
     int TR = SDP_CT_ROWS;
     const int64_t col_blocks = (T.n_cols + 31) / 32;
     while (TR > 4 && col_blocks * ((G.order[0] + TR - 1) / TR) < 148 * 6) TR >>= 1;
-    const size_t tshm = (size_t)32 * (TR * P + 1) * 8 + (size_t)NW * 32 * T.W * 8 + (size_t)32 * T.W * 4;
+    const int bound = column_bound_on(G, T);
+    const PVals pv = column_pvals(T);
+    const size_t tshm = (size_t)32 * (((TR + bound) * P) | 1) * 8 + (size_t)NW * 32 * T.W * 8 + (size_t)32 * T.W * 4;
     dim3 grid((unsigned)col_blocks, (unsigned)((G.order[0] + TR - 1) / TR));
     const int64_t pitch = T.col_pairs ? SDP_COLUMN_PITCH2(G.order[0], T.W) : SDP_COLUMN_PITCH(G.order[0], T.W);
     if (g_wait_peers) {
@@ -1942,11 +2015,11 @@ static int launch_column_table(const GridT<double>& G, const SdpTables& T, const
         const PeersDev P2 = *g_wait_peers;
         g_wait_peers = nullptr;
         launch_pdl(k_column_table<D, true>, grid, dim3(256), tshm, st,
-                   G, T, Jprev, pitch, P2, (unsigned long long)tuning().p2p_timeout_s * 1000000000ULL, TR);
+                   G, T, Jprev, pitch, P2, (unsigned long long)tuning().p2p_timeout_s * 1000000000ULL, TR, pv, bound);
     } else {
         PeersDev none;
         memset(&none, 0, sizeof(none));
-        launch_pdl(k_column_table<D, false>, grid, dim3(256), tshm, st, G, T, Jprev, pitch, none, 0ULL, TR);
+        launch_pdl(k_column_table<D, false>, grid, dim3(256), tshm, st, G, T, Jprev, pitch, none, 0ULL, TR, pv, bound);
     }
     SDP_LAUNCH_CHECK();
     return SDP_OK;
@@ -1955,15 +2028,24 @@ static int launch_column_table(const GridT<double>& G, const SdpTables& T, const
 // MAXT: launch bound (512 threads leave 128 registers per thread, 640 leave 102, 768 leave 85).
 // prepass: 0 = the CTA gathers its table from J_prev, 1 = copies it from col_table with
 // vector loads, 2 = with one bulk asynchronous copy (TMA engine, SASS UBLKCP) on an mbarrier.
-template <int D, int WM, int UB, int PF, bool FULL, int MAXT>     // FULL: W == WM, every slot live
+// PRUNE: the column's bound (SdpTables.col_bound) comes with its table, behind it in shared
+// memory; a group of UB controls is skipped when no lane needs any of them (column_skip: it
+// provably loses against the lane's best so far).  Each lane first evaluates the control it
+// chose in the previous sweep (part_idx, when it is a control of the item), so that the best
+// is good from the first group on.  The minimum over the controls, ties to the lowest index
+// (`better`), does not depend on the order they are visited in: the results are those of
+// PRUNE = false, bit for bit.  `stats` (optional): warp steps met and skipped.
+template <int D, int WM, int UB, int PF, bool FULL, int MAXT, bool PRUNE>     // FULL: W == WM, every slot live
 __global__ void __launch_bounds__(MAXT, 1)
 k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jprev,
                     double* __restrict__ part_val, int32_t* __restrict__ part_idx,
-                    double inv_stride0, PVals PV, int64_t pitch, int prepass, int dynamic) {
+                    double inv_stride0, PVals PV, int64_t pitch, int prepass, int dynamic,
+                    double sum_p, unsigned long long* __restrict__ stats) {
     constexpr int NW = D - 1;
     extern __shared__ __align__(128) unsigned char csm[];
     __shared__ int next_item[2];                        // dynamic hand-out of the items of a column (two, used in turn)
     double* R_sh = reinterpret_cast<double*>(csm);      // [order[0]][P] + slack = `pitch` doubles
+    const double2* B_sh = reinterpret_cast<const double2*>(csm + pitch * 8);     // PRUNE: [order[0]] (m, A)
     __shared__ int cw_sh[WM];
     __shared__ double lw_sh[NW][WM];
     __shared__ __align__(8) uint64_t tbar;              // completion of the bulk copy of a table
@@ -2003,10 +2085,17 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
             if (threadIdx.x == 0) {
                 const unsigned char* src = reinterpret_cast<const unsigned char*>(T.col_table + (int64_t)col * pitch);
                 const uint32_t bytes = (uint32_t)(pitch * 8);
+                const uint32_t bbytes = PRUNE ? (uint32_t)rows * 16u : 0u;
                 const uint32_t bar = smem_u32(&tbar);
-                mbar_expect_tx(bar, bytes);
+                mbar_expect_tx(bar, bytes + bbytes);
                 for (uint32_t o = 0; o < bytes; o += 32768u)
                     bulk_g2s(smem_u32(csm + o), src + o, min(32768u, bytes - o), bar);
+                if (PRUNE) {
+                    // the bound, on the same barrier
+                    const unsigned char* bsrc = reinterpret_cast<const unsigned char*>(T.col_bound + (int64_t)col * rows * 2);
+                    for (uint32_t o = 0; o < bbytes; o += 32768u)
+                        bulk_g2s(smem_u32(csm + bytes + o), bsrc + o, min(32768u, bbytes - o), bar);
+                }
             }
             if (prepass == 2) {          // (3: the wait moves behind the first item's loads)
                 mbar_wait(smem_u32(&tbar), tphase);
@@ -2025,6 +2114,11 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
                 for (int j = 0; j < 8; ++j) dst[k + j * blockDim.x] = v[j];
             }
             for (; k < n2; k += blockDim.x) dst[k] = src[k];
+            if (PRUNE) {
+                const double2* __restrict__ bsrc = reinterpret_cast<const double2*>(T.col_bound + (int64_t)col * rows * 2);
+                double2* bdst = reinterpret_cast<double2*>(R_sh + pitch);
+                for (int r = threadIdx.x; r < rows; r += blockDim.x) bdst[r] = bsrc[r];
+            }
         } else {
             if (threadIdx.x < W) {
                 // the column's w-part: lane 0 of its first tile
@@ -2042,6 +2136,12 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
 #pragma unroll
                 for (int k = 0; k < NW; ++k) lam[k + 1] = lw_sh[k][w];
                 R_sh[r * P + w] = Lerp<double, D, 1>::eval(Jprev, r * stride0 + cw_sh[w], G.stride, lam);
+            }
+            if (PRUNE) {
+                __syncthreads();
+                double2* bdst = reinterpret_cast<double2*>(R_sh + pitch);
+                for (int r = threadIdx.x; r < rows; r += blockDim.x)
+                    bdst[r] = r < rows - 1 ? column_bound(R_sh + r * P, P, W, PV) : make_double2(0.0, CUDART_NAN);
             }
         }
         if (prepass < 2) __syncthreads();
@@ -2065,6 +2165,22 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
             double best_v = CUDART_INF;
             int best_i = INT_MAX;
             const int last = it.u_count - 1;
+            // PRUNE: the lane's choice of the previous sweep, if it is one of this item's controls
+            // (read before this warp overwrites it below; any other value is ignored)
+            int seed = -1;
+            int c_s = 0;
+            double g_s = 0.0, l_s = 0.0;
+            if (PRUNE) {
+                const int s = part_idx[item_id * 32 + lane];
+                if (s >= it.u_begin && s - it.u_begin < it.u_count && s < Us) {
+                    seed = s;
+                    const int64_t o = (int64_t)(s - it.u_begin) * 32;
+                    c_s = cup[o];
+                    g_s = gp[o];
+                    l_s = lup[o];
+                }
+            }
+            int n_steps = 0, n_skipped = 0;
 
             // PF groups of UB controls are in flight: group k of the run sits in stage k % PF
             // (rows past the run repeat its last row)
@@ -2083,6 +2199,24 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
                 mbar_wait(smem_u32(&tbar), tphase);
                 have_table = true;
             }
+            if (PRUNE && seed >= 0) {
+                // the seed, evaluated with the very operations of the loop below
+                const double oml = sub_(1.0, l_s);
+                const int q = __double2int_rn(__dmul_rn((double)c_s, inv_stride0));
+                const double* Ra = R_sh + q * P;
+                double acc = 0.0;
+#pragma unroll
+                for (int w = 0; w < WM; ++w) {
+                    const double v = add_(mul_(oml, Ra[w]), mul_(l_s, Ra[P + w]));
+                    const double jg = add_(g_s, v);
+                    const double nxt = T.expect ? add_(acc, mul_(jg, PV.v[w])) : jg;
+                    acc = (FULL || w < W) ? nxt : acc;
+                }
+                if (better(acc, seed, best_v, best_i)) {
+                    best_v = acc;
+                    best_i = seed;
+                }
+            }
             for (int uu0 = 0; uu0 < it.u_count; uu0 += UB * PF) {
 #pragma unroll
                 for (int s = 0; s < PF; ++s) {
@@ -2090,6 +2224,7 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
                     if (uu < it.u_count) {                    // warp-uniform
                         double gv[UB], lu[UB], oml[UB];
                         const double* Ra[UB];
+                        bool need = !PRUNE;
 #pragma unroll
                         for (int b = 0; b < UB; ++b) {
                             gv[b] = g_n[s][b];
@@ -2099,6 +2234,9 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
                             // below 2^31; padding entries hold cell 0)
                             const int q = __double2int_rn(__dmul_rn((double)c_n[s][b], inv_stride0));
                             Ra[b] = R_sh + q * P;
+                            // (padding lanes and rows past the run never need a control)
+                            if (PRUNE && uu + b <= last && it.u_begin + uu + b < Us)
+                                need |= !column_skip(B_sh[q], gv[b], lu[b], sum_p, best_v);
                         }
                         if (uu + UB * PF < it.u_count) {
 #pragma unroll
@@ -2107,6 +2245,13 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
                                 c_n[s][b] = __ldcs(cup + o);
                                 g_n[s][b] = __ldcs(gp + o);
                                 l_n[s][b] = __ldcs(lup + o);
+                            }
+                        }
+                        if (PRUNE) {
+                            ++n_steps;
+                            if (!__any_sync(0xffffffffu, need)) {
+                                ++n_skipped;
+                                continue;
                             }
                         }
                         // slots >= W read past the W live values of a row (its pad, the next row,
@@ -2137,6 +2282,10 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
             }
             part_val[item_id * 32 + lane] = best_v;
             part_idx[item_id * 32 + lane] = best_i;
+            if (PRUNE && stats && lane == 0) {
+                atomicAdd(stats, (unsigned long long)n_steps);
+                atomicAdd(stats + 1, (unsigned long long)n_skipped);
+            }
         }
         if (prepass >= 2) {
             // a warp that got no item of this run still observes the copy's completion: thread 0
@@ -2149,51 +2298,100 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
     }
 }
 
+// pruning sweep: warp steps met / skipped, counted with "col_prune_stats" (sdp_col_prune_counts)
+static unsigned long long* g_prune_stats = nullptr;
+extern "C" int sdp_col_prune_counts(int64_t* steps, int64_t* skipped) {
+    if (!steps || !skipped) return fail(SDP_EINVAL, "%s", "sdp_col_prune_counts: NULL pointer");
+    *steps = *skipped = 0;
+    if (!g_prune_stats) return SDP_OK;
+    unsigned long long h[2];
+    cudaError_t e = cudaDeviceSynchronize();
+    if (e == cudaSuccess) e = cudaMemcpy(h, g_prune_stats, sizeof(h), cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess) e = cudaMemset(g_prune_stats, 0, sizeof(h));
+    if (e != cudaSuccess) return fail(SDP_ECUDA, "sdp_col_prune_counts: %s", cudaGetErrorString(e));
+    *steps = (int64_t)h[0];
+    *skipped = (int64_t)h[1];
+    return SDP_OK;
+}
+
+template <int D, int WM, int UB, int PF, int MAXT, bool PRUNE>
+static int set_column_attrs(size_t shm) {
+    static size_t attr_set = 0;          // per instantiation
+    if (attr_set >= shm) return SDP_OK;
+    cudaError_t e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE>,
+                                         cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm);
+    if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE>,
+                                 cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm);
+    // the largest shared-memory carve-out (the kernel streams with evict-first loads: 2 % L1 hit
+    // rate): k_combine_column_small asks for the same one, so that one of its CTAs can join a
+    // resident CTA of this kernel without the SM draining to change its configuration
+    if (e == cudaSuccess && tuning().carveout)
+        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE>,
+                                 cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if (e == cudaSuccess && tuning().carveout)
+        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE>,
+                                 cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if (e != cudaSuccess) return fail(SDP_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
+    attr_set = shm;
+    return SDP_OK;
+}
+
+template <int D, int WM, int UB, int PF, int MAXT, bool PRUNE>
+static void launch_fact_column_kp(const GridT<double>& G, const SdpTables& T, const double* Jprev,
+                                  double* part_val, int32_t* part_idx, cudaStream_t st, int threads, size_t shm,
+                                  int64_t pitch, int prepass, double sum_p, unsigned long long* stats) {
+    const PVals pv = column_pvals(T);
+    const double inv0 = 1.0 / (double)G.stride[0];
+    const int dynamic = (T.col_launch_hint & 0xffff) ? !((T.col_launch_hint >> 16) & 1) : tuning().col_dynamic;
+    if (T.W == WM)
+        launch_pdl(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE>, dim3((unsigned)T.n_segs), dim3(threads),
+                   shm, st, G, T, Jprev, part_val, part_idx, inv0, pv, pitch, prepass, dynamic, sum_p, stats);
+    else
+        launch_pdl(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE>, dim3((unsigned)T.n_segs), dim3(threads),
+                   shm, st, G, T, Jprev, part_val, part_idx, inv0, pv, pitch, prepass, dynamic, sum_p, stats);
+}
+
 template <int D, int WM, int UB, int PF, int MAXT>
 static int launch_fact_column_k(const GridT<double>& G, const SdpTables& T, const double* Jprev,
                                 double* part_val, int32_t* part_idx, cudaStream_t st, int threads) {
     const int64_t pitch = SDP_COLUMN_PITCH(G.order[0], T.W);
-    const size_t shm = (size_t)pitch * 8;
-    if (shm > SDP_COLUMN_MAX_SMEM_BYTES)
+    if ((size_t)pitch * 8 > SDP_COLUMN_MAX_SMEM_BYTES)
         return fail(SDP_EINVAL, "%s", "sdp_sweep: layout CF: the column table does not fit shared memory");
     const int prepass = tuning().col_prepass;
     if (prepass && !T.col_table_ready) {
         int rc = launch_column_table<D>(G, T, Jprev, st);
         if (rc) return rc;
     }
-    static size_t attr_set = 0;          // per instantiation
-    if (attr_set < shm) {
-        cudaError_t e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, true, MAXT>,
-                                             cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm);
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, false, MAXT>,
-                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm);
-        // the largest shared-memory carve-out (the kernel streams with evict-first loads: 2 % L1 hit
-        // rate): k_combine_column_small asks for the same one, so that one of its CTAs can join a
-        // resident CTA of this kernel without the SM draining to change its configuration
-        if (e == cudaSuccess && tuning().carveout)
-            e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, true, MAXT>,
-                                     cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (e == cudaSuccess && tuning().carveout)
-            e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, false, MAXT>,
-                                     cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-        if (e != cudaSuccess) return fail(SDP_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
-        attr_set = shm;
+    const bool prune = tuning().col_prune && column_bound_on(G, T);
+    const size_t shm = (size_t)pitch * 8 + (prune ? (size_t)G.order[0] * 16 : 0);
+    int rc = prune ? set_column_attrs<D, WM, UB, PF, MAXT, true>(shm) : set_column_attrs<D, WM, UB, PF, MAXT, false>(shm);
+    if (rc) return rc;
+    if (prune) {
+        unsigned long long* stats = nullptr;
+        if (tuning().col_prune_stats) {
+            if (!g_prune_stats) {
+                cudaError_t e = cudaMalloc(&g_prune_stats, 2 * sizeof(unsigned long long));
+                if (e == cudaSuccess) e = cudaMemset(g_prune_stats, 0, 2 * sizeof(unsigned long long));
+                if (e != cudaSuccess) {
+                    g_prune_stats = nullptr;
+                    return fail(SDP_ECUDA, "col_prune_stats: %s", cudaGetErrorString(e));
+                }
+            }
+            stats = g_prune_stats;
+        }
+        const PVals pv = column_pvals(T);
+        double sum_p = 0.0;                  // (in w order: tablebuild.column_prune_skip)
+        for (int w = 0; w < T.W; ++w) sum_p += pv.v[w];
+        launch_fact_column_kp<D, WM, UB, PF, MAXT, true>(G, T, Jprev, part_val, part_idx, st, threads, shm, pitch,
+                                                         prepass, sum_p, stats);
+    } else {
+        launch_fact_column_kp<D, WM, UB, PF, MAXT, false>(G, T, Jprev, part_val, part_idx, st, threads, shm, pitch,
+                                                          prepass, 0.0, nullptr);
     }
-    PVals pv;
-    for (int w = 0; w < SDP_FACTORED_MAX_W_REG; ++w)
-        pv.v[w] = (w < T.W) ? (T.expect ? T.p_host[w] : 1.0) : 0.0;
-    const double inv0 = 1.0 / (double)G.stride[0];
-    const int dynamic = (T.col_launch_hint & 0xffff) ? !((T.col_launch_hint >> 16) & 1) : tuning().col_dynamic;
-    if (T.W == WM)
-        launch_pdl(k_sweep_fact_column<D, WM, UB, PF, true, MAXT>, dim3((unsigned)T.n_segs), dim3(threads), shm, st,
-                   G, T, Jprev, part_val, part_idx, inv0, pv, pitch, prepass, dynamic);
-    else
-        launch_pdl(k_sweep_fact_column<D, WM, UB, PF, false, MAXT>, dim3((unsigned)T.n_segs), dim3(threads), shm, st,
-                   G, T, Jprev, part_val, part_idx, inv0, pv, pitch, prepass, dynamic);
-    note_kernel("%sk_sweep_fact_column<%d,%d,%d,%d,%s,%d> [%d CTAs x %d threads]",
+    note_kernel("%sk_sweep_fact_column<%d,%d,%d,%d,%s,%d%s> [%d CTAs x %d threads]",
                 (prepass && !T.col_table_ready) ? "k_column_table + " : "", D, WM, UB, PF,
-                T.W == WM ? "true" : "false", MAXT, (int)T.n_segs, threads);
+                T.W == WM ? "true" : "false", MAXT, prune ? ",prune" : "", (int)T.n_segs, threads);
     SDP_LAUNCH_CHECK();
     return SDP_OK;
 }
@@ -2400,7 +2598,7 @@ template <int D, int WM>
 static int launch_fact_column2_w(const GridT<double>& G, const SdpTables& T, const double* Jprev,
                                  double* part_val, int32_t* part_idx, cudaStream_t st) {
     const int hint_threads = T.col_launch_hint & 0xffff;
-    const int threads = hint_threads ? clampi(hint_threads, 128, 768) / 32 * 32 : tuning().col_threads;
+    const int threads = hint_threads ? clampi(hint_threads, 128, 768) / 32 * 32 : (tuning().col_threads ? tuning().col_threads : 768);
     if (threads > 640) return launch_fact_column2_k<D, WM, 768>(G, T, Jprev, part_val, part_idx, st, threads);
     return launch_fact_column2_k<D, WM, 640>(G, T, Jprev, part_val, part_idx, st, threads);
 }
@@ -2413,7 +2611,13 @@ static int launch_fact_column_w(const GridT<double>& G, const SdpTables& T, cons
     // run best with 640 threads round-robin, long ones with 768 and first come first served
     const int hint_threads = T.col_launch_hint & 0xffff;
     const int ub = tuning().col_ub, pf = tuning().col_pf;
-    const int threads = hint_threads ? clampi(hint_threads, 128, 768) / 32 * 32 : tuning().col_threads;
+    // default CTA size: 768 threads (one group of 2 controls in flight per lane); the pruning sweep
+    // skips ~94 % of the evaluations of config #5 and is then bound by the latency of the (x,u)
+    // stream, which 640 threads with two groups in flight hide better: 1.003 against 1.044 ms per
+    // sweep (profiles/r3_prune_timing.json, "launch_shapes")
+    const int auto_threads = (tuning().col_prune && column_bound_on(G, T)) ? 640 : 768;
+    const int threads = hint_threads ? clampi(hint_threads, 128, 768) / 32 * 32
+                                     : (tuning().col_threads ? tuning().col_threads : auto_threads);
     if (threads > 640) {       // 85 registers per thread
         if (ub == 2) return launch_fact_column_k<D, WM, 2, 1, 768>(G, T, Jprev, part_val, part_idx, st, threads);
         return pf == 2 ? launch_fact_column_k<D, WM, 1, 2, 768>(G, T, Jprev, part_val, part_idx, st, threads)

@@ -276,6 +276,35 @@ def column_piece_cuts(col_csum, fractions, n_ctas=0):
     return cuts + [n_cols]
 
 
+def column_prune_skip(g, lam, R0, R1, p, expect, best):
+    """Layout CF, pruning: the skip decision of the column sweep for one control (twin of the device
+    code: column_bound in the pre-pass, column_skip in the sweep; DESIGN.md section 4).  The control
+    interpolates with weight `lam` between table rows R0 and R1 (W values each), `g` is its stage
+    cost, `p` the W probabilities (expect = 0: W = 1 and p = [1]), `best` the lane's best value so
+    far.  True: the value the sweep would compute is strictly greater than `best`.  Returns False
+    wherever the sweep does not prune (p outside [0, 1], expect = 0 with W > 1, W > 9)."""
+    R0, R1 = np.asarray(R0, dtype=np.float64), np.asarray(R1, dtype=np.float64)
+    W = len(R0)
+    pv = [float(x) for x in p] if expect else [1.0] * W
+    if W > _cabi.FACTORED_MAX_W_REG or (not expect and W != 1) or not all(0.0 <= x <= 1.0 for x in pv):
+        return False
+    sum_p = 0.0
+    for x in pv:
+        sum_p += x
+    with np.errstate(invalid="ignore", over="ignore"):
+        m, a = np.float64(0.0), np.float64(0.0)
+        for w in range(W):
+            m = m + np.float64(pv[w]) * np.fmin(R0[w], R1[w])
+            a = np.fmax(a, np.fmax(abs(R0[w]), abs(R1[w])))
+        if np.isnan(R0).any() or np.isnan(R1).any():
+            a = np.float64(np.nan)
+        g = np.float64(g)
+        ga = abs(g) + a
+        margin = ga * np.float64(sum_p) * np.float64(2.0 ** -48) + np.float64(2.0 ** -1000)
+        lb = (g * np.float64(sum_p) + m) - margin
+        return bool(0.0 <= lam <= 1.0 and ga <= 2.0 ** 1000 and lb > best)
+
+
 def row_aligned(bounds, n_cols):
     """slab boundaries moved to the nearest multiple of n_cols (whole rows of axis 0),
     kept monotone"""
@@ -333,6 +362,7 @@ class SweepTables(object):
         self.n_segs = 0
         self.item_u_count_host = None
         self.col_table = None      # device fp64 scratch: the column tables of the current sweep
+        self.col_bound = None      # device fp64 scratch: their per-row bounds (SdpTables.col_bound)
         self.run_end = None        # device int64 [n_items]: end of every item's (band, column) run
         self.pairs = False         # layout CF with two rows per lane (SdpTables.col_pairs)
         self.pos_row = self.work_dev = self.work_host = None
@@ -396,6 +426,7 @@ def fill_c_tables(T):
             c.n_cols, c.tiles_per_col = T.n_cols, T.tiles_per_col
             c.seg_begin, c.n_segs = T.seg_begin.data_ptr(), T.n_segs
             c.col_table = T.col_table.data_ptr()
+            c.col_bound = T.col_bound.data_ptr()
             c.col_table_ready = 0
             if T.item_order is not None:
                 # several bands: the whole-list launch walks the bands of a column back to back
@@ -1068,8 +1099,9 @@ class ShardBuild(object):
                 T.work_dev, T.pos_row = up[-2], up[-1]
             self.ensure("col_table", self.n_cols_loc * _cabi.column_pitch(plan.n_rows0, plan.W, T.pairs),
                         torch.float64)
+            self.ensure("col_bound", self.n_cols_loc * plan.n_rows0 * 2, torch.float64)
         else:
-            T.col_table = None
+            T.col_table = T.col_bound = None
         T.band_views = None
 
     def _column_work(self, items, item_begin, up):
@@ -1121,7 +1153,8 @@ class ShardBuild(object):
         torch, dev = _torch(), plan.dev
         n_part = max(T.n_items, 1) * (32 if self.tiled else 1)
         T.part_val = torch.empty(n_part, dtype=torch.float64, device=dev)
-        T.part_idx = torch.empty(n_part, dtype=torch.int32, device=dev)
+        # (-1: no choice yet; the column sweep starts each item from the choice of the previous sweep)
+        T.part_idx = torch.full((n_part,), -1, dtype=torch.int32, device=dev)
         T.J_out = torch.empty(max(n, 1), dtype=torch.float64, device=dev)
         T.argmin = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
         T.c_tables = fill_c_tables(T)
