@@ -265,7 +265,9 @@ const char* sdp_last_kernel(void);
  * evaluate every control, 0; the results are the same),
  * "col_prune_stats" (0|1: count the warp steps of the pruning sweep and those skipped, read and
  * reset by sdp_col_prune_counts; off by default, for measurements only),
- * "p2p_timeout_s" (bound of the peer-flag waits, default 600 s, then the kernel traps).
+ * "p2p_timeout_s" (bound of the peer-flag waits, default 600 s, then the kernel traps),
+ * "chain_threads" (sdp_chain_sample: threads per CTA, 32..1024 in multiples of 32; 0 = default,
+ * 256; the results do not depend on it).
  * Not thread-safe against concurrent launches. */
 int sdp_set_option(const char* name, int value);
 /* With "col_prune_stats" on: the warp steps (groups of col_ub controls of one item) that the
@@ -485,6 +487,48 @@ int sdp_forward_build(const SdpGrid* grid, int32_t W, int32_t g_per_w, const dou
  * and the residual), a one-CTA reduction of those partials. */
 int sdp_forward_steps(const SdpForwardOp* op, double* mu_a, double* mu_b, int32_t n_steps,
                       double* cost_out, double* resid_out, double* hist, double* scratch, void* stream);
+
+/* K1''' - sample paths of the chain of a fixed policy (Monte-Carlo trajectories).
+ * New feature, no reference counterpart as a kernel: the reference simulates the policy on the host
+ * (examples/20 .../storage_control.py:217,246).  The chain is the one of sdp_forward_*, sampled:
+ * from state x, draw node w with probability p_w (u in [0,1), t = u*cdf[W-1], w the first index
+ * with t < cdf[w], W-1 if none), then for every axis k draw v_k in [0,1) and take the upper corner
+ * when v_k < clamp(lam_k, 0, 1); the next state is cell + sum_k eps_k*M_k and the path's total
+ * gets acc = acc + g(x, w).  A transition with some lam_k outside [0,1] (an extrapolated next
+ * state, projected onto the grid box by the clamp) is counted as clamped; a NaN lam_k gives
+ * eps_k = 0 and counts the transition as NaN.
+ * Random numbers: Philox-4x32-10, key = seed (low word first), counter (path, step, call, 0),
+ * step the global step, call = 0, 1, 2 the calls of the step: 1 + d doubles, double j from words
+ * 2(j%2), 2(j%2)+1 of call j/2 as ((lo | hi << 32) >> 11) * 2^-53.  Initial states drawn from a
+ * CDF use step SDP_CHAIN_INIT_STEP.  A path's results depend only on (seed, path index, tables),
+ * not on the launch shape; the only atomics are integer counter sums. */
+#define SDP_CHAIN_INIT_STEP 0xFFFFFFFFu
+/* doubles per (x, w) record: [cell (int32 in the low word) | lam_0 .. lam_{d-1} | g | pad to even]:
+ * 32 bytes (one sector) for d <= 2, 48 for d = 3, 4 */
+#define SDP_CHAIN_REC(d) (2 * (((d) + 3) / 2))
+/* Pack the [w][n] policy-table planes (layout of sdp_policy_eval, g_per_w as there) into one record
+ * per (x, w), record e = w*n + x at rec + e*SDP_CHAIN_REC(d).  rec: device, 16-byte aligned,
+ * n*W*SDP_CHAIN_REC(d) doubles, owned by the caller. */
+int sdp_chain_pack(const SdpGrid* grid, int32_t W, int32_t g_per_w, const int32_t* cell, const double* lam,
+                   int64_t lam_plane, const double* g, int64_t n, double* rec, void* stream);
+/* Advance M paths by n_steps steps, global steps step0 .. step0 + n_steps - 1, one thread per path,
+ * the state in registers.  cdf: device [W], cumulative node probabilities (host np.cumsum).
+ * fresh != 0: paths start at global step step0 with total 0 and hit -1, from state[i] or, when
+ * start_cdf (device [n], cumulative, in C order) is given, from a state drawn with it (written to
+ * state[i]); fresh == 0: resume from state, total, hit as a previous launch left them.
+ * At every global step s in [step0, step0 + n_steps], before the transition out of s:
+ *   target (device bit mask, bit y%32 of word y/32, or NULL): hit[i] = s if hit[i] < 0 and the
+ *   state is in the target;  rec_steps (device [n_rec], strictly increasing, or NULL): when
+ *   s == rec_steps[j], rec_out[j*M + i] = the state.
+ * On return state / total / hit hold the state at step0 + n_steps, the summed stage costs and the
+ * first step in the target.  counters (device [2], accumulated, zeroed by the caller):
+ * counters[0] += clamped transitions, counters[1] += NaN transitions.  1 <= M < 2^31, n_steps >= 0,
+ * step0 + n_steps < 2^32 - 1. */
+int sdp_chain_sample(const SdpGrid* grid, int32_t W, const double* cdf, const double* rec, int64_t M,
+                     int32_t n_steps, int64_t step0, uint64_t seed, int32_t fresh, const double* start_cdf,
+                     const uint32_t* target, const int32_t* rec_steps, int32_t n_rec, int32_t* state,
+                     double* total, int32_t* hit, int32_t* rec_out, unsigned long long* counters,
+                     void* stream);
 
 /* K3 - argmin index -> control values, the `u_grids[i].flatten()[ind_opt[i]]` of
  * stodynprog.py:686-689 for every state at once.  lo/hi: device [n][nc] box

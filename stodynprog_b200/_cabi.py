@@ -109,6 +109,12 @@ class SdpForwardOp(ctypes.Structure):
 
 
 FWD_PIECE = 1024   # SDP_FWD_PIECE: entries per piece of a long row of the forward operator
+CHAIN_INIT_STEP = 0xFFFFFFFF   # SDP_CHAIN_INIT_STEP: Philox step word of the initial-state draws
+
+
+def chain_rec(d):
+    """SDP_CHAIN_REC: doubles per packed (x, w) record of sdp_chain_sample"""
+    return 2 * ((d + 3) // 2)
 
 
 # numpy mirrors of the per-state descriptor and the work item (host-built arrays
@@ -174,6 +180,9 @@ SIGNATURES = {
                                          ctypes.POINTER(SdpForwardOp), _vp, _i64, _vp]),
     "sdp_forward_steps": (ctypes.c_int, [ctypes.POINTER(SdpForwardOp), _vp, _vp, _i32, _vp, _vp, _vp, _vp,
                                          _vp]),
+    "sdp_chain_pack": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _i64, _vp, _i64, _vp, _vp]),
+    "sdp_chain_sample": (ctypes.c_int, [_gp, _i32, _vp, _vp, _i64, _i32, _i64, ctypes.c_uint64, _i32, _vp, _vp,
+                                        _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sdp_policy_values": (ctypes.c_int, [_i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sdp_sweep_finalize_cols": (ctypes.c_int, [ctypes.POINTER(SdpTables), _vp, _vp, _vp, _vp, _i64, _i64,
                                                _i32, _vp, _vp, _vp, _vp, _i32, _vp]),

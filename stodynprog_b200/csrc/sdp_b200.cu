@@ -1075,6 +1075,7 @@ struct Tuning {
     int pdl;           // programmatic dependent launch of pre-pass / column sweep / combine (1) or plain launches (0)
     int small_combine; // sdp_sweep_finalize_cols: the 128-thread combine that fits next to a streaming CTA (1) or the 1024-thread one (0)
     int carveout;      // layout CF: streaming kernel and small combine ask for the largest shared-memory carve-out (1) or leave it to the driver (0)
+    int chain_threads; // sdp_chain_sample: threads per CTA (0 = 256); the results do not depend on it
     int dbg_exchange;  // TIMING EXPERIMENTS ONLY (wrong results): 1 = no stores to remote ranks, 2 = no system fence, 4 = relaxed flag stores
 };
 static int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
@@ -1123,6 +1124,7 @@ static Tuning& tuning() {
         x.pdl = env_int("SDP_PDL", 1) != 0;
         x.small_combine = env_int("SDP_SMALL_COMBINE", 1) != 0;
         x.carveout = env_int("SDP_CARVEOUT", 1) != 0;
+        x.chain_threads = 0;
         return x;
     }();
     return t;
@@ -1151,6 +1153,7 @@ extern "C" int sdp_set_option(const char* name, int value) {
     else if (!strcmp(name, "dbg_exchange")) t.dbg_exchange = value;
     else if (!strcmp(name, "pdl")) t.pdl = value != 0;
     else if (!strcmp(name, "small_combine")) t.small_combine = value != 0;
+    else if (!strcmp(name, "chain_threads")) t.chain_threads = value ? clampi(value, 32, 1024) / 32 * 32 : 0;
     else return fail(SDP_EINVAL, "sdp_set_option: unknown option %s", name);
     return SDP_OK;
 }
@@ -3928,6 +3931,225 @@ extern "C" int sdp_forward_steps(const SdpForwardOp* op, double* mu_a, double* m
         in = out;
         out = const_cast<double*>(t);
     }
+    return SDP_OK;
+}
+
+// ---------------------------------------------------------------------------
+// K1''': sample paths of a fixed policy's chain (include/sdp_b200.h).  New feature: the
+// reference simulates the policy on the host (storage_control.py:217,246).  One thread per path,
+// its state in registers; a transition reads one packed (x, w) record, one 32-byte sector for
+// d <= 2.  Random numbers are counter-based (Philox-4x32-10), so a path's results depend only on
+// (seed, path, tables), not on the launch shape.
+// ---------------------------------------------------------------------------
+#define SDP_CHAIN_THREADS 256
+
+// Philox-4x32-10 (Salmon et al., SC'11; the Random123 reference): 10 rounds, key bumped between them
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+    for (int i = 0; i < 10; ++i) {
+        if (i) { k.x += 0x9E3779B9u; k.y += 0xBB67AE85u; }
+        const uint32_t hi0 = __umulhi(0xD2511F53u, c.x), lo0 = 0xD2511F53u * c.x;
+        const uint32_t hi1 = __umulhi(0xCD9E8D57u, c.z), lo1 = 0xCD9E8D57u * c.z;
+        c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+    }
+    return c;
+}
+
+// a double in [0, 1) from two words: the top 53 bits of (lo | hi << 32), exact
+__device__ __forceinline__ double chain_u01(uint32_t lo, uint32_t hi) {
+    return (double)((((uint64_t)hi << 32) | lo) >> 11) * 0x1p-53;
+}
+
+// first index j < len with t < C[j], len - 1 if none (C non-decreasing)
+__device__ __forceinline__ int chain_search(const double* C, int len, double t) {
+    int lo = 0, hi = len - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (t < C[mid]) hi = mid;
+        else lo = mid + 1;
+    }
+    return lo;
+}
+
+template <int D>
+__global__ void __launch_bounds__(256)
+k_chain_pack(int W, int g_per_w, int64_t n, const int32_t* __restrict__ cell, const double* __restrict__ lam,
+             int64_t lam_plane, const double* __restrict__ g, double* __restrict__ rec) {
+    constexpr int REC = SDP_CHAIN_REC(D);
+    const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (e >= n * W) return;
+    double r[REC];
+    r[0] = __longlong_as_double((long long)(uint32_t)cell[e]);
+#pragma unroll
+    for (int k = 0; k < D; ++k) r[1 + k] = lam[(int64_t)k * lam_plane + e];
+    r[1 + D] = g[g_per_w ? e : e % n];
+    if (REC > D + 2) r[REC - 1] = 0.0;
+    double2* out = reinterpret_cast<double2*>(rec + e * REC);
+#pragma unroll
+    for (int j = 0; j < REC / 2; ++j) out[j] = make_double2(r[2 * j], r[2 * j + 1]);
+}
+
+// one thread per path.  Per global step s: record, target test, then the transition out of s
+template <int D>
+__global__ void __launch_bounds__(1024)
+k_chain_sample(GridT<double> G, int W, const double* __restrict__ cdf, const double* __restrict__ rec, int64_t n,
+               int64_t M, int n_steps, uint32_t step0, uint2 key, int fresh, const double* __restrict__ start_cdf,
+               const uint32_t* __restrict__ target, const int32_t* __restrict__ rec_steps, int n_rec,
+               int32_t* __restrict__ state, double* __restrict__ total, int32_t* __restrict__ hit,
+               int32_t* __restrict__ rec_out, unsigned long long* __restrict__ counters) {
+    constexpr int REC = SDP_CHAIN_REC(D);
+    extern __shared__ double chain_cdf[];
+    __shared__ unsigned int chain_cnt[2];
+    for (int j = threadIdx.x; j < W; j += blockDim.x) chain_cdf[j] = cdf[j];
+    if (threadIdx.x < 2) chain_cnt[threadIdx.x] = 0u;
+    __syncthreads();
+    const double cmax = chain_cdf[W - 1];
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned int n_clamped = 0, n_nan = 0;
+    if (i < M) {
+        const uint32_t path = (uint32_t)i;
+        int x, h;
+        double acc;
+        if (fresh) {
+            acc = 0.0;
+            h = -1;
+            if (start_cdf) {
+                const uint4 r = philox4x32_10(make_uint4(path, SDP_CHAIN_INIT_STEP, 0u, 0u), key);
+                const double t = chain_u01(r.x, r.y) * __ldg(start_cdf + n - 1);
+                int lo = 0, hi = (int)n - 1;
+                while (lo < hi) {
+                    const int mid = (lo + hi) >> 1;
+                    if (t < __ldg(start_cdf + mid)) hi = mid;
+                    else lo = mid + 1;
+                }
+                x = lo;
+            } else {
+                x = state[i];
+            }
+        } else {
+            x = state[i];
+            acc = total[i];
+            h = hit[i];
+        }
+        int r = 0;
+        while (r < n_rec && (uint32_t)__ldg(rec_steps + r) < step0) ++r;
+#pragma unroll 1
+        for (int k = 0;; ++k) {
+            const uint32_t s = step0 + (uint32_t)k;
+            if (r < n_rec && (uint32_t)__ldg(rec_steps + r) == s) rec_out[(int64_t)r++ * M + i] = x;
+            if (target && h < 0 && ((__ldg(target + (x >> 5)) >> (x & 31)) & 1u)) h = (int)s;
+            if (k == n_steps) break;
+            const uint4 r0 = philox4x32_10(make_uint4(path, s, 0u, 0u), key);
+            const int w = chain_search(chain_cdf, W, chain_u01(r0.x, r0.y) * cmax);
+            const double2* R = reinterpret_cast<const double2*>(rec + ((int64_t)w * n + x) * REC);
+            double q[REC];
+#pragma unroll
+            for (int j = 0; j < REC / 2; ++j) {
+                const double2 t = __ldg(R + j);
+                q[2 * j] = t.x;
+                q[2 * j + 1] = t.y;
+            }
+            double v[D];
+            v[0] = chain_u01(r0.z, r0.w);
+            if (D >= 2) {
+                const uint4 r1 = philox4x32_10(make_uint4(path, s, 1u, 0u), key);
+                v[1 % D] = chain_u01(r1.x, r1.y);
+                if (D >= 3) v[2 % D] = chain_u01(r1.z, r1.w);
+            }
+            if (D >= 4) {
+                const uint4 r2 = philox4x32_10(make_uint4(path, s, 2u, 0u), key);
+                v[3 % D] = chain_u01(r2.x, r2.y);
+            }
+            int y = (int)(uint32_t)__double_as_longlong(q[0]);
+            bool clamped = false, nan = false;
+#pragma unroll
+            for (int kk = 0; kk < D; ++kk) {
+                double l = q[1 + kk];
+                if (l != l) {
+                    nan = true;
+                    continue;
+                }
+                if (l < 0.0) { l = 0.0; clamped = true; }
+                else if (l > 1.0) { l = 1.0; clamped = true; }
+                if (v[kk] < l) y += G.stride[kk];
+            }
+            acc = add_(acc, q[1 + D]);
+            n_clamped += clamped;
+            n_nan += nan;
+            x = y;
+        }
+        state[i] = x;
+        total[i] = acc;
+        hit[i] = h;
+    }
+    n_clamped = __reduce_add_sync(0xffffffffu, n_clamped);
+    n_nan = __reduce_add_sync(0xffffffffu, n_nan);
+    if ((threadIdx.x & 31) == 0 && (n_clamped | n_nan)) {
+        atomicAdd(chain_cnt, n_clamped);
+        atomicAdd(chain_cnt + 1, n_nan);
+    }
+    __syncthreads();
+    if (threadIdx.x == 0 && (chain_cnt[0] | chain_cnt[1])) {
+        atomicAdd(counters, (unsigned long long)chain_cnt[0]);
+        atomicAdd(counters + 1, (unsigned long long)chain_cnt[1]);
+    }
+}
+
+extern "C" int sdp_chain_pack(const SdpGrid* grid, int32_t W, int32_t g_per_w, const int32_t* cell,
+                              const double* lam, int64_t lam_plane, const double* g, int64_t n, double* rec,
+                              void* stream) {
+    GridT<double> G;
+    int64_t ng = 0;
+    int rc = make_grid<double>(grid, &G, &ng);
+    if (rc) return rc;
+    if (W < 1 || n != ng || lam_plane < W * n || n * W >= (int64_t)INT_MAX)
+        return fail(SDP_EINVAL, "%s", "sdp_chain_pack: bad sizes");
+    if (!cell || !lam || !g || !rec) return fail(SDP_EINVAL, "%s", "sdp_chain_pack: NULL pointer");
+    if (((uintptr_t)rec) & 15) return fail(SDP_EINVAL, "%s", "sdp_chain_pack: rec not 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned b = (unsigned)((n * W + 255) / 256);
+    switch (grid->d) {
+        case 1: k_chain_pack<1><<<b, 256, 0, st>>>(W, g_per_w, n, cell, lam, lam_plane, g, rec); break;
+        case 2: k_chain_pack<2><<<b, 256, 0, st>>>(W, g_per_w, n, cell, lam, lam_plane, g, rec); break;
+        case 3: k_chain_pack<3><<<b, 256, 0, st>>>(W, g_per_w, n, cell, lam, lam_plane, g, rec); break;
+        default: k_chain_pack<4><<<b, 256, 0, st>>>(W, g_per_w, n, cell, lam, lam_plane, g, rec); break;
+    }
+    SDP_LAUNCH_CHECK();
+    return SDP_OK;
+}
+
+extern "C" int sdp_chain_sample(const SdpGrid* grid, int32_t W, const double* cdf, const double* rec, int64_t M,
+                                int32_t n_steps, int64_t step0, uint64_t seed, int32_t fresh,
+                                const double* start_cdf, const uint32_t* target, const int32_t* rec_steps,
+                                int32_t n_rec, int32_t* state, double* total, int32_t* hit, int32_t* rec_out,
+                                unsigned long long* counters, void* stream) {
+    GridT<double> G;
+    int64_t n = 0;
+    int rc = make_grid<double>(grid, &G, &n);
+    if (rc) return rc;
+    if (W < 1 || M < 1 || M >= ((int64_t)1 << 31) || n_steps < 0 || step0 < 0 || n_rec < 0 ||
+        step0 + n_steps >= (int64_t)SDP_CHAIN_INIT_STEP || n * W >= (int64_t)INT_MAX)
+        return fail(SDP_EINVAL, "%s", "sdp_chain_sample: bad sizes");
+    if ((size_t)W * 8 > 48 * 1024) return fail(SDP_EINVAL, "%s", "sdp_chain_sample: W > 6144 nodes");
+    if (!cdf || !rec || !state || !total || !hit || !counters || (n_rec && (!rec_steps || !rec_out)))
+        return fail(SDP_EINVAL, "%s", "sdp_chain_sample: NULL pointer");
+    if (((uintptr_t)rec) & 15) return fail(SDP_EINVAL, "%s", "sdp_chain_sample: rec not 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    const int threads = tuning().chain_threads ? tuning().chain_threads : SDP_CHAIN_THREADS;
+    const unsigned blocks = (unsigned)((M + threads - 1) / threads);
+    const size_t shm = (size_t)W * 8;
+    const uint2 key = make_uint2((uint32_t)seed, (uint32_t)(seed >> 32));
+#define SDP_CHAIN_ARGS G, W, cdf, rec, n, M, n_steps, (uint32_t)step0, key, fresh, fresh ? start_cdf : nullptr, \
+        target, rec_steps, n_rec, state, total, hit, rec_out, counters
+    switch (grid->d) {
+        case 1: k_chain_sample<1><<<blocks, threads, shm, st>>>(SDP_CHAIN_ARGS); break;
+        case 2: k_chain_sample<2><<<blocks, threads, shm, st>>>(SDP_CHAIN_ARGS); break;
+        case 3: k_chain_sample<3><<<blocks, threads, shm, st>>>(SDP_CHAIN_ARGS); break;
+        default: k_chain_sample<4><<<blocks, threads, shm, st>>>(SDP_CHAIN_ARGS); break;
+    }
+#undef SDP_CHAIN_ARGS
+    SDP_LAUNCH_CHECK();
+    note_kernel("k_chain_sample<D=%d>, %d threads", grid->d, threads);
     return SDP_OK;
 }
 

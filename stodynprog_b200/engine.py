@@ -240,6 +240,17 @@ class PolicyTables(object):
         self.bounds = None
 
 
+class ChainTables(object):
+    """The path sampler's tables of a fixed policy (sdp_chain_*): packed (x, w) records, device
+    fp64 [n*W*chain_rec(d)], and the cumulative node probabilities, device fp64 [W]."""
+
+    def __init__(self):
+        self.grid = None
+        self.W = 1
+        self.n = 0
+        self.rec = self.cdf = None
+
+
 class Engine(object):
     """Owns the device, the stream, the process group and the launches."""
 
@@ -1607,6 +1618,39 @@ class Engine(object):
                 converged = True
                 break
         return mu_a, done, residuals, converged
+
+    # -- sample paths (Monte-Carlo trajectories) -------------------------
+    def chain_tables(self, P):
+        """The sampler's view of the policy tables `P` (sdp_chain_pack): one packed record per
+        (x, w) and the cumulative node probabilities.  One rank only."""
+        torch = _torch()
+        if self.coll.world > 1 or P.n_states != int(np.prod(P.grid.order[:P.grid.d])):
+            raise NotImplementedError(
+                "path sampling runs on one rank: a path leaves the slab of its rank (not implemented)")
+        n, d = P.n_states, P.grid.d
+        C = ChainTables()
+        C.grid, C.W, C.n = P.grid, P.W, n
+        C.rec = torch.empty(n * P.W * _cabi.chain_rec(d), dtype=torch.float64, device=self.device)
+        rc = self.lib.sdp_chain_pack(ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.cell), self._ptr(P.lam),
+                                     P.lam_plane, self._ptr(P.g), n, self._ptr(C.rec), self.stream)
+        _cabi.check(rc, "sdp_chain_pack")
+        C.cdf = self.to_device(np.cumsum(P.p.cpu().numpy()))
+        return C
+
+    def chain_sample(self, C, state, total, hit, n_steps, step0, seed, fresh, counters, start_cdf=None,
+                     target=None, rec_steps=None, rec_out=None):
+        """Advance the paths (device state int32 / total fp64 / hit int32 [M]) by n_steps steps from
+        global step step0 (sdp_chain_sample).  fresh: start at step0 from `state`, or from a state
+        drawn with `start_cdf`; otherwise resume.  target: device uint32 bit mask; rec_steps: device
+        int32 (increasing), rec_out [len(rec_steps) * M]; counters: device uint64 [2] (clamped, NaN
+        transitions), accumulated."""
+        n_rec = 0 if rec_steps is None else int(rec_steps.numel())
+        rc = self.lib.sdp_chain_sample(ctypes.byref(C.grid), C.W, self._ptr(C.cdf), self._ptr(C.rec),
+                                       int(state.numel()), int(n_steps), int(step0), int(seed), 1 if fresh else 0,
+                                       self._ptr(start_cdf), self._ptr(target), self._ptr(rec_steps), n_rec,
+                                       self._ptr(state), self._ptr(total), self._ptr(hit), self._ptr(rec_out),
+                                       self._ptr(counters), self.stream)
+        _cabi.check(rc, "sdp_chain_sample")
 
     # -- interpolation ----------------------------------------------------
     def interp(self, grid, values, s):

@@ -676,6 +676,141 @@ class DPSolver(object):
             print('\rstationary distribution run in {:.2f} s ({:d} steps)'.format(exec_time, n_done))
         return pi, info
 
+    def _check_start(self, start, n_paths):
+        """(flat start indices int32 [n_paths], None) or (None, C-order CDF of the start distribution)"""
+        state_dims = self._state_grid_shape
+        n = int(np.prod(state_dims))
+        if isinstance(start, tuple):
+            if len(start) != len(state_dims) or not all(isinstance(i, (int, np.integer)) for i in start) or \
+                    not all(0 <= i < m for i, m in zip(start, state_dims)):
+                raise ValueError('`start` as a tuple should be a multi-index of the state grid of shape {:s}, '
+                                 'not {:s}'.format(str(state_dims), str(start)))
+            return np.full(n_paths, np.ravel_multi_index(start, state_dims), dtype=np.int32), None
+        start = np.asarray(start)
+        if np.issubdtype(start.dtype, np.integer):
+            self._check_shape('start', start, (n_paths,))
+            if start.size and (start.min() < 0 or start.max() >= n):
+                raise ValueError('flat indices in `start` must lie in [0, {:d})'.format(n))
+            return start.astype(np.int32), None
+        if not np.issubdtype(start.dtype, np.floating):
+            raise ValueError('`start` should be a multi-index (tuple), an integer array of flat indices or '
+                             'a distribution (float array)')
+        self._check_shape('start', start, state_dims)
+        if not np.all(np.isfinite(start)) or np.any(start < 0) or not start.sum() > 0:
+            raise ValueError('the start distribution must be finite, non-negative and not all zero')
+        return None, np.cumsum(start.reshape(-1).astype(float))
+
+    def _chain_tables(self, pol, t_k=None):
+        eng = self.engine
+        P = eng.build_policy_tables(self, np.asarray(pol, dtype=float), t_k=t_k, deterministic=True)
+        return eng.chain_tables(P)
+
+    def sample_paths(self, pol, start, n_steps, n_paths, seed=0, target=None, record=(), report_time=True):
+        """sample `n_paths` paths of `n_steps` steps of the chain of the policy `pol` (Monte-Carlo
+        trajectories on the GPU, one thread per path).  Not in the reference as such: its
+        examples simulate the policy on the host.
+
+        The chain is the one of propagate_distribution, sampled: from state x a perturbation node
+        w is drawn with its probability, then the next state's cell corner along every axis k is
+        the upper one with probability lambda_k, the interpolation weight; the stage cost
+        g(x, pol(x), w) is added to the path's total.  Where a next state lies outside the grid
+        box, lambda_k is outside [0, 1] and is clamped to it (a probability cannot be negative):
+        the sample projects that next state onto the grid box.  Such transitions are counted
+        (info['clamped_share']); with none, the sampled chain is exactly the chain J is computed
+        with.  A NaN weight takes the lower corner and is counted in info['nan_transitions'].
+
+        Random numbers are Philox-4x32-10 keyed by `seed`, counter (path, step, call): a path's
+        results depend only on (seed, path index, policy), and are bit-identical run to run.
+
+        pol: state_dims + (nb_control,) for a stationary system; (T,) + state_dims + (nb_control,)
+            as returned by bellman_recursion for a time-dependent one (step k applies pol[k] at
+            instant k, n_steps <= T).
+        start: a tuple, the multi-index every path starts from; an integer array of n_paths flat
+            C-order indices; or a float array of shape state_dims, non-negative, the (not
+            necessarily normalised) distribution the initial states are drawn from.
+        target: boolean array of shape state_dims, or None.
+        record: steps in [0, n_steps] at which the states are returned.
+
+        Returns (total_cost [n_paths], info) with info = {'hit_step' [n_paths]: first step (0 ..
+        n_steps) at which the path is in `target`, -1 if never; 'states' [len(record), n_paths]:
+        flat indices of the states at the recorded steps; 'final_state' [n_paths]; 'clamped_share';
+        'nan_transitions'; 'n_paths'; 'n_steps'; 'seed'}.
+        """
+        import torch
+        t_start = datetime.now()
+        state_dims = self._state_grid_shape
+        nb_control = len(self.sys.control)
+        pol = np.asarray(pol)
+        if self.sys.stationnary:
+            self._check_shape('pol', pol, state_dims + (nb_control,))
+        else:
+            T = pol.shape[0] if pol.ndim == len(state_dims) + 2 else 0
+            self._check_shape('pol', pol, (max(T, 1),) + state_dims + (nb_control,))
+        n_steps, n_paths, seed = int(n_steps), int(n_paths), int(seed)
+        if n_steps < 0:
+            raise ValueError('n_steps must be >= 0')
+        if not self.sys.stationnary and n_steps > T:
+            raise ValueError('n_steps = {:d} exceeds the horizon of `pol` ({:d} instants)'.format(n_steps, T))
+        if not 1 <= n_paths < 2 ** 31:
+            raise ValueError('n_paths must be in [1, 2**31), not {:d}'.format(n_paths))
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError('seed must be in [0, 2**64)')
+        start_idx, start_cdf = self._check_start(start, n_paths)
+        if target is not None:
+            target = np.asarray(target)
+            self._check_shape('target', target, state_dims)
+            if target.dtype != bool:
+                raise ValueError('`target` must be a boolean array')
+        record = np.asarray(record)
+        if record.size and not np.issubdtype(record.dtype, np.integer):
+            raise ValueError('`record` must hold integer steps')
+        record = record.astype(np.int64).reshape(-1)
+        if np.any((record < 0) | (record > n_steps)):
+            raise ValueError('`record` steps must lie in [0, n_steps] = [0, {:d}]'.format(n_steps))
+        rec_steps, rec_inv = np.unique(record, return_inverse=True)
+        if report_time:
+            print('path sampling...', end='')
+        eng = self.engine
+        dev = eng.device
+        M = n_paths
+        state = eng.to_device(start_idx) if start_idx is not None else \
+            torch.empty(M, dtype=torch.int32, device=dev)
+        total = torch.empty(M, dtype=torch.float64, device=dev)
+        hit = torch.empty(M, dtype=torch.int32, device=dev)
+        counters = torch.zeros(2, dtype=torch.int64, device=dev)
+        kw = {"start_cdf": eng.to_device(start_cdf) if start_cdf is not None else None,
+              "target": eng.to_device(self._target_mask(target)) if target is not None else None,
+              "rec_steps": eng.to_device(rec_steps.astype(np.int32)) if rec_steps.size else None,
+              "rec_out": torch.empty(rec_steps.size * M, dtype=torch.int32, device=dev) if rec_steps.size else None}
+        if self.sys.stationnary:
+            C = self._chain_tables(pol)
+            eng.chain_sample(C, state, total, hit, n_steps, 0, seed, True, counters, **kw)
+        else:
+            # the chain changes with the instant: tables rebuilt per step, the paths resume on the
+            # device with the global step in the random counter
+            for k in range(max(n_steps, 1)):
+                C = self._chain_tables(pol[k], t_k=k)
+                eng.chain_sample(C, state, total, hit, min(n_steps, 1), k, seed, k == 0, counters, **kw)
+                del C
+        outs = [total, hit, state, counters] + ([kw["rec_out"]] if rec_steps.size else [])
+        host = eng.to_host(*outs)
+        total_h, hit_h, final_h, cnt = host[:4]
+        states = host[4].reshape(rec_steps.size, M)[rec_inv] if rec_steps.size else np.zeros((0, M), np.int32)
+        info = {'hit_step': hit_h, 'states': states, 'final_state': final_h,
+                'clamped_share': float(cnt[0]) / (M * n_steps) if n_steps else 0.0,
+                'nan_transitions': int(cnt[1]), 'n_paths': M, 'n_steps': n_steps, 'seed': seed}
+        exec_time = (datetime.now() - t_start).total_seconds()
+        if report_time:
+            print('\rpath sampling run in {:.2f} s ({:d} paths x {:d} steps)'.format(exec_time, M, n_steps))
+        return total_h, info
+
+    @staticmethod
+    def _target_mask(target):
+        """boolean state_dims array -> 32-bit words, bit y % 32 of word y // 32 = target[y] (C order)"""
+        bits = np.packbits(target.reshape(-1), bitorder='little')
+        bits = np.concatenate([bits, np.zeros(-bits.size % 4, np.uint8)])
+        return bits.view('<i4').astype(np.int32)      # the same bits; torch copies int32
+
     # ------------------------------------------------------------------
     def print_summary(self):
         """summary of the discretisation (reference stodynprog.py:814-875)"""
