@@ -523,7 +523,9 @@ int sdp_chain_pack(const SdpGrid* grid, int32_t W, int32_t g_per_w, const int32_
  * On return state / total / hit hold the state at step0 + n_steps, the summed stage costs and the
  * first step in the target.  counters (device [2], accumulated, zeroed by the caller):
  * counters[0] += clamped transitions, counters[1] += NaN transitions.  1 <= M < 2^31, n_steps >= 0,
- * step0 + n_steps < 2^32 - 1. */
+ * step0 + n_steps < 2^32 - 1.  The node CDF (8 W bytes) is the launch's dynamic shared memory; with
+ * the kernel's static shared memory it must fit the 48 KB a launch gets without an opt-in, which
+ * bounds W a little below 6144 (the bound is in the SDP_EINVAL message). */
 int sdp_chain_sample(const SdpGrid* grid, int32_t W, const double* cdf, const double* rec, int64_t M,
                      int32_t n_steps, int64_t step0, uint64_t seed, int32_t fresh, const double* start_cdf,
                      const uint32_t* target, const int32_t* rec_steps, int32_t n_rec, int32_t* state,

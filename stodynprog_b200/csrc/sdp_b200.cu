@@ -4130,7 +4130,18 @@ extern "C" int sdp_chain_sample(const SdpGrid* grid, int32_t W, const double* cd
     if (W < 1 || M < 1 || M >= ((int64_t)1 << 31) || n_steps < 0 || step0 < 0 || n_rec < 0 ||
         step0 + n_steps >= (int64_t)SDP_CHAIN_INIT_STEP || n * W >= (int64_t)INT_MAX)
         return fail(SDP_EINVAL, "%s", "sdp_chain_sample: bad sizes");
-    if ((size_t)W * 8 > 48 * 1024) return fail(SDP_EINVAL, "%s", "sdp_chain_sample: W > 6144 nodes");
+    // the node CDF is the dynamic shared memory of the launch: without an opt-in, the kernel's
+    // static shared memory (chain_cnt and what the toolchain reserves) and the CDF share 48 KB
+    const void* fn = grid->d == 1 ? (const void*)k_chain_sample<1> : grid->d == 2 ? (const void*)k_chain_sample<2>
+                   : grid->d == 3 ? (const void*)k_chain_sample<3> : (const void*)k_chain_sample<4>;
+    cudaFuncAttributes fa;
+    SDP_CUDA_CHECK(cudaFuncGetAttributes(&fa, fn));
+    if ((size_t)W * 8 > (size_t)fa.maxDynamicSharedSizeBytes) {
+        char msg[160];
+        snprintf(msg, sizeof(msg), "sdp_chain_sample: W > %d nodes (%d bytes of dynamic shared memory)",
+                 fa.maxDynamicSharedSizeBytes / 8, fa.maxDynamicSharedSizeBytes);
+        return fail(SDP_EINVAL, "%s", msg);
+    }
     if (!cdf || !rec || !state || !total || !hit || !counters || (n_rec && (!rec_steps || !rec_out)))
         return fail(SDP_EINVAL, "%s", "sdp_chain_sample: NULL pointer");
     if (((uintptr_t)rec) & 15) return fail(SDP_EINVAL, "%s", "sdp_chain_sample: rec not 16-byte aligned");

@@ -132,7 +132,8 @@ def cuda_api(product):
 # oracle: P as a scipy.sparse matrix, built from dyn/cost and the oracle's cell search
 # ---------------------------------------------------------------------------
 def oracle_chain(solver, pol, t_k=None):
-    """(P [N x N] csr, g_bar [N]) of the policy `pol` (state_dims + (nc,)) at instant t_k"""
+    """(P [N x N] csr, g_bar [N]) of the policy `pol` (state_dims + (nc,)) at instant t_k; the
+    perturbation nodes are those of the product of all the perturbation grids"""
     sys = solver.sys
     grids = [np.asarray(g, dtype=float) for g in solver.state_grid]
     dims = tuple(len(g) for g in grids)
@@ -140,8 +141,12 @@ def oracle_chain(solver, pol, t_k=None):
     mesh = [m.reshape(n, 1) for m in np.meshgrid(*grids, indexing="ij")]
     u = [pol[..., i].reshape(n, 1) for i in range(pol.shape[-1])]
     if len(solver.perturb_grid):
-        w_args = (np.asarray(solver.perturb_grid[0], dtype=float).reshape(1, -1),)
-        p = np.asarray(solver.perturb_proba[0], dtype=float)
+        # several perturbations: the C-order product of their grids, each passed as a flat (1, W)
+        # row, with the products of the marginal probabilities as the joint law
+        ws = np.meshgrid(*[np.asarray(g, dtype=float) for g in solver.perturb_grid], indexing="ij")
+        ps = np.meshgrid(*[np.asarray(q, dtype=float) for q in solver.perturb_proba], indexing="ij")
+        w_args = tuple(w.reshape(1, -1) for w in ws)
+        p = np.prod(ps, axis=0).reshape(-1)
     else:
         w_args, p = (), np.ones(1)
     W = len(p)

@@ -408,10 +408,10 @@ def test_searev_small_golden(api):
 # ---------------------------------------------------------------------------
 # semantics: ties, NaN, deterministic branch, w-dependent cost, 4-D state
 # ---------------------------------------------------------------------------
-def _toy(api, d=1, cost_kind="plain", n_u=37, **kw):
-    """small synthetic system exercising the generic paths"""
+def _toy(api, d=1, cost_kind="plain", n_u=37, n_w=5, **kw):
+    """small synthetic system exercising the generic paths; n_w perturbation nodes on
+    [-0.9, 0.9], or none (a deterministic system) with n_w = 0"""
     import scipy.stats as stats
-    n_w = 5
 
     def dyn(*a):
         x, (u, w) = a[:d], a[d:]
@@ -433,23 +433,26 @@ def _toy(api, d=1, cost_kind="plain", n_u=37, **kw):
         return base
 
     names = ['x%d' % i for i in range(d)]
-    src = "def dyn_f({0}, u, w): return dyn({0}, u, w)\n" \
-          "def cost_f({0}, u, w): return cost({0}, u, w)\n" \
-          "def box_f({0}): return box({0})\n".format(', '.join(names))
+    w_arg, w_val = (", w", "w") if n_w else ("", "0.0")
+    src = "def dyn_f({0}, u{1}): return dyn({0}, u, {2})\n" \
+          "def cost_f({0}, u{1}): return cost({0}, u, {2})\n" \
+          "def box_f({0}): return box({0})\n".format(', '.join(names), w_arg, w_val)
     ns = {'dyn': dyn, 'cost': cost, 'box': box}
     exec(src, ns)
-    sys = api.SysDescription((d, 1, 1), name='toy%d' % d)
+    sys = api.SysDescription((d, 1, 1 if n_w else 0), name='toy%d' % d)
     sys.dyn = ns['dyn_f']
     sys.control_box = ns['box_f']
     sys.cost = ns['cost_f']
-    sys.perturb_laws = [stats.norm(0, 0.3)]
+    if n_w:
+        sys.perturb_laws = [stats.norm(0, 0.3)]
     sv = api.DPSolver(sys, **kw)
     sizes = [6, 5, 4, 3][:d]
     args = []
     for n in sizes:
         args += [-1.0, 2.0, n]
     sv.discretize_state(*args)
-    sv.discretize_perturb(-0.9, 0.9, n_w)
+    if n_w:
+        sv.discretize_perturb(-0.9, 0.9, n_w)
     sv.control_steps = (2.0 / n_u,)
     return sv
 
