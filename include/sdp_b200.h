@@ -267,6 +267,8 @@ const char* sdp_last_kernel(void);
  * reset by sdp_col_prune_counts; off by default, for measurements only),
  * "p2p_timeout_s" (bound of the peer-flag waits, default 600 s, then the kernel traps),
  * "chain_threads" (sdp_chain_sample: threads per CTA, 32..1024 in multiples of 32; 0 = default,
+ * 256; the results do not depend on it),
+ * "fp_threads" (sdp_first_passage: threads per CTA, 32..1024 in multiples of 32; 0 = default,
  * 256; the results do not depend on it).
  * Not thread-safe against concurrent launches. */
 int sdp_set_option(const char* name, int value);
@@ -531,6 +533,35 @@ int sdp_chain_sample(const SdpGrid* grid, int32_t W, const double* cdf, const do
                      const uint32_t* target, const int32_t* rec_steps, int32_t n_rec, int32_t* state,
                      double* total, int32_t* hit, int32_t* rec_out, unsigned long long* counters,
                      void* stream);
+
+/* K1'''' - first-passage analysis of the chain of a fixed policy: for a target set, the
+ * probability of reaching it, and the expected steps and stage cost before reaching it, from every
+ * state.  New feature, no reference counterpart.  A backward recursion over the policy tables of
+ * sdp_policy_eval (same [w][n] planes: cell, lam, g, p, g_per_w as there), one thread per state,
+ * three value functions carried together.  On a target state (bit y%32 of word y/32 of `target`,
+ * device) a step writes (P, S, C) = (1, 0, 0) without reading its table entries; elsewhere,
+ * with the nested lerp I[.] of every other kernel at the next state of each node w in order:
+ *   P = acc + I[P]*p_w                 (acc from 0, then P = acc)
+ *   S = 1 + (acc + I[S]*p_w)           (the 1 added after the loop)
+ *   C = acc + (g + I[C])*p_w           (exactly the fixed-policy backup of sdp_policy_eval)
+ * clamp != 0: every weight lam_k is first replaced by (lam_k < 0 || isnan(lam_k) ? 0 :
+ * (lam_k > 1 ? 1 : lam_k)), the chain sdp_chain_sample samples; clamp == 0: the weights are
+ * used as they are, the chain J is computed with.
+ * Values are records of 4 doubles per state, (P, S, C, 0): a corner gather reads one 32-byte
+ * sector.  V_a (the values at the step the call starts from) / V_b: device [n][4], 16-byte
+ * aligned, ping-pong; on return the values after n_steps steps are in V_a if n_steps is even,
+ * V_b if odd.  The recursion starts from (1_target, 0, 0).
+ * hist (device [(n_steps+1)][n][4], or NULL): entry j = the values after j steps of the call
+ * (entry 0 = V_a).  resid_out (device [1], or NULL): max over the states and the three values of
+ * |new - old| in the last step (0 when n_steps == 0); any NaN makes it NaN.  counters (device
+ * uint64 [1], or NULL, accumulated): += the number of (x, w) entries of non-target states with a
+ * weight outside [0, 1] or NaN, counted once per call (in its first step).  n_states must be the
+ * whole grid (one rank).  The only atomics are integer ones: results are bit-identical run to
+ * run, whatever the launch shape and however the steps are split over calls. */
+int sdp_first_passage(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p, const int32_t* cell,
+                      const double* lam, int64_t lam_plane, const double* g, int64_t n_states,
+                      const uint32_t* target, int32_t clamp, double* V_a, double* V_b, int32_t n_steps,
+                      double* hist, double* resid_out, unsigned long long* counters, void* stream);
 
 /* K3 - argmin index -> control values, the `u_grids[i].flatten()[ind_opt[i]]` of
  * stodynprog.py:686-689 for every state at once.  lo/hi: device [n][nc] box

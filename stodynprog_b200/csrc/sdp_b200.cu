@@ -6,8 +6,9 @@
 //   * the per-state backup _value_at_state_vect (stodynprog/stodynprog.py:639-691)
 //     looped over the state grid by value_iteration (:511-515)
 //   * the policy-evaluation iteration of eval_policy (:743-763)
-// and adds the forward (transposed) application of a fixed policy's chain, which the
-// reference has no counterpart for (K1'', distribution propagation).
+// and adds, with no reference counterpart, the forward (transposed) application of a fixed
+// policy's chain (K1'', distribution propagation), path sampling (K1''') and the first-passage
+// recursion to a target set (K1'''').
 //
 // This is a gather-reduce, not a contraction: no tensor cores.  The sweep kernel
 // streams the dense (cell, lambda, g) tables once from HBM with 128-bit
@@ -1076,6 +1077,7 @@ struct Tuning {
     int small_combine; // sdp_sweep_finalize_cols: the 128-thread combine that fits next to a streaming CTA (1) or the 1024-thread one (0)
     int carveout;      // layout CF: streaming kernel and small combine ask for the largest shared-memory carve-out (1) or leave it to the driver (0)
     int chain_threads; // sdp_chain_sample: threads per CTA (0 = 256); the results do not depend on it
+    int fp_threads;    // sdp_first_passage: threads per CTA (0 = 256); the results do not depend on it
     int dbg_exchange;  // TIMING EXPERIMENTS ONLY (wrong results): 1 = no stores to remote ranks, 2 = no system fence, 4 = relaxed flag stores
 };
 static int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
@@ -1125,6 +1127,7 @@ static Tuning& tuning() {
         x.small_combine = env_int("SDP_SMALL_COMBINE", 1) != 0;
         x.carveout = env_int("SDP_CARVEOUT", 1) != 0;
         x.chain_threads = 0;
+        x.fp_threads = 0;
         return x;
     }();
     return t;
@@ -1154,6 +1157,7 @@ extern "C" int sdp_set_option(const char* name, int value) {
     else if (!strcmp(name, "pdl")) t.pdl = value != 0;
     else if (!strcmp(name, "small_combine")) t.small_combine = value != 0;
     else if (!strcmp(name, "chain_threads")) t.chain_threads = value ? clampi(value, 32, 1024) / 32 * 32 : 0;
+    else if (!strcmp(name, "fp_threads")) t.fp_threads = value ? clampi(value, 32, 1024) / 32 * 32 : 0;
     else return fail(SDP_EINVAL, "sdp_set_option: unknown option %s", name);
     return SDP_OK;
 }
@@ -4161,6 +4165,163 @@ extern "C" int sdp_chain_sample(const SdpGrid* grid, int32_t W, const double* cd
 #undef SDP_CHAIN_ARGS
     SDP_LAUNCH_CHECK();
     note_kernel("k_chain_sample<D=%d>, %d threads", grid->d, threads);
+    return SDP_OK;
+}
+
+// ---------------------------------------------------------------------------
+// K1'''': first-passage analysis of a fixed policy's chain (include/sdp_b200.h).  New feature.
+// The one-thread-per-state pass of k_policy_eval over the same [w][n] planes, with a target
+// mask, optionally clamped weights and three value functions (P, S, C) in one 32-byte record
+// per state, so that a corner gather fetches all three in one sector.
+// ---------------------------------------------------------------------------
+#define SDP_FP_THREADS 256
+
+// the nested lerp of Lerp<double, D, K> applied to the three values of the records
+template <int D, int K>
+struct Lerp3 {
+    __device__ __forceinline__ static void eval(const double* __restrict__ V, int base, const int (&stride)[SDP_MAX_D],
+                                                const double (&lam)[D], double& P, double& S, double& C) {
+        double aP, aS, aC, bP, bS, bC;
+        Lerp3<D, K + 1>::eval(V, base, stride, lam, aP, aS, aC);
+        Lerp3<D, K + 1>::eval(V, base + (K == D - 1 ? 1 : stride[K]), stride, lam, bP, bS, bC);
+        const double l = lam[K], m = sub_(1.0, l);
+        P = add_(mul_(m, aP), mul_(l, bP));
+        S = add_(mul_(m, aS), mul_(l, bS));
+        C = add_(mul_(m, aC), mul_(l, bC));
+    }
+};
+template <int D>
+struct Lerp3<D, D> {
+    __device__ __forceinline__ static void eval(const double* __restrict__ V, int base, const int (&)[SDP_MAX_D],
+                                                const double (&)[D], double& P, double& S, double& C) {
+        const double2* r = reinterpret_cast<const double2*>(V + 4 * (int64_t)base);
+        const double2 a = __ldg(r), b = __ldg(r + 1);
+        P = a.x;
+        S = a.y;
+        C = b.x;
+    }
+};
+
+// non-negative doubles (and NaN with the sign bit cleared, above +inf) order like their bits
+__device__ __forceinline__ unsigned long long fp_absdiff_bits(double a, double b) {
+    return (unsigned long long)__double_as_longlong(fabs(sub_(a, b)));
+}
+
+template <int D, bool CLAMP>
+__global__ void __launch_bounds__(1024)
+k_first_passage(GridT<double> G, int W, int g_per_w, const double* __restrict__ p, const int32_t* __restrict__ cell,
+                const double* __restrict__ lam, int64_t lam_plane, const double* __restrict__ g, int64_t n,
+                const uint32_t* __restrict__ target, const double* __restrict__ V_in, double* __restrict__ V_out,
+                double* __restrict__ hist_out, unsigned long long* __restrict__ outside,
+                unsigned long long* __restrict__ resid) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned int n_out = 0;
+    unsigned long long r = 0;
+    if (i < n) {
+        double P = 1.0, S = 0.0, C = 0.0;
+        if (!((__ldg(target + (i >> 5)) >> (i & 31)) & 1u)) {
+            double aP = 0.0, aS = 0.0, aC = 0.0;
+            double gv = g_per_w ? 0.0 : g[i];
+            for (int w = 0; w < W; ++w) {
+                const int64_t off = (int64_t)w * n + i;
+                double l[D];
+                bool out = false;
+#pragma unroll
+                for (int k = 0; k < D; ++k) {
+                    double lk = lam[(int64_t)k * lam_plane + off];
+                    out |= !(lk >= 0.0 && lk <= 1.0);
+                    if (CLAMP) lk = (lk < 0.0 || isnan(lk)) ? 0.0 : (lk > 1.0 ? 1.0 : lk);
+                    l[k] = lk;
+                }
+                if (g_per_w) gv = g[off];
+                double vP, vS, vC;
+                Lerp3<D, 0>::eval(V_in, cell[off], G.stride, l, vP, vS, vC);
+                const double pw = p[w];
+                aP = add_(aP, mul_(vP, pw));
+                aS = add_(aS, mul_(vS, pw));
+                aC = add_(aC, mul_(add_(gv, vC), pw));
+                n_out += out;
+            }
+            P = aP;
+            S = add_(1.0, aS);
+            C = aC;
+        }
+        if (resid) {
+            const double2* o = reinterpret_cast<const double2*>(V_in + 4 * i);
+            const double2 a = o[0], b = o[1];
+            const unsigned long long dP = fp_absdiff_bits(P, a.x), dS = fp_absdiff_bits(S, a.y),
+                                     dC = fp_absdiff_bits(C, b.x);
+            r = dP > dS ? dP : dS;
+            r = r > dC ? r : dC;
+        }
+        double2* v = reinterpret_cast<double2*>(V_out + 4 * i);
+        v[0] = make_double2(P, S);
+        v[1] = make_double2(C, 0.0);
+        if (hist_out) {
+            double2* h = reinterpret_cast<double2*>(hist_out + 4 * i);
+            h[0] = make_double2(P, S);
+            h[1] = make_double2(C, 0.0);
+        }
+    }
+    if (outside) {
+        n_out = __reduce_add_sync(0xffffffffu, n_out);
+        if ((threadIdx.x & 31) == 0 && n_out) atomicAdd(outside, (unsigned long long)n_out);
+    }
+    if (resid) {
+#pragma unroll
+        for (int s = 16; s > 0; s >>= 1) {
+            const unsigned long long o = __shfl_xor_sync(0xffffffffu, r, s);
+            r = o > r ? o : r;
+        }
+        if ((threadIdx.x & 31) == 0 && r) atomicMax(resid, r);
+    }
+}
+
+extern "C" int sdp_first_passage(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p,
+                                 const int32_t* cell, const double* lam, int64_t lam_plane, const double* g,
+                                 int64_t n_states, const uint32_t* target, int32_t clamp, double* V_a, double* V_b,
+                                 int32_t n_steps, double* hist, double* resid_out, unsigned long long* counters,
+                                 void* stream) {
+    GridT<double> G;
+    int64_t n = 0;
+    int rc = make_grid<double>(grid, &G, &n);
+    if (rc) return rc;
+    if (W < 1 || n_steps < 0 || n_states != n || lam_plane < W * n)
+        return fail(SDP_EINVAL, "%s", "sdp_first_passage: bad sizes (n_states must be the whole grid)");
+    if (!p || !cell || !lam || !g || !target || !V_a || !V_b)
+        return fail(SDP_EINVAL, "%s", "sdp_first_passage: NULL pointer");
+    if ((((uintptr_t)V_a) | ((uintptr_t)V_b) | ((uintptr_t)hist)) & 15)
+        return fail(SDP_EINVAL, "%s", "sdp_first_passage: V_a, V_b, hist not 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (hist) SDP_CUDA_CHECK(cudaMemcpyAsync(hist, V_a, 32 * n, cudaMemcpyDeviceToDevice, st));
+    unsigned long long* resid = reinterpret_cast<unsigned long long*>(resid_out);
+    if (resid) SDP_CUDA_CHECK(cudaMemsetAsync(resid, 0, sizeof(double), st));
+    const int threads = tuning().fp_threads ? tuning().fp_threads : SDP_FP_THREADS;
+    const unsigned blocks = (unsigned)((n + threads - 1) / threads);
+    const double* in = V_a;
+    double* out = V_b;
+    for (int k = 0; k < n_steps; ++k) {
+        double* h = hist ? hist + (int64_t)(k + 1) * 4 * n : nullptr;
+        unsigned long long* c = k == 0 ? counters : nullptr;
+        unsigned long long* r = k + 1 == n_steps ? resid : nullptr;
+#define SDP_FP_LAUNCH(D_)                                                                                        \
+        if (clamp) k_first_passage<D_, true><<<blocks, threads, 0, st>>>(G, W, g_per_w, p, cell, lam, lam_plane, \
+                                                                         g, n, target, in, out, h, c, r);        \
+        else k_first_passage<D_, false><<<blocks, threads, 0, st>>>(G, W, g_per_w, p, cell, lam, lam_plane, g,  \
+                                                                    n, target, in, out, h, c, r);
+        switch (grid->d) {
+            case 1: SDP_FP_LAUNCH(1) break;
+            case 2: SDP_FP_LAUNCH(2) break;
+            case 3: SDP_FP_LAUNCH(3) break;
+            default: SDP_FP_LAUNCH(4) break;
+        }
+#undef SDP_FP_LAUNCH
+        SDP_LAUNCH_CHECK();
+        const double* t = in;
+        in = out;
+        out = const_cast<double*>(t);
+    }
+    if (n_steps > 0) note_kernel("k_first_passage<D=%d,%s>, %d threads", grid->d, clamp ? "clamp" : "noclamp", threads);
     return SDP_OK;
 }
 

@@ -1652,6 +1652,26 @@ class Engine(object):
                                        self._ptr(counters), self.stream)
         _cabi.check(rc, "sdp_chain_sample")
 
+    # -- first-passage analysis ------------------------------------------
+    def first_passage(self, P, target, clamp, V_a, V_b, n_steps, hist=None, resid_out=None, counters=None):
+        """n_steps steps of the first-passage recursion over the policy tables `P`
+        (sdp_first_passage), ping-pong between V_a (the values the call starts from) and V_b
+        (device fp64 [n*4], records (P, S, C, 0)).  target: device uint32 bit mask; hist: device
+        [(n_steps+1)*n*4], entry j after j steps; resid_out [1]: sup-norm change of the last step;
+        counters: device uint64 [1], += the entries with a weight outside [0, 1] (once per call).
+        One rank only.  Returns the tensor holding the final values."""
+        if self.coll.world > 1 or P.n_states != int(np.prod(P.grid.order[:P.grid.d])):
+            raise NotImplementedError(
+                "first-passage analysis runs on one rank: a state's next states leave the slab of its "
+                "rank (not implemented)")
+        rc = self.lib.sdp_first_passage(ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.p), self._ptr(P.cell),
+                                        self._ptr(P.lam), P.lam_plane, self._ptr(P.g), P.n_states,
+                                        self._ptr(target), 1 if clamp else 0, self._ptr(V_a), self._ptr(V_b),
+                                        int(n_steps), self._ptr(hist), self._ptr(resid_out), self._ptr(counters),
+                                        self.stream)
+        _cabi.check(rc, "sdp_first_passage")
+        return V_a if n_steps % 2 == 0 else V_b
+
     # -- interpolation ----------------------------------------------------
     def interp(self, grid, values, s):
         """values: host (n_v, n_grid); s: host (d, n_s) -> host (n_v, n_s).

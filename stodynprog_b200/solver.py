@@ -804,6 +804,132 @@ class DPSolver(object):
             print('\rpath sampling run in {:.2f} s ({:d} paths x {:d} steps)'.format(exec_time, M, n_steps))
         return total_h, info
 
+    def first_passage(self, pol, target, n_steps=None, clamp=True, history=False, tol=None, check_every=50,
+                      report_time=True):
+        """first-passage analysis of the chain of the policy `pol` with respect to the set
+        `target`, exact and for every start state at once (a backward recursion on the GPU, one
+        thread per state).  Not in the reference.
+
+        Let tau be the first step k >= 0 at which the path is in `target` (a start in the target
+        gives tau = 0, as sample_paths' hit_step).  Over a horizon of n = n_steps steps this returns,
+        for every start state x:
+            prob[x]  = P_x(tau <= n), the probability of reaching the target within n steps;
+            steps[x] = E_x[min(tau, n)], the expected number of steps before reaching it;
+            cost[x]  = the expected stage cost accumulated before tau, within the horizon.
+        They are computed backwards from (1_target, 0, 0) at step n: off the target,
+        P_k = sum_w p_w I[P_{k+1}](f(x, w)), S_k = 1 + sum_w p_w I[S_{k+1}], C_k = sum_w p_w (g + I[C_{k+1}]),
+        with I the multilinear interpolation at the next state; on the target (1, 0, 0).
+
+        clamp=True (default): the interpolation weights are clamped to [0, 1] (NaN: 0), the chain
+            sample_paths samples, so that prob is a true probability.  clamp=False: the weights are
+            used as they are, the chain J is computed with (eval_policy, propagate_distribution);
+            near the boundary its values can leave [0, 1].  With an empty target and clamp=False,
+            cost is eval_policy(pol, n) bit for bit.
+        pol: state_dims + (nb_control,) for a stationary system (n_steps required); (T,) +
+            state_dims + (nb_control,) as returned by bellman_recursion for a time-dependent one
+            (step k applies pol[k] at instant k; n_steps defaults to T).
+        target: boolean array of shape state_dims.
+        history: return every V_k, k = 0 .. n: prob, steps, cost of shape (n+1,) + state_dims,
+            entry k the values from step k (prob[n] = 1_target).  For a stationary system prob[k]
+            is the probability of reaching the target within n - k steps, so the whole law of
+            tau from x is P_x(tau <= j) = prob[n - j][x]; from a start distribution mu0 it is
+            <mu0, prob[n - j]>.
+        tol (stationary systems only): n_steps becomes a maximum; every `check_every` steps the
+            sup-norm change of the last step (over the three outputs) is read back, and the
+            recursion stops when it is <= tol.  prob then tends to P_x(tau < inf), and steps and
+            cost to E_x[tau] and the expected cost before tau wherever the target is reached
+            almost surely.  Where it is not, steps grows without bound (by up to one per step)
+            and `converged` stays False.
+
+        Returns (prob, steps, cost, info), info = {'n_steps': the steps done, 'converged': whether
+        a tol run met tol, 'residuals': the residual read at each check, 'outside_share': the share
+        of the (x, w) table entries of non-target states whose weights were clamped (clamp=True)
+        or extrapolate (clamp=False), over all the instants used}.
+        """
+        import torch
+        t_start = datetime.now()
+        state_dims = self._state_grid_shape
+        nb_control = len(self.sys.control)
+        pol = np.asarray(pol)
+        if self.sys.stationnary:
+            self._check_shape('pol', pol, state_dims + (nb_control,))
+            if n_steps is None:
+                raise ValueError('n_steps is required for a stationary system')
+        else:
+            T = pol.shape[0] if pol.ndim == len(state_dims) + 2 else 0
+            self._check_shape('pol', pol, (max(T, 1),) + state_dims + (nb_control,))
+            if n_steps is None:
+                n_steps = T
+            if n_steps > T:
+                raise ValueError('n_steps = {:d} exceeds the horizon of `pol` ({:d} instants)'.format(
+                    int(n_steps), T))
+            if tol is not None:
+                raise ValueError('tol needs a stationary system')
+        n_steps = int(n_steps)
+        if n_steps < 0:
+            raise ValueError('n_steps must be >= 0')
+        if int(check_every) < 1:
+            raise ValueError('check_every must be >= 1')
+        target = np.asarray(target)
+        self._check_shape('target', target, state_dims)
+        if target.dtype != bool:
+            raise ValueError('`target` must be a boolean array')
+        if report_time:
+            print('first-passage analysis...', end='')
+        eng = self.engine
+        n = int(np.prod(state_dims))
+        V0 = np.zeros((n, 4))
+        V0[:, 0] = target.reshape(-1)
+        V_a = eng.to_device(V0.reshape(-1))
+        V_b = torch.empty_like(V_a)
+        mask = eng.to_device(self._target_mask(target))
+        counters = torch.zeros(1, dtype=torch.int64, device=eng.device)
+        hist = torch.empty((n_steps + 1) * n * 4, dtype=torch.float64, device=eng.device) if history else None
+        residuals, converged, done, entries = [], False, 0, 0
+        if self.sys.stationnary:
+            P = eng.build_policy_tables(self, np.asarray(pol, dtype=float), deterministic=True)
+            chunk = n_steps if tol is None else int(check_every)
+            resid = torch.zeros(1, dtype=torch.float64, device=eng.device) if tol is not None else None
+            while True:
+                k = min(chunk, n_steps - done)
+                out = eng.first_passage(P, mask, clamp, V_a, V_b, k, counters=counters, resid_out=resid,
+                                        hist=hist[done * n * 4:(done + k + 1) * n * 4] if history else None)
+                if out is V_b:
+                    V_a, V_b = V_b, V_a
+                done += k
+                entries += P.W * n if k else 0
+                if tol is not None and k > 0:
+                    r = float(resid.cpu().numpy()[0])
+                    residuals.append(r)
+                    if r <= tol:
+                        converged = True
+                        break
+                if done >= n_steps:
+                    break
+        else:
+            # the chain changes with the instant: tables rebuilt per step, swept from instant n-1 to 0
+            for k in range(n_steps - 1, -1, -1):
+                P = eng.build_policy_tables(self, np.asarray(pol[k], dtype=float), t_k=k, deterministic=True)
+                j = n_steps - 1 - k
+                eng.first_passage(P, mask, clamp, V_a, V_b, 1, counters=counters,
+                                  hist=hist[j * n * 4:(j + 2) * n * 4] if history else None)
+                V_a, V_b = V_b, V_a
+                done += 1
+                entries += P.W * n
+                del P
+        V, cnt = eng.to_host(hist if history else V_a, counters)
+        if history:
+            V = V[:(done + 1) * n * 4].reshape(done + 1, n, 4)[::-1]
+        shape = ((done + 1,) if history else ()) + state_dims
+        V = V.reshape(shape[:-len(state_dims)] + (n, 4))
+        prob, steps, cost = (np.ascontiguousarray(V[..., j]).reshape(shape) for j in range(3))
+        info = {'n_steps': done, 'converged': converged, 'residuals': residuals,
+                'outside_share': float(cnt[0]) / entries if entries else 0.0}
+        exec_time = (datetime.now() - t_start).total_seconds()
+        if report_time:
+            print('\rfirst-passage analysis run in {:.2f} s ({:d} steps)'.format(exec_time, done))
+        return prob, steps, cost, info
+
     @staticmethod
     def _target_mask(target):
         """boolean state_dims array -> 32-bit words, bit y % 32 of word y // 32 = target[y] (C order)"""
