@@ -690,18 +690,35 @@ def test_product_does_not_import_the_oracle():
                 assert "liboracle" not in txt and "sdp_oracle" not in txt, f
 
 
+# the kernel families that divide: the IEEE division sequence is built from FMAs, which is
+# exact by construction.  Every other kernel promises an exact operation order (bit-identity to
+# the oracle or to a numpy model, the rounding margin of DESIGN.md section 4) and must have none.
+FMA_ALLOWED = {"k_build_tables", "k_build_tables_tiled", "k_build_factored", "k_build_factored_tiled",
+               "k_cell_setup", "k_interp", "k_policy_values", "k_combine_column", "k_combine_column_small"}
+
+
+def _kernel_family(fn):
+    """the kernel's name without template arguments or parameter types (_Z<len><name>...)"""
+    m = re.match(r"_Z(\d+)(\w+)", fn)
+    return m.group(2)[:int(m.group(1))] if m else fn
+
+
 def test_sass_has_no_fma_in_sweep_kernels(product):
-    """the parity contract forbids contraction: the sweep / policy kernels must
-    contain no DFMA (divisions in the setup kernels legitimately use it)"""
+    """the parity contract forbids contraction: no kernel may contain DFMA / FFMA except the
+    division-bearing families of FMA_ALLOWED; a new kernel with FMA fails with its name"""
     res = subprocess.run(["cuobjdump", "-sass", _cabi.LIB_PATH], capture_output=True, text=True)
     if res.returncode != 0:
         pytest.skip("cuobjdump unavailable")
-    fn, bad = None, {}
+    fn, bad, families = None, {}, set()
     for line in res.stdout.splitlines():
         m = re.search(r"Function : (\S+)", line)
         if m:
             fn = m.group(1)
-        elif "DFMA" in line and fn and re.search(r"k_sweep|k_policy_eval|k_sub_scalar", fn):
+            families.add(_kernel_family(fn))
+        elif fn and re.search(r"\b[DF]FMA", line) and _kernel_family(fn) not in FMA_ALLOWED:
             bad[fn] = bad.get(fn, 0) + 1
     assert not bad, bad
+    # (not vacuous: the kernels that promise an exact order are all in the library)
+    assert {"k_sweep_tiled", "k_policy_eval", "k_sub_scalar", "k_first_passage", "k_fwd_rows", "k_chain_sample",
+            "k_column_table", "k_supnorm_diff"} <= families
     assert "UBLKCP" in res.stdout      # the TMA-fed variant is built (bulk async copies)

@@ -129,13 +129,30 @@ def test_cell_setup_bit_exact(eng, d):
 # ---------------------------------------------------------------------------
 # K2: interpolation
 # ---------------------------------------------------------------------------
+def _interp_on_path(product, path, monkeypatch, *args):
+    """multilinear_interpolation through the host routine (path "host": no launch) or the K2
+    kernel (path "device": HOST_MAX_POINTS set to 0), checked by the launch counter, so that a
+    change in the routing fails instead of hiding a path"""
+    from stodynprog_b200 import _cabi
+    if path == "device":
+        monkeypatch.setattr(product.interp, "HOST_MAX_POINTS", 0)
+    else:
+        assert args[3].shape[0] * args[4].shape[1] <= product.interp.HOST_MAX_POINTS
+    lib = _cabi.load_library()
+    n0 = lib.sdp_launch_count()
+    out = product.multilinear_interpolation(*args)
+    assert (lib.sdp_launch_count() > n0) == (path == "device")
+    return out
+
+
 @gpu
 @pytest.mark.parametrize("d", [1, 2, 3, 4])
-def test_interp_golden_bit_exact(product, d):
+@pytest.mark.parametrize("path", ["host", "device"])
+def test_interp_golden_bit_exact(product, path, d, monkeypatch):
     """against outputs of the reference's compiled Cython routine"""
     G = golden("interp_kat.npz")
-    out = product.multilinear_interpolation(G["d%d_smin" % d], G["d%d_smax" % d], G["d%d_orders" % d],
-                                            G["d%d_values" % d], G["d%d_s" % d])
+    out = _interp_on_path(product, path, monkeypatch, G["d%d_smin" % d], G["d%d_smax" % d], G["d%d_orders" % d],
+                          G["d%d_values" % d], G["d%d_s" % d])
     ref = G["d%d_out" % d]
     assert np.array_equal(np.isnan(out), np.isnan(ref))
     ok = ~np.isnan(ref)
@@ -144,13 +161,14 @@ def test_interp_golden_bit_exact(product, d):
 
 @gpu
 @pytest.mark.parametrize("d", [1, 2, 3, 4])
-def test_interp_f32_golden(product, d):
+@pytest.mark.parametrize("path", ["host", "device"])
+def test_interp_f32_golden(product, path, d, monkeypatch):
     G = golden("interp_kat.npz")
     with np.errstate(over="ignore"):
         s32 = np.ascontiguousarray(G["d%d_s" % d].astype(np.float32))
-    out = product.multilinear_interpolation(G["d%d_smin" % d].astype(np.float32),
-                                            G["d%d_smax" % d].astype(np.float32), G["d%d_orders" % d],
-                                            G["d%d_values" % d].astype(np.float32), s32)
+    out = _interp_on_path(product, path, monkeypatch, G["d%d_smin" % d].astype(np.float32),
+                          G["d%d_smax" % d].astype(np.float32), G["d%d_orders" % d],
+                          G["d%d_values" % d].astype(np.float32), s32)
     assert out.dtype == np.float32
     ref = G["d%d_out_f32" % d]
     # NaN payloads are not part of the contract (x86 makes 0xFFC00000, CUDA's
