@@ -268,8 +268,8 @@ const char* sdp_last_kernel(void);
  * "p2p_timeout_s" (bound of the peer-flag waits, default 600 s, then the kernel traps),
  * "chain_threads" (sdp_chain_sample: threads per CTA, 32..1024 in multiples of 32; 0 = default,
  * 256; the results do not depend on it),
- * "fp_threads" (sdp_first_passage: threads per CTA, 32..1024 in multiples of 32; 0 = default,
- * 256; the results do not depend on it).
+ * "fp_threads" (sdp_first_passage and sdp_cost_moments: threads per CTA, 32..1024 in multiples
+ * of 32; 0 = default, 256; the results do not depend on it).
  * Not thread-safe against concurrent launches. */
 int sdp_set_option(const char* name, int value);
 /* With "col_prune_stats" on: the warp steps (groups of col_ub controls of one item) that the
@@ -562,6 +562,29 @@ int sdp_first_passage(const SdpGrid* grid, int32_t W, int32_t g_per_w, const dou
                       const double* lam, int64_t lam_plane, const double* g, int64_t n_states,
                       const uint32_t* target, int32_t clamp, double* V_a, double* V_b, int32_t n_steps,
                       double* hist, double* resid_out, unsigned long long* counters, void* stream);
+
+/* K1''''' - moments of the total stage cost of a fixed policy's chain, before a target set or
+ * over the whole horizon: mean, variance and third central moment, from every state.  New
+ * feature, no reference counterpart.  The pass of sdp_first_passage (same tables, target mask,
+ * clamp, records, hist, resid_out, counters, refusals and fp_threads), with the record (M, V, K, 0):
+ * over the steps left, M the mean of the cost G accumulated before the target, V its variance and
+ * K its third central moment E[(G - M)^3].  target may be NULL (no target: the whole horizon).
+ * On a target state a step writes (0, 0, 0) without reading its table entries; elsewhere, with
+ * I[.] the nested lerp at the next state of node w and c the corners of its cell, two passes
+ * over the nodes w in order:
+ *   m = acc + (g + I[M])*p_w             (acc from 0: the fixed-policy backup of sdp_policy_eval)
+ * then, centred on this step's m,
+ *   d_c = (g + M(c)) - m,  a_c = V(c) + d_c*d_c,  b_c = K(c) + d_c*(3*V(c) + d_c*d_c)
+ *   V = acc + I[a]*p_w,    K = acc + I[b]*p_w   (acc from 0; I[a], I[b] lerps of the a_c, b_c)
+ * (the laws of total variance and total cumulance).  The centred form loses no digits to
+ * E[G^2] - M^2, and with clamp != 0 every term of V is non-negative, so V >= 0 exactly.  The
+ * recursion starts from (0, 0, 0).  resid_out: max over the states and the three values of
+ * |new - old| in the last step (NaN if any is NaN).  With clamp == 0 and no target, M is the
+ * result of sdp_policy_eval bit for bit; M is always the C of sdp_first_passage bit for bit. */
+int sdp_cost_moments(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p, const int32_t* cell,
+                     const double* lam, int64_t lam_plane, const double* g, int64_t n_states,
+                     const uint32_t* target, int32_t clamp, double* V_a, double* V_b, int32_t n_steps,
+                     double* hist, double* resid_out, unsigned long long* counters, void* stream);
 
 /* K3 - argmin index -> control values, the `u_grids[i].flatten()[ind_opt[i]]` of
  * stodynprog.py:686-689 for every state at once.  lo/hi: device [n][nc] box

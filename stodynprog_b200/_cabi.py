@@ -185,6 +185,8 @@ SIGNATURES = {
                                         _vp, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sdp_first_passage": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _i32,
                                          _vp, _vp, _vp, _vp]),
+    "sdp_cost_moments": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _i32, _vp, _vp, _i32,
+                                        _vp, _vp, _vp, _vp]),
     "sdp_policy_values": (ctypes.c_int, [_i64, _i32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "sdp_sweep_finalize_cols": (ctypes.c_int, [ctypes.POINTER(SdpTables), _vp, _vp, _vp, _vp, _i64, _i64,
                                                _i32, _vp, _vp, _vp, _vp, _i32, _vp]),

@@ -7,8 +7,8 @@
 //     looped over the state grid by value_iteration (:511-515)
 //   * the policy-evaluation iteration of eval_policy (:743-763)
 // and adds, with no reference counterpart, the forward (transposed) application of a fixed
-// policy's chain (K1'', distribution propagation), path sampling (K1''') and the first-passage
-// recursion to a target set (K1'''').
+// policy's chain (K1'', distribution propagation), path sampling (K1'''), the first-passage
+// recursion to a target set (K1'''') and the moments of the total cost (K1''''').
 //
 // This is a gather-reduce, not a contraction: no tensor cores.  The sweep kernel
 // streams the dense (cell, lambda, g) tables once from HBM with 128-bit
@@ -1077,7 +1077,7 @@ struct Tuning {
     int small_combine; // sdp_sweep_finalize_cols: the 128-thread combine that fits next to a streaming CTA (1) or the 1024-thread one (0)
     int carveout;      // layout CF: streaming kernel and small combine ask for the largest shared-memory carve-out (1) or leave it to the driver (0)
     int chain_threads; // sdp_chain_sample: threads per CTA (0 = 256); the results do not depend on it
-    int fp_threads;    // sdp_first_passage: threads per CTA (0 = 256); the results do not depend on it
+    int fp_threads;    // sdp_first_passage, sdp_cost_moments: threads per CTA (0 = 256); the results do not depend on it
     int dbg_exchange;  // TIMING EXPERIMENTS ONLY (wrong results): 1 = no stores to remote ranks, 2 = no system fence, 4 = relaxed flag stores
 };
 static int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v); }
@@ -4322,6 +4322,208 @@ extern "C" int sdp_first_passage(const SdpGrid* grid, int32_t W, int32_t g_per_w
         out = const_cast<double*>(t);
     }
     if (n_steps > 0) note_kernel("k_first_passage<D=%d,%s>, %d threads", grid->d, clamp ? "clamp" : "noclamp", threads);
+    return SDP_OK;
+}
+
+// ---------------------------------------------------------------------------
+// K1''''': moments of a fixed policy's total cost (include/sdp_b200.h).  New feature.
+// The pass of k_first_passage with (M, V, K, 0) records: mean, variance and third central
+// moment of the cost before the target.  Two passes over the nodes per state: the mean first,
+// then the variance and third moment centred on it, so that no raw moment is ever formed.
+// ---------------------------------------------------------------------------
+
+// pass 1: the nested lerp of Lerp<double, D, K> applied to the means of the records
+template <int D, int K>
+struct LerpM {
+    __device__ __forceinline__ static double eval(const double* __restrict__ V, int base,
+                                                  const int (&stride)[SDP_MAX_D], const double (&lam)[D]) {
+        const double a = LerpM<D, K + 1>::eval(V, base, stride, lam);
+        const double b = LerpM<D, K + 1>::eval(V, base + (K == D - 1 ? 1 : stride[K]), stride, lam);
+        const double l = lam[K], m = sub_(1.0, l);
+        return add_(mul_(m, a), mul_(l, b));
+    }
+};
+template <int D>
+struct LerpM<D, D> {
+    __device__ __forceinline__ static double eval(const double* __restrict__ V, int base, const int (&)[SDP_MAX_D],
+                                                  const double (&)[D]) {
+        return __ldg(V + 4 * (int64_t)base);
+    }
+};
+
+// pass 2: the same lerp of a_c = V_c + d_c^2 and b_c = K_c + d_c (3 V_c + d_c^2), formed at each
+// corner c from its record, with d_c = (gv + M_c) - m the corner's deviation from the mean m
+template <int D, int K>
+struct LerpAB {
+    __device__ __forceinline__ static void eval(const double* __restrict__ V, int base, const int (&stride)[SDP_MAX_D],
+                                                const double (&lam)[D], double gv, double mean, double& A,
+                                                double& B) {
+        double aA, aB, bA, bB;
+        LerpAB<D, K + 1>::eval(V, base, stride, lam, gv, mean, aA, aB);
+        LerpAB<D, K + 1>::eval(V, base + (K == D - 1 ? 1 : stride[K]), stride, lam, gv, mean, bA, bB);
+        const double l = lam[K], m = sub_(1.0, l);
+        A = add_(mul_(m, aA), mul_(l, bA));
+        B = add_(mul_(m, aB), mul_(l, bB));
+    }
+};
+template <int D>
+struct LerpAB<D, D> {
+    __device__ __forceinline__ static void eval(const double* __restrict__ V, int base, const int (&)[SDP_MAX_D],
+                                                const double (&)[D], double gv, double mean, double& A, double& B) {
+        const double* r = V + 4 * (int64_t)base;
+        const double2 mv = __ldg(reinterpret_cast<const double2*>(r));
+        const double dl = sub_(add_(gv, mv.x), mean), dd = mul_(dl, dl);
+        A = add_(mv.y, dd);
+        B = add_(__ldg(r + 2), mul_(dl, add_(mul_(3.0, mv.y), dd)));
+    }
+};
+
+// the D weights of table entry `off`, clamped when CLAMP; returns whether one is outside [0, 1] or NaN
+template <int D, bool CLAMP>
+__device__ __forceinline__ bool cm_weights(const double* __restrict__ lam, int64_t lam_plane, int64_t off,
+                                           double (&l)[D]) {
+    bool out = false;
+#pragma unroll
+    for (int k = 0; k < D; ++k) {
+        double lk = lam[(int64_t)k * lam_plane + off];
+        out |= !(lk >= 0.0 && lk <= 1.0);
+        if (CLAMP) lk = (lk < 0.0 || isnan(lk)) ? 0.0 : (lk > 1.0 ? 1.0 : lk);
+        l[k] = lk;
+    }
+    return out;
+}
+
+template <int D, bool CLAMP>
+__global__ void __launch_bounds__(1024)
+k_cost_moments(GridT<double> G, int W, int g_per_w, const double* __restrict__ p, const int32_t* __restrict__ cell,
+               const double* __restrict__ lam, int64_t lam_plane, const double* __restrict__ g, int64_t n,
+               const uint32_t* __restrict__ target, const double* __restrict__ V_in, double* __restrict__ V_out,
+               double* __restrict__ hist_out, unsigned long long* __restrict__ outside,
+               unsigned long long* __restrict__ resid) {
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    unsigned int n_out = 0;
+    unsigned long long r = 0;
+    if (i < n) {
+        double M = 0.0, Var = 0.0, K3 = 0.0;
+        if (!(target && ((__ldg(target + (i >> 5)) >> (i & 31)) & 1u))) {
+            const double g0 = g_per_w ? 0.0 : g[i];
+            for (int w = 0; w < W; ++w) {
+                const int64_t off = (int64_t)w * n + i;
+                double l[D];
+                n_out += cm_weights<D, CLAMP>(lam, lam_plane, off, l);
+                const double gv = g_per_w ? g[off] : g0;
+                M = add_(M, mul_(add_(gv, LerpM<D, 0>::eval(V_in, cell[off], G.stride, l)), p[w]));
+            }
+            for (int w = 0; w < W; ++w) {
+                const int64_t off = (int64_t)w * n + i;
+                double l[D];
+                cm_weights<D, CLAMP>(lam, lam_plane, off, l);
+                const double gv = g_per_w ? g[off] : g0;
+                double a, b;
+                if constexpr (D <= 2) {
+                    LerpAB<D, 0>::eval(V_in, cell[off], G.stride, l, gv, M, a, b);
+                } else {
+                    // the outer level of LerpAB<D, 0>, its two halves one after the other: the
+                    // gathers of both at once do not fit the 64 registers of a 1024-thread launch
+                    const int base = cell[off];
+                    double aA = 0.0, aB = 0.0, bA = 0.0, bB = 0.0;
+#pragma unroll 1
+                    for (int h = 0; h < 2; ++h) {
+                        double x, y;
+                        LerpAB<D, 1>::eval(V_in, base + h * G.stride[0], G.stride, l, gv, M, x, y);
+                        if (h == 0) {
+                            aA = x;
+                            aB = y;
+                        } else {
+                            bA = x;
+                            bB = y;
+                        }
+                    }
+                    const double m0 = sub_(1.0, l[0]);
+                    a = add_(mul_(m0, aA), mul_(l[0], bA));
+                    b = add_(mul_(m0, aB), mul_(l[0], bB));
+                }
+                const double pw = p[w];
+                Var = add_(Var, mul_(a, pw));
+                K3 = add_(K3, mul_(b, pw));
+            }
+        }
+        if (resid) {
+            const double2* o = reinterpret_cast<const double2*>(V_in + 4 * i);
+            const double2 a = o[0], b = o[1];
+            const unsigned long long dM = fp_absdiff_bits(M, a.x), dV = fp_absdiff_bits(Var, a.y),
+                                     dK = fp_absdiff_bits(K3, b.x);
+            r = dM > dV ? dM : dV;
+            r = r > dK ? r : dK;
+        }
+        double2* v = reinterpret_cast<double2*>(V_out + 4 * i);
+        v[0] = make_double2(M, Var);
+        v[1] = make_double2(K3, 0.0);
+        if (hist_out) {
+            double2* h = reinterpret_cast<double2*>(hist_out + 4 * i);
+            h[0] = make_double2(M, Var);
+            h[1] = make_double2(K3, 0.0);
+        }
+    }
+    if (outside) {
+        n_out = __reduce_add_sync(0xffffffffu, n_out);
+        if ((threadIdx.x & 31) == 0 && n_out) atomicAdd(outside, (unsigned long long)n_out);
+    }
+    if (resid) {
+#pragma unroll
+        for (int s = 16; s > 0; s >>= 1) {
+            const unsigned long long o = __shfl_xor_sync(0xffffffffu, r, s);
+            r = o > r ? o : r;
+        }
+        if ((threadIdx.x & 31) == 0 && r) atomicMax(resid, r);
+    }
+}
+
+extern "C" int sdp_cost_moments(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p,
+                                const int32_t* cell, const double* lam, int64_t lam_plane, const double* g,
+                                int64_t n_states, const uint32_t* target, int32_t clamp, double* V_a, double* V_b,
+                                int32_t n_steps, double* hist, double* resid_out, unsigned long long* counters,
+                                void* stream) {
+    GridT<double> G;
+    int64_t n = 0;
+    int rc = make_grid<double>(grid, &G, &n);
+    if (rc) return rc;
+    if (W < 1 || n_steps < 0 || n_states != n || lam_plane < W * n)
+        return fail(SDP_EINVAL, "%s", "sdp_cost_moments: bad sizes (n_states must be the whole grid)");
+    if (!p || !cell || !lam || !g || !V_a || !V_b)
+        return fail(SDP_EINVAL, "%s", "sdp_cost_moments: NULL pointer");
+    if ((((uintptr_t)V_a) | ((uintptr_t)V_b) | ((uintptr_t)hist)) & 15)
+        return fail(SDP_EINVAL, "%s", "sdp_cost_moments: V_a, V_b, hist not 16-byte aligned");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (hist) SDP_CUDA_CHECK(cudaMemcpyAsync(hist, V_a, 32 * n, cudaMemcpyDeviceToDevice, st));
+    unsigned long long* resid = reinterpret_cast<unsigned long long*>(resid_out);
+    if (resid) SDP_CUDA_CHECK(cudaMemsetAsync(resid, 0, sizeof(double), st));
+    const int threads = tuning().fp_threads ? tuning().fp_threads : SDP_FP_THREADS;
+    const unsigned blocks = (unsigned)((n + threads - 1) / threads);
+    const double* in = V_a;
+    double* out = V_b;
+    for (int k = 0; k < n_steps; ++k) {
+        double* h = hist ? hist + (int64_t)(k + 1) * 4 * n : nullptr;
+        unsigned long long* c = k == 0 ? counters : nullptr;
+        unsigned long long* r = k + 1 == n_steps ? resid : nullptr;
+#define SDP_CM_LAUNCH(D_)                                                                                       \
+        if (clamp) k_cost_moments<D_, true><<<blocks, threads, 0, st>>>(G, W, g_per_w, p, cell, lam, lam_plane, \
+                                                                        g, n, target, in, out, h, c, r);        \
+        else k_cost_moments<D_, false><<<blocks, threads, 0, st>>>(G, W, g_per_w, p, cell, lam, lam_plane, g,  \
+                                                                   n, target, in, out, h, c, r);
+        switch (grid->d) {
+            case 1: SDP_CM_LAUNCH(1) break;
+            case 2: SDP_CM_LAUNCH(2) break;
+            case 3: SDP_CM_LAUNCH(3) break;
+            default: SDP_CM_LAUNCH(4) break;
+        }
+#undef SDP_CM_LAUNCH
+        SDP_LAUNCH_CHECK();
+        const double* t = in;
+        in = out;
+        out = const_cast<double*>(t);
+    }
+    if (n_steps > 0) note_kernel("k_cost_moments<D=%d,%s>, %d threads", grid->d, clamp ? "clamp" : "noclamp", threads);
     return SDP_OK;
 }
 

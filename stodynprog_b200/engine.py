@@ -1672,6 +1672,24 @@ class Engine(object):
         _cabi.check(rc, "sdp_first_passage")
         return V_a if n_steps % 2 == 0 else V_b
 
+    # -- moments of the total cost ------------------------------------------
+    def cost_moments(self, P, target, clamp, V_a, V_b, n_steps, hist=None, resid_out=None, counters=None):
+        """n_steps steps of the cost-moment recursion over the policy tables `P`
+        (sdp_cost_moments), with the conventions of first_passage: records (M, V, K, 0) of the
+        mean, variance and third central moment of the cost; target: device uint32 bit mask or
+        None (no target).  One rank only.  Returns the tensor holding the final values."""
+        if self.coll.world > 1 or P.n_states != int(np.prod(P.grid.order[:P.grid.d])):
+            raise NotImplementedError(
+                "the cost moments run on one rank: a state's next states leave the slab of its "
+                "rank (not implemented)")
+        rc = self.lib.sdp_cost_moments(ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.p), self._ptr(P.cell),
+                                       self._ptr(P.lam), P.lam_plane, self._ptr(P.g), P.n_states,
+                                       self._ptr(target), 1 if clamp else 0, self._ptr(V_a), self._ptr(V_b),
+                                       int(n_steps), self._ptr(hist), self._ptr(resid_out), self._ptr(counters),
+                                       self.stream)
+        _cabi.check(rc, "sdp_cost_moments")
+        return V_a if n_steps % 2 == 0 else V_b
+
     # -- interpolation ----------------------------------------------------
     def interp(self, grid, values, s):
         """values: host (n_v, n_grid); s: host (d, n_s) -> host (n_v, n_s).

@@ -846,6 +846,69 @@ class DPSolver(object):
         of the (x, w) table entries of non-target states whose weights were clamped (clamp=True)
         or extrapolate (clamp=False), over all the instants used}.
         """
+        return self._backward_analysis('first-passage analysis', self.engine.first_passage, pol, np.asarray(target),
+                                       n_steps, clamp, history, tol, check_every, report_time, 1.0)
+
+    def cost_moments(self, pol, n_steps=None, target=None, clamp=True, history=False, tol=None, check_every=50,
+                     report_time=True):
+        """mean, variance and third central moment of the total stage cost of the policy `pol`,
+        exact and for every start state at once (a backward recursion on the GPU, one thread per
+        state).  Not in the reference: sample_paths estimates the same from one start at a time.
+
+        Let tau be the first step k >= 0 at which the path is in `target` (tau = inf without a
+        target) and G = sum_{k < min(tau, n)} g(x_k, pol(x_k), w_k) the stage cost accumulated
+        before tau within the horizon of n = n_steps steps.  This returns, for every start state x:
+            mean[x]  = E_x[G]  (eval_policy(pol, n) without a target; first_passage's cost with one);
+            var[x]   = Var_x[G];
+            third[x] = E_x[(G - mean[x])^3].
+        The standard deviation is sqrt(var) and the skewness third / var**1.5.  From a start
+        distribution mu0 (normalised to sum 1), with mbar = <mu0, mean> and d = mean - mbar:
+            E[G] = mbar,  Var[G] = <mu0, var + d**2>,  E[(G - mbar)^3] = <mu0, third + 3 var d + d**3>.
+        They are computed backwards from (0, 0, 0) at step n; at each step, off the target, the mean
+        m = sum_w p_w (g + I[M](f(x, w))) first, then, with each corner c of the next state's cell
+        centred on m, d_c = g + M(c) - m: V = sum_w p_w I[V(c) + d_c**2],
+        K = sum_w p_w I[K(c) + d_c (3 V(c) + d_c**2)] (the laws of total variance and total
+        cumulance; I the multilinear interpolation at the next state); on the target (0, 0, 0).
+        The centred form keeps the digits that E[G**2] - mean**2 would lose where the mean is large
+        against the spread, and with clamp=True var >= 0 holds exactly.
+
+        clamp=True (default): the interpolation weights are clamped to [0, 1] (NaN: 0), the chain
+            sample_paths samples.  clamp=False: the weights are used as they are, the chain J is
+            computed with.
+        pol: state_dims + (nb_control,) for a stationary system (n_steps required); (T,) +
+            state_dims + (nb_control,) as returned by bellman_recursion for a time-dependent one
+            (step k applies pol[k] at instant k; n_steps defaults to T).  Deterministic systems
+            are accepted.
+        target: boolean array of shape state_dims, or None (the cost over the whole horizon).
+        history: return every step k = 0 .. n: mean, var, third of shape (n+1,) + state_dims.  For
+            a stationary system entry k holds the moments of the cost over the last n - k steps,
+            so it shows how the spread grows with the horizon.
+        tol (stationary systems with a target only): n_steps becomes a maximum; every
+            `check_every` steps the sup-norm change of the last step (over the three outputs) is
+            read back, and the recursion stops when it is <= tol: the moments of the cost before
+            tau, wherever tau is almost surely finite.  Without a target the mean and variance grow
+            without bound.
+
+        Returns (mean, var, third, info), info = {'n_steps': the steps done, 'converged': whether a
+        tol run met tol, 'residuals': the residual read at each check, 'outside_share': the share of
+        the (x, w) table entries of non-target states whose weights were clamped (clamp=True) or
+        extrapolate (clamp=False), over all the instants used}.
+        """
+        if target is not None:
+            target = np.asarray(target)
+        elif tol is not None:
+            raise ValueError('tol needs a target: without one the moments grow without bound')
+        return self._backward_analysis('cost moments', self.engine.cost_moments, pol, target, n_steps, clamp,
+                                       history, tol, check_every, report_time, 0.0)
+
+    def _backward_analysis(self, what, run, pol, target, n_steps, clamp, history, tol, check_every, report_time,
+                           on_target):
+        """the driver of first_passage and cost_moments: the argument checks, then n_steps steps of
+        the backward recursion `run` (Engine.first_passage or .cost_moments) from the records
+        (on_target if the state is in `target` else 0, 0, 0, 0); stationary systems in chunks of
+        check_every steps when tol is given, time-dependent ones instant by instant from n-1 to 0.
+        target: boolean state_dims array, or None (no target, no mask).  Returns the first three
+        values of the records (with `history`, every step, entry k = step k) and info."""
         import torch
         t_start = datetime.now()
         state_dims = self._state_grid_shape
@@ -870,19 +933,20 @@ class DPSolver(object):
             raise ValueError('n_steps must be >= 0')
         if int(check_every) < 1:
             raise ValueError('check_every must be >= 1')
-        target = np.asarray(target)
-        self._check_shape('target', target, state_dims)
-        if target.dtype != bool:
-            raise ValueError('`target` must be a boolean array')
+        if target is not None:
+            self._check_shape('target', target, state_dims)
+            if target.dtype != bool:
+                raise ValueError('`target` must be a boolean array')
         if report_time:
-            print('first-passage analysis...', end='')
+            print(what + '...', end='')
         eng = self.engine
         n = int(np.prod(state_dims))
         V0 = np.zeros((n, 4))
-        V0[:, 0] = target.reshape(-1)
+        if target is not None:
+            V0[:, 0] = np.where(target.reshape(-1), on_target, 0.0)
         V_a = eng.to_device(V0.reshape(-1))
         V_b = torch.empty_like(V_a)
-        mask = eng.to_device(self._target_mask(target))
+        mask = eng.to_device(self._target_mask(target)) if target is not None else None
         counters = torch.zeros(1, dtype=torch.int64, device=eng.device)
         hist = torch.empty((n_steps + 1) * n * 4, dtype=torch.float64, device=eng.device) if history else None
         residuals, converged, done, entries = [], False, 0, 0
@@ -892,8 +956,8 @@ class DPSolver(object):
             resid = torch.zeros(1, dtype=torch.float64, device=eng.device) if tol is not None else None
             while True:
                 k = min(chunk, n_steps - done)
-                out = eng.first_passage(P, mask, clamp, V_a, V_b, k, counters=counters, resid_out=resid,
-                                        hist=hist[done * n * 4:(done + k + 1) * n * 4] if history else None)
+                out = run(P, mask, clamp, V_a, V_b, k, counters=counters, resid_out=resid,
+                          hist=hist[done * n * 4:(done + k + 1) * n * 4] if history else None)
                 if out is V_b:
                     V_a, V_b = V_b, V_a
                 done += k
@@ -911,8 +975,8 @@ class DPSolver(object):
             for k in range(n_steps - 1, -1, -1):
                 P = eng.build_policy_tables(self, np.asarray(pol[k], dtype=float), t_k=k, deterministic=True)
                 j = n_steps - 1 - k
-                eng.first_passage(P, mask, clamp, V_a, V_b, 1, counters=counters,
-                                  hist=hist[j * n * 4:(j + 2) * n * 4] if history else None)
+                run(P, mask, clamp, V_a, V_b, 1, counters=counters,
+                    hist=hist[j * n * 4:(j + 2) * n * 4] if history else None)
                 V_a, V_b = V_b, V_a
                 done += 1
                 entries += P.W * n
@@ -922,13 +986,13 @@ class DPSolver(object):
             V = V[:(done + 1) * n * 4].reshape(done + 1, n, 4)[::-1]
         shape = ((done + 1,) if history else ()) + state_dims
         V = V.reshape(shape[:-len(state_dims)] + (n, 4))
-        prob, steps, cost = (np.ascontiguousarray(V[..., j]).reshape(shape) for j in range(3))
+        a, b, c = (np.ascontiguousarray(V[..., j]).reshape(shape) for j in range(3))
         info = {'n_steps': done, 'converged': converged, 'residuals': residuals,
                 'outside_share': float(cnt[0]) / entries if entries else 0.0}
         exec_time = (datetime.now() - t_start).total_seconds()
         if report_time:
-            print('\rfirst-passage analysis run in {:.2f} s ({:d} steps)'.format(exec_time, done))
-        return prob, steps, cost, info
+            print('\r{:s} run in {:.2f} s ({:d} steps)'.format(what, exec_time, done))
+        return a, b, c, info
 
     @staticmethod
     def _target_mask(target):
