@@ -276,6 +276,33 @@ int sdp_set_option(const char* name, int value);
  * pruning column sweeps have met, and how many of them skipped the evaluation, since the previous
  * call.  Synchronizes the device.  Both are 0 when nothing was counted. */
 int sdp_col_prune_counts(int64_t* steps, int64_t* skipped);
+/* The same for group skipping: the groups of controls (sdp_column_groups_build) that the pruning
+ * sweeps have met, and how many of them were passed over whole.  A group passed over also counts
+ * as its warp steps, all skipped, in sdp_col_prune_counts. */
+int sdp_col_group_counts(int64_t* groups, int64_t* skipped);
+
+/* Layout CF, group skipping (DESIGN.md section 4).  The controls of every work item are cut into
+ * groups of K (a multiple of 4, at most 64); for every (item, group, lane) a 16-byte summary of
+ * the lane's live controls - the least stage cost, a bound of |g|, the lowest and highest table
+ * row, whether every weight is in [0, 1] - lets the pruning sweep pass over a group that provably
+ * loses for all 32 lanes without reading its (x,u) stream.  The results are those of the sweep
+ * without it, bit for bit.
+ * sdp_column_groups_bytes: the size of the caller-owned buffer for tables `tab` (copies the item
+ * list to the host after synchronizing `stream`).
+ * sdp_column_groups_build: fills `buf` (16-byte aligned, >= that size) from the u-part of `tab`
+ * on `stream` and registers it for every sweep whose tables have the same items, cell, lam, g
+ * and n_items (any item range or order: the column pieces find it); returns when the summary is
+ * ready, with its id.  The buffer must live until the registration ends: sdp_column_groups_release,
+ * a new build for the same tables, or a table build (sdp_build_tables*) writing into the same
+ * cell, lam or g.  A sweep whose tables have no registered summary runs without group skipping.
+ * Option "col_groups" (0|1, default 1) turns the use of registered summaries off and on.
+ * sdp_column_groups_info: K and the window length L of the rows' bound minima chosen for a
+ * registered summary (0, 0: not registered). */
+int sdp_column_groups_bytes(const SdpTables* tab, int32_t K, void* stream, int64_t* bytes);
+int sdp_column_groups_build(const SdpGrid* grid, const SdpTables* tab, int32_t K, void* buf, int64_t bytes,
+                            void* stream, int64_t* id);
+int sdp_column_groups_release(int64_t id);
+int sdp_column_groups_info(int64_t id, int32_t* K, int32_t* L);
 
 /* K0a - cell search on explicit points.
  * Replaces the cell-search half of multilinear_interpolation_{1..4}d

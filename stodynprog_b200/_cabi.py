@@ -149,6 +149,12 @@ SIGNATURES = {
     "sdp_last_kernel": (ctypes.c_char_p, []),
     "sdp_set_option": (ctypes.c_int, [ctypes.c_char_p, ctypes.c_int]),
     "sdp_col_prune_counts": (ctypes.c_int, [ctypes.POINTER(_i64), ctypes.POINTER(_i64)]),
+    "sdp_col_group_counts": (ctypes.c_int, [ctypes.POINTER(_i64), ctypes.POINTER(_i64)]),
+    "sdp_column_groups_bytes": (ctypes.c_int, [ctypes.POINTER(SdpTables), _i32, _vp, ctypes.POINTER(_i64)]),
+    "sdp_column_groups_build": (ctypes.c_int, [_gp, ctypes.POINTER(SdpTables), _i32, _vp, _i64, _vp,
+                                               ctypes.POINTER(_i64)]),
+    "sdp_column_groups_release": (ctypes.c_int, [_i64]),
+    "sdp_column_groups_info": (ctypes.c_int, [_i64, ctypes.POINTER(_i32), ctypes.POINTER(_i32)]),
     "sdp_cell_setup": (ctypes.c_int, [_gp, _i64, _vp, _vp, _vp, _vp]),
     "sdp_build_tables": (ctypes.c_int, [_gp, _i32, _i32, _i64, _vp, _vp, _vp, _vp, _i64, _vp,
                                         _i32, _vp]),

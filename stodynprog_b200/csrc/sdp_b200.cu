@@ -34,6 +34,8 @@
 #include <limits.h>
 #include <math.h>
 #include <atomic>
+#include <mutex>
+#include <vector>
 
 #include <cub/device/device_scan.cuh>
 #include <cub/device/device_segmented_sort.cuh>
@@ -305,10 +307,13 @@ k_build_tables(GridT<double> G, int W, int g_per_w, int tiles_per_state,
     }
 }
 
+static void column_groups_drop(const void* cell, const void* lam, const void* g);
+
 extern "C" int sdp_build_tables(const SdpGrid* grid, int32_t W, int32_t g_per_w, int64_t n_states,
                                 const SdpStateDesc* desc, const double* staging, int32_t* cell,
                                 double* lam, int64_t lam_plane, double* g, int32_t max_Upad,
                                 void* stream) {
+    column_groups_drop(cell, lam, g);      // (their group summaries describe the old entries)
     GridT<double> G;
     int rc = make_grid<double>(grid, &G, nullptr);
     if (rc) return rc;
@@ -366,6 +371,7 @@ extern "C" int sdp_build_tables_tiled(const SdpGrid* grid, int32_t W, int32_t g_
                                       const int64_t* tile_off, const int64_t* tile_g_off,
                                       const int32_t* tile_U, int32_t max_tile_U, int32_t* cell,
                                       double* lam, int64_t lam_plane, double* g, void* stream) {
+    column_groups_drop(cell, lam, g);      // (their group summaries describe the old entries)
     GridT<double> G;
     int rc = make_grid<double>(grid, &G, nullptr);
     if (rc) return rc;
@@ -484,6 +490,7 @@ extern "C" int sdp_build_tables_factored(const SdpGrid* grid, int32_t W, int32_t
                                          double* lam, int64_t lam_plane, double* g, int32_t max_Upad,
                                          int32_t* cell_w, double* lam_w, int64_t lam_w_plane,
                                          void* stream) {
+    column_groups_drop(cell, lam, g);      // (their group summaries describe the old entries)
     GridT<double> G;
     int rc = make_grid<double>(grid, &G, nullptr);
     if (rc) return rc;
@@ -513,6 +520,7 @@ extern "C" int sdp_build_tables_factored_tiled(const SdpGrid* grid, int32_t W, i
                                                int32_t max_tile_U, int32_t* cell, double* lam,
                                                int64_t lam_plane, double* g, int32_t* cell_w,
                                                double* lam_w, int64_t lam_w_plane, void* stream) {
+    column_groups_drop(cell, lam, g);      // (their group summaries describe the old entries)
     GridT<double> G;
     int rc = make_grid<double>(grid, &G, nullptr);
     if (rc) return rc;
@@ -1073,6 +1081,7 @@ struct Tuning {
     int col_prepass;   // layout CF: column tables from the coalesced pre-pass, copied by vector loads (1) or by the TMA engine (2); 0: gathered by every CTA
     int col_prune;     // layout CF with SdpTables.col_bound: skip the controls that provably lose (1) or evaluate all (0)
     int col_prune_stats; // layout CF pruning sweep: count warp steps and skipped ones (measurements only)
+    int col_groups;    // layout CF pruning sweep: pass over whole groups of controls by their registered summaries (1) or not (0)
     int pdl;           // programmatic dependent launch of pre-pass / column sweep / combine (1) or plain launches (0)
     int small_combine; // sdp_sweep_finalize_cols: the 128-thread combine that fits next to a streaming CTA (1) or the 1024-thread one (0)
     int carveout;      // layout CF: streaming kernel and small combine ask for the largest shared-memory carve-out (1) or leave it to the driver (0)
@@ -1122,6 +1131,7 @@ static Tuning& tuning() {
         x.col_dynamic = env_int("SDP_COL_DYNAMIC", 1) != 0;
         x.col_prune = env_int("SDP_COL_PRUNE", 1) != 0;
         x.col_prune_stats = 0;
+        x.col_groups = env_int("SDP_COL_GROUPS", 1) != 0;
         x.dbg_exchange = 0;
         x.pdl = env_int("SDP_PDL", 1) != 0;
         x.small_combine = env_int("SDP_SMALL_COMBINE", 1) != 0;
@@ -1153,6 +1163,7 @@ extern "C" int sdp_set_option(const char* name, int value) {
     else if (!strcmp(name, "col_dynamic")) t.col_dynamic = value != 0;
     else if (!strcmp(name, "col_prune")) t.col_prune = value != 0;
     else if (!strcmp(name, "col_prune_stats")) t.col_prune_stats = value != 0;
+    else if (!strcmp(name, "col_groups")) t.col_groups = value != 0;
     else if (!strcmp(name, "dbg_exchange")) t.dbg_exchange = value;
     else if (!strcmp(name, "pdl")) t.pdl = value != 0;
     else if (!strcmp(name, "small_combine")) t.small_combine = value != 0;
@@ -1910,6 +1921,239 @@ __device__ __forceinline__ bool column_skip(double2 b, double g, double l, doubl
     return (l >= 0.0) & (l <= 1.0) & (ga <= 0x1p1000) & (lb > best);
 }
 
+// Group skipping (sdp_column_groups_build, DESIGN.md section 4).  The controls of a work item are
+// cut into groups of K; for each (item, group, lane) a 16-byte summary of the lane's live controls
+// of the group: .x = gmin = min g, .y = bits [0,32) gabs >= max |g| (fp32 rounded up), [32,48)
+// qlo, [48,64) qhi (lowest / highest table row).  qlo = 0xffff: no live control; qhi = 0xffff:
+// not eligible (a weight outside [0, 1], a NaN in g, or a row past rows-2).  With
+// m_lo <= min m(q) over [qlo, qhi] and Acol >= A(q) over rows 0..rows-2, the group's lb and
+// margin bound those of column_skip for every member, so a group skip implies that column_skip
+// skips each member.  Twin: tablebuild.column_group_skip.
+__device__ __forceinline__ bool column_group_skip(double gmin, double gabs, double m_lo, double acol,
+                                                  double sum_p, double best) {
+    const double ga = add_(gabs, acol);
+    const double margin = add_(mul_(mul_(ga, sum_p), 0x1p-48), 0x1p-1000);
+    const double lb = sub_(add_(mul_(gmin, sum_p), m_lo), margin);
+    return (ga <= 0x1p1000) & (lb > best);
+}
+// Wm[q] = min m over [q, min(q+L, rows-1)): the minimum over [qlo, qhi] is that of two windows
+// when the span is at most 2L (a superset's, still a lower bound, below L); wider spans need
+// the group
+__device__ __forceinline__ bool column_group_need(double2 s, const double* Wm, int L, double acol,
+                                                  double sum_p, double best) {
+    const unsigned long long y = (unsigned long long)__double_as_longlong(s.y);
+    const int lo = (int)((y >> 32) & 0xffffu), hi = (int)(y >> 48);
+    if (lo == 0xffff) return false;
+    if (hi - lo >= 2 * L) return true;
+    const double m = fmin(Wm[lo], Wm[max(lo, hi - L + 1)]);
+    return !column_group_skip(s.x, (double)__uint_as_float((uint32_t)y), m, acol, sum_p, best);
+}
+
+#define SDP_CG_HIST_BYTES 256      // head of the summary buffer: histogram of the spans (32 x uint64)
+#define SDP_CG_MAX_K 64
+// one warp per item; also counts the spans qhi-qlo+1 of the eligible summaries by ceil(log2)
+__global__ void __launch_bounds__(256)
+k_column_groups(SdpTables T, double inv_stride0, int rows, int K, const int64_t* __restrict__ gbase,
+                double2* __restrict__ ent, unsigned long long* __restrict__ hist) {
+    __shared__ unsigned int h_sh[32];
+    if (threadIdx.x < 32) h_sh[threadIdx.x] = 0;
+    __syncthreads();
+    const int lane = threadIdx.x & 31;
+    const int64_t item = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (item < T.n_items) {
+        const SdpItem it = T.items[item];
+        const int Us = T.U[(int64_t)it.state * 32 + lane];
+        const int ng = (it.u_count + K - 1) / K;
+        for (int gi = 0; gi < ng; ++gi) {
+            double gmin = CUDART_INF, gabs = 0.0;
+            int qlo = INT_MAX, qhi = -1;
+            bool live = false, ok = true;
+            for (int j = 0; j < K; ++j) {
+                const int uu = gi * K + j;
+                if (uu >= it.u_count || it.u_begin + uu >= Us) break;
+                const int64_t o = it.entry_base + (int64_t)uu * 32 + lane;
+                const double gv = T.g[o], l = T.lam[o];
+                // (the row exactly as the sweep computes it)
+                const int q = __double2int_rn(__dmul_rn((double)T.cell[o], inv_stride0));
+                live = true;
+                gmin = fmin(gmin, gv);
+                gabs = fmax(gabs, fabs(gv));
+                qlo = min(qlo, q);
+                qhi = max(qhi, q);
+                ok &= (l >= 0.0) & (l <= 1.0) & (gv == gv);
+            }
+            unsigned long long y;
+            if (!live) {
+                y = 0xffffull << 32;
+                gmin = 0.0;
+            } else if (!ok || qlo < 0 || qhi > rows - 2) {
+                y = (0xffffull << 48) | __float_as_uint(CUDART_INF_F);
+            } else {
+                y = ((unsigned long long)qhi << 48) | ((unsigned long long)qlo << 32) |
+                    __float_as_uint(__double2float_ru(gabs));
+                atomicAdd(&h_sh[32 - __clz(qhi - qlo)], 1u);        // span <= 2^bucket
+            }
+            ent[(gbase[item] + gi) * 32 + lane] = make_double2(gmin, __longlong_as_double((long long)y));
+        }
+    }
+    __syncthreads();
+    if (threadIdx.x < 32 && h_sh[threadIdx.x]) atomicAdd(hist + threadIdx.x, (unsigned long long)h_sh[threadIdx.x]);
+}
+
+// summaries registered by sdp_column_groups_build, keyed on the u-part of the tables (a copy of
+// SdpTables with other item ranges, such as a column piece, finds them); a table build (K0)
+// that writes a registered u-part drops the registration
+struct ColGroupsReg {
+    int64_t id;
+    const void *items, *cell, *lam, *g;
+    int64_t n_items;
+    int rows, stride0, K, L;
+    const int64_t* gbase;
+    const double2* ent;
+};
+struct ColGroups {             // kernel argument; ent == nullptr: no group skipping
+    const int64_t* gbase;
+    const double2* ent;
+    int K, L;
+};
+static std::mutex g_cg_mu;
+static std::vector<ColGroupsReg> g_cg;
+static int64_t g_cg_next = 1;
+static void column_groups_drop(const void* cell, const void* lam, const void* g) {
+    std::lock_guard<std::mutex> lk(g_cg_mu);
+    for (size_t k = 0; k < g_cg.size();)
+        if (g_cg[k].cell == cell || g_cg[k].lam == lam || g_cg[k].g == g) g_cg.erase(g_cg.begin() + k);
+        else ++k;
+}
+static ColGroups column_groups_find(const GridT<double>& G, const SdpTables& T) {
+    ColGroups c;
+    memset(&c, 0, sizeof(c));
+    std::lock_guard<std::mutex> lk(g_cg_mu);
+    for (const ColGroupsReg& r : g_cg)
+        if (r.items == T.items && r.cell == T.cell && r.lam == T.lam && r.g == T.g && r.n_items == T.n_items &&
+            r.rows == G.order[0] && r.stride0 == G.stride[0]) {
+            c.gbase = r.gbase;
+            c.ent = r.ent;
+            c.K = r.K;
+            c.L = r.L;
+        }
+    return c;
+}
+
+// the first group of every item (prefix sums of ceil(u_count / K), from a host copy of the items)
+// and the bytes of the summary buffer
+static int column_groups_layout(const SdpTables* tab, int K, cudaStream_t st, std::vector<int64_t>* gbase,
+                                int64_t* bytes, const char* what) {
+    if (!tab || !bytes) return fail(SDP_EINVAL, "%s: NULL pointer", what);
+    if (tab->layout != SDP_LAYOUT_COLUMN_FACTORED || tab->col_pairs || !tab->items || tab->n_items < 0)
+        return fail(SDP_EINVAL, "%s: needs layout CF tables with one row per lane", what);
+    if (K < 4 || K > SDP_CG_MAX_K || (K & 3)) return fail(SDP_EINVAL, "%s: K must be a multiple of 4 in 4..64", what);
+    std::vector<SdpItem> items((size_t)tab->n_items);
+    cudaError_t e = cudaStreamSynchronize(st);
+    if (e == cudaSuccess && tab->n_items)
+        e = cudaMemcpy(items.data(), tab->items, sizeof(SdpItem) * (size_t)tab->n_items, cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) return fail(SDP_ECUDA, what, cudaGetErrorString(e));
+    gbase->assign((size_t)tab->n_items + 1, 0);
+    for (int64_t k = 0; k < tab->n_items; ++k)
+        (*gbase)[k + 1] = (*gbase)[k] + (items[k].u_count + K - 1) / K;
+    *bytes = SDP_CG_HIST_BYTES + ((8 * tab->n_items + 15) & ~(int64_t)15) + (*gbase)[tab->n_items] * 32 * 16;
+    return SDP_OK;
+}
+
+extern "C" int sdp_column_groups_bytes(const SdpTables* tab, int32_t K, void* stream, int64_t* bytes) {
+    std::vector<int64_t> gbase;
+    return column_groups_layout(tab, K, (cudaStream_t)stream, &gbase, bytes, "sdp_column_groups_bytes: %s");
+}
+
+extern "C" int sdp_column_groups_build(const SdpGrid* grid, const SdpTables* tab, int32_t K, void* buf,
+                                       int64_t bytes, void* stream, int64_t* id) {
+    const char* what = "sdp_column_groups_build: %s";
+    if (!grid || !id) return fail(SDP_EINVAL, what, "NULL pointer");
+    *id = 0;
+    GridT<double> G;
+    int rc = make_grid<double>(grid, &G, nullptr);
+    if (rc) return rc;
+    cudaStream_t st = (cudaStream_t)stream;
+    std::vector<int64_t> gbase;
+    int64_t need = 0;
+    rc = column_groups_layout(tab, K, st, &gbase, &need, what);
+    if (rc) return rc;
+    if (!buf || ((uintptr_t)buf & 15) || bytes < need) return fail(SDP_EINVAL, what, "buffer missing, misaligned or too small");
+    const int rows = G.order[0];
+    if (rows >= 0xffff) return fail(SDP_EINVAL, what, "more than 65534 rows on axis 0");
+    column_groups_drop(tab->cell, tab->lam, tab->g);
+    unsigned long long* hist = reinterpret_cast<unsigned long long*>(buf);
+    int64_t* gb = reinterpret_cast<int64_t*>(reinterpret_cast<unsigned char*>(buf) + SDP_CG_HIST_BYTES);
+    double2* ent = reinterpret_cast<double2*>(reinterpret_cast<unsigned char*>(buf) + SDP_CG_HIST_BYTES +
+                                              ((8 * tab->n_items + 15) & ~(int64_t)15));
+    cudaError_t e = cudaMemsetAsync(hist, 0, SDP_CG_HIST_BYTES, st);
+    if (e == cudaSuccess && tab->n_items)
+        e = cudaMemcpyAsync(gb, gbase.data(), 8 * (size_t)tab->n_items, cudaMemcpyHostToDevice, st);
+    if (e != cudaSuccess) return fail(SDP_ECUDA, what, cudaGetErrorString(e));
+    if (tab->n_items) {
+        const int64_t blocks = (tab->n_items + 7) / 8;
+        k_column_groups<<<(unsigned)blocks, 256, 0, st>>>(*tab, 1.0 / (double)G.stride[0], rows, K, gb, ent, hist);
+        SDP_LAUNCH_CHECK();
+    }
+    unsigned long long h[32];
+    e = cudaMemcpyAsync(h, hist, sizeof(h), cudaMemcpyDeviceToHost, st);
+    if (e == cudaSuccess) e = cudaStreamSynchronize(st);
+    if (e != cudaSuccess) return fail(SDP_ECUDA, what, cudaGetErrorString(e));
+    // window length L: the smallest power of two whose 2L covers the spans of 90 % of the
+    // eligible summaries (at most 64: the windows are built per column in shared memory)
+    unsigned long long total = 0, cum = 0;
+    for (int b = 0; b < 32; ++b) total += h[b];
+    int L = 1;
+    for (int b = 0; b < 32 && total; ++b) {
+        cum += h[b];
+        if (cum * 10 >= total * 9) {
+            L = b > 1 ? 1 << (b - 1) : 1;
+            break;
+        }
+    }
+    L = L > 64 ? 64 : L;
+    ColGroupsReg r;
+    r.items = tab->items;
+    r.cell = tab->cell;
+    r.lam = tab->lam;
+    r.g = tab->g;
+    r.n_items = tab->n_items;
+    r.rows = rows;
+    r.stride0 = G.stride[0];
+    r.K = K;
+    r.L = L;
+    r.gbase = gb;
+    r.ent = ent;
+    std::lock_guard<std::mutex> lk(g_cg_mu);
+    r.id = g_cg_next++;
+    g_cg.push_back(r);
+    *id = r.id;
+    return SDP_OK;
+}
+
+extern "C" int sdp_column_groups_release(int64_t id) {
+    std::lock_guard<std::mutex> lk(g_cg_mu);
+    for (size_t k = 0; k < g_cg.size(); ++k)
+        if (g_cg[k].id == id) {
+            g_cg.erase(g_cg.begin() + k);
+            break;
+        }
+    return SDP_OK;
+}
+
+// the window length of a registered summary (0: none), for measurements and tests
+extern "C" int sdp_column_groups_info(int64_t id, int32_t* K, int32_t* L) {
+    if (!K || !L) return fail(SDP_EINVAL, "%s", "sdp_column_groups_info: NULL pointer");
+    *K = *L = 0;
+    std::lock_guard<std::mutex> lk(g_cg_mu);
+    for (const ColGroupsReg& r : g_cg)
+        if (r.id == id) {
+            *K = r.K;
+            *L = r.L;
+        }
+    return SDP_OK;
+}
+
 #define SDP_CT_ROWS 16
 // `WAIT`: every CTA first waits (lanes 0..world-1, ld.acquire.sys on the local flags) until all
 // ranks have published the current epoch, i.e. until the J slabs of the previous sweep have
@@ -2041,13 +2285,19 @@ static int launch_column_table(const GridT<double>& G, const SdpTables& T, const
 // chose in the previous sweep (part_idx, when it is a control of the item), so that the best
 // is good from the first group on.  The minimum over the controls, ties to the lowest index
 // (`better`), does not depend on the order they are visited in: the results are those of
-// PRUNE = false, bit for bit.  `stats` (optional): warp steps met and skipped.
-template <int D, int WM, int UB, int PF, bool FULL, int MAXT, bool PRUNE>     // FULL: W == WM, every slot live
+// PRUNE = false, bit for bit.  `stats` (optional): warp steps met and skipped, groups met and
+// skipped.  PRUNE with CG.ent: the controls are walked by groups of CG.K (column_group_need, the
+// window minima Wm behind the bound in shared memory); the summaries of the next SDP_CG_DEPTH
+// groups are in flight, and a group that no lane needs is passed over without touching its
+// (x,u) stream.  The next surviving group is found (with the best values so far) before the
+// current one is evaluated, so that its first loads are issued behind the current group's.
+#define SDP_CG_DEPTH 2
+template <int D, int WM, int UB, int PF, bool FULL, int MAXT, bool PRUNE, bool GR = false>     // FULL: W == WM, every slot live
 __global__ void __launch_bounds__(MAXT, 1)
 k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jprev,
                     double* __restrict__ part_val, int32_t* __restrict__ part_idx,
                     double inv_stride0, PVals PV, int64_t pitch, int prepass, int dynamic,
-                    double sum_p, unsigned long long* __restrict__ stats) {
+                    double sum_p, unsigned long long* __restrict__ stats, ColGroups CG) {
     constexpr int NW = D - 1;
     extern __shared__ __align__(128) unsigned char csm[];
     __shared__ int next_item[2];                        // dynamic hand-out of the items of a column (two, used in turn)
@@ -2056,6 +2306,8 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
     __shared__ int cw_sh[WM];
     __shared__ double lw_sh[NW][WM];
     __shared__ __align__(8) uint64_t tbar;              // completion of the bulk copy of a table
+    __shared__ double acol_sh[32];                      // CG: per-warp maxima of A
+    double* Wm_sh = reinterpret_cast<double*>(csm + pitch * 8 + (int64_t)G.order[0] * 16);     // CG: [order[0]]
     uint32_t tphase = 0;
     if (threadIdx.x == 0) {
         mbar_init(smem_u32(&tbar), 1);
@@ -2152,6 +2404,35 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
             }
         }
         if (prepass < 2) __syncthreads();
+        double acol = 0.0;
+        if (GR) {
+            // the window minima of m and Acol = max A over rows 0..rows-2 (NaN when one is NaN)
+            if (!have_table) {
+                mbar_wait(smem_u32(&tbar), tphase);
+                have_table = true;
+            }
+            const int L = CG.L;
+            double a = 0.0;
+            bool nan = false;
+            for (int q = threadIdx.x; q < rows - 1; q += blockDim.x) {
+                const int qe = min(q + L, rows - 1);
+                double m = B_sh[q].x;
+                for (int r = q + 1; r < qe; ++r) m = fmin(m, B_sh[r].x);
+                Wm_sh[q] = m;
+                const double aq = B_sh[q].y;
+                nan |= aq != aq;
+                a = fmax(a, aq);
+            }
+#pragma unroll
+            for (int o = 16; o; o >>= 1) a = fmax(a, __shfl_xor_sync(0xffffffffu, a, o));
+            nan = __any_sync(0xffffffffu, nan);
+            if (lane == 0) acol_sh[warp] = nan ? CUDART_NAN : a;
+            __syncthreads();
+            for (int k = 0; k < nwarps; ++k) {
+                const double x = acol_sh[k];
+                acol = (x != x || acol != acol) ? CUDART_NAN : fmax(acol, x);
+            }
+        }
 
         // the warps share the items of the column: round-robin, or (dynamic) first come first
         // served - the items differ in length and a column piece may hold only a few of them
@@ -2187,21 +2468,34 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
                     l_s = lup[o];
                 }
             }
-            int n_steps = 0, n_skipped = 0;
+            int n_steps = 0, n_skipped = 0, n_groups = 0, n_gskipped = 0;
+            constexpr bool grp = GR;
 
             // PF groups of UB controls are in flight: group k of the run sits in stage k % PF
             // (rows past the run repeat its last row)
             int c_n[PF][UB];
             double g_n[PF][UB], l_n[PF][UB];
-#pragma unroll
-            for (int s = 0; s < PF; ++s)
+            auto load_stage = [&](int s, int uu) {
 #pragma unroll
                 for (int b = 0; b < UB; ++b) {
-                    const int64_t o = (int64_t)min(s * UB + b, last) * 32;
+                    const int64_t o = (int64_t)min(uu + b, last) * 32;
                     c_n[s][b] = __ldcs(cup + o);
                     g_n[s][b] = __ldcs(gp + o);
                     l_n[s][b] = __ldcs(lup + o);
                 }
+            };
+            // CG: the summaries of groups gnext .. gnext+SDP_CG_DEPTH-1
+            const int ng = grp ? (it.u_count + CG.K - 1) / CG.K : 0;
+            const double2* __restrict__ sp = grp ? CG.ent + CG.gbase[item_id] * 32 + lane : nullptr;
+            double2 ring[SDP_CG_DEPTH];
+            if (grp) {
+#pragma unroll
+                for (int r = 0; r < SDP_CG_DEPTH; ++r)
+                    if (r < ng) ring[r] = __ldcs(sp + (int64_t)r * 32);
+            } else {
+#pragma unroll
+                for (int s = 0; s < PF; ++s) load_stage(s, s * UB);
+            }
             if (!have_table) {           // (warp-uniform; first item of the run only)
                 mbar_wait(smem_u32(&tbar), tphase);
                 have_table = true;
@@ -2224,66 +2518,107 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
                     best_i = seed;
                 }
             }
-            for (int uu0 = 0; uu0 < it.u_count; uu0 += UB * PF) {
+            // one warp step: the UB controls uu.. of stage s; then stage s takes position `pre`
+            // (< 0: nothing more to load)
+            auto step = [&](int s, int uu, int pre) {
+                double gv[UB], lu[UB], oml[UB];
+                const double* Ra[UB];
+                bool need = !PRUNE;
 #pragma unroll
-                for (int s = 0; s < PF; ++s) {
-                    const int uu = uu0 + s * UB;
-                    if (uu < it.u_count) {                    // warp-uniform
-                        double gv[UB], lu[UB], oml[UB];
-                        const double* Ra[UB];
-                        bool need = !PRUNE;
+                for (int b = 0; b < UB; ++b) {
+                    gv[b] = g_n[s][b];
+                    lu[b] = l_n[s][b];
+                    oml[b] = sub_(1.0, lu[b]);
+                    // row q0 = cell_u / stride0 exactly (cell_u is a multiple of stride0
+                    // below 2^31; padding entries hold cell 0)
+                    const int q = __double2int_rn(__dmul_rn((double)c_n[s][b], inv_stride0));
+                    Ra[b] = R_sh + q * P;
+                    // (padding lanes and rows past the run never need a control)
+                    if (PRUNE && uu + b <= last && it.u_begin + uu + b < Us)
+                        need |= !column_skip(B_sh[q], gv[b], lu[b], sum_p, best_v);
+                }
+                if (pre >= 0) load_stage(s, pre);
+                if (PRUNE) {
+                    ++n_steps;
+                    if (!__any_sync(0xffffffffu, need)) {
+                        ++n_skipped;
+                        return;
+                    }
+                }
+                // slots >= W read past the W live values of a row (its pad, the next row,
+                // or the slack behind the table) and are discarded below: no guards
+                double v[UB][WM];
 #pragma unroll
-                        for (int b = 0; b < UB; ++b) {
-                            gv[b] = g_n[s][b];
-                            lu[b] = l_n[s][b];
-                            oml[b] = sub_(1.0, lu[b]);
-                            // row q0 = cell_u / stride0 exactly (cell_u is a multiple of stride0
-                            // below 2^31; padding entries hold cell 0)
-                            const int q = __double2int_rn(__dmul_rn((double)c_n[s][b], inv_stride0));
-                            Ra[b] = R_sh + q * P;
-                            // (padding lanes and rows past the run never need a control)
-                            if (PRUNE && uu + b <= last && it.u_begin + uu + b < Us)
-                                need |= !column_skip(B_sh[q], gv[b], lu[b], sum_p, best_v);
+                for (int b = 0; b < UB; ++b)
+#pragma unroll
+                    for (int w = 0; w < WM; ++w)
+                        v[b][w] = add_(mul_(oml[b], Ra[b][w]), mul_(lu[b], Ra[b][P + w]));
+#pragma unroll
+                for (int b = 0; b < UB; ++b) {
+                    double acc = 0.0;
+#pragma unroll
+                    for (int w = 0; w < WM; ++w) {
+                        const double jg = add_(gv[b], v[b][w]);
+                        const double nxt = T.expect ? add_(acc, mul_(jg, PV.v[w])) : jg;
+                        acc = (FULL || w < W) ? nxt : acc;   // slots past W do not take part
+                    }
+                    const int u = it.u_begin + uu + b;
+                    if (uu + b <= last && u < Us && better(acc, u, best_v, best_i)) {
+                        best_v = acc;
+                        best_i = u;
+                    }
+                }
+            };
+            if (grp) {
+                // the next group that some lane needs (judged with the best values so far: they
+                // only decrease, so a skip stays valid); the ones passed over count as skipped
+                // warp steps
+                int gnext = 0;
+                auto survivor = [&]() -> int {
+                    while (gnext < ng) {
+                        const double2 sm = ring[0];
+#pragma unroll
+                        for (int r = 0; r + 1 < SDP_CG_DEPTH; ++r) ring[r] = ring[r + 1];
+                        if (gnext + SDP_CG_DEPTH < ng) ring[SDP_CG_DEPTH - 1] = __ldcs(sp + (int64_t)(gnext + SDP_CG_DEPTH) * 32);
+                        const int gi = gnext++;
+                        ++n_groups;
+                        if (__any_sync(0xffffffffu, column_group_need(sm, Wm_sh, CG.L, acol, sum_p, best_v)))
+                            return gi;
+                        const int nsteps = (min(CG.K, it.u_count - gi * CG.K) + UB - 1) / UB;
+                        ++n_gskipped;
+                        n_steps += nsteps;
+                        n_skipped += nsteps;
+                    }
+                    return -1;
+                };
+                int cur = survivor();
+                if (cur >= 0) {
+#pragma unroll
+                    for (int s = 0; s < PF; ++s) load_stage(s, cur * CG.K + s * UB);
+                }
+                while (cur >= 0) {
+                    const int nxt = survivor();
+                    // (K is a multiple of UB*PF: only the item's last group ends early, and no
+                    // group follows it)
+                    const int a = cur * CG.K, bend = min(a + CG.K, it.u_count);
+                    for (int uu0 = a; uu0 < bend; uu0 += UB * PF) {
+#pragma unroll
+                        for (int s = 0; s < PF; ++s) {
+                            const int uu = uu0 + s * UB;
+                            const int p = uu + UB * PF;
+                            if (uu < bend)                    // warp-uniform
+                                step(s, uu, p < bend ? p : (nxt >= 0 ? nxt * CG.K + (p - bend) : -1));
                         }
-                        if (uu + UB * PF < it.u_count) {
+                    }
+                    cur = nxt;
+                }
+            } else {
+                for (int uu0 = 0; uu0 < it.u_count; uu0 += UB * PF) {
 #pragma unroll
-                            for (int b = 0; b < UB; ++b) {
-                                const int64_t o = (int64_t)min(uu + UB * PF + b, last) * 32;
-                                c_n[s][b] = __ldcs(cup + o);
-                                g_n[s][b] = __ldcs(gp + o);
-                                l_n[s][b] = __ldcs(lup + o);
-                            }
-                        }
-                        if (PRUNE) {
-                            ++n_steps;
-                            if (!__any_sync(0xffffffffu, need)) {
-                                ++n_skipped;
-                                continue;
-                            }
-                        }
-                        // slots >= W read past the W live values of a row (its pad, the next row,
-                        // or the slack behind the table) and are discarded below: no guards
-                        double v[UB][WM];
-#pragma unroll
-                        for (int b = 0; b < UB; ++b)
-#pragma unroll
-                            for (int w = 0; w < WM; ++w)
-                                v[b][w] = add_(mul_(oml[b], Ra[b][w]), mul_(lu[b], Ra[b][P + w]));
-#pragma unroll
-                        for (int b = 0; b < UB; ++b) {
-                            double acc = 0.0;
-#pragma unroll
-                            for (int w = 0; w < WM; ++w) {
-                                const double jg = add_(gv[b], v[b][w]);
-                                const double nxt = T.expect ? add_(acc, mul_(jg, PV.v[w])) : jg;
-                                acc = (FULL || w < W) ? nxt : acc;   // slots past W do not take part
-                            }
-                            const int u = it.u_begin + uu + b;
-                            if (uu + b <= last && u < Us && better(acc, u, best_v, best_i)) {
-                                best_v = acc;
-                                best_i = u;
-                            }
-                        }
+                    for (int s = 0; s < PF; ++s) {
+                        const int uu = uu0 + s * UB;
+                        if (uu < it.u_count)                  // warp-uniform
+                            step(s, uu, uu + UB * PF < it.u_count ? uu + UB * PF : -1);
                     }
                 }
             }
@@ -2292,6 +2627,10 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
             if (PRUNE && stats && lane == 0) {
                 atomicAdd(stats, (unsigned long long)n_steps);
                 atomicAdd(stats + 1, (unsigned long long)n_skipped);
+                if (grp) {
+                    atomicAdd(stats + 2, (unsigned long long)n_groups);
+                    atomicAdd(stats + 3, (unsigned long long)n_gskipped);
+                }
             }
         }
         if (prepass >= 2) {
@@ -2305,58 +2644,66 @@ k_sweep_fact_column(GridT<double> G, SdpTables T, const double* __restrict__ Jpr
     }
 }
 
-// pruning sweep: warp steps met / skipped, counted with "col_prune_stats" (sdp_col_prune_counts)
+// pruning sweep: warp steps met / skipped, groups met / skipped, counted with "col_prune_stats"
+// (sdp_col_prune_counts, sdp_col_group_counts)
 static unsigned long long* g_prune_stats = nullptr;
-extern "C" int sdp_col_prune_counts(int64_t* steps, int64_t* skipped) {
-    if (!steps || !skipped) return fail(SDP_EINVAL, "%s", "sdp_col_prune_counts: NULL pointer");
-    *steps = *skipped = 0;
+static int read_prune_stats(int k, int64_t* a, int64_t* b, const char* what) {
+    if (!a || !b) return fail(SDP_EINVAL, "%s: NULL pointer", what);
+    *a = *b = 0;
     if (!g_prune_stats) return SDP_OK;
     unsigned long long h[2];
     cudaError_t e = cudaDeviceSynchronize();
-    if (e == cudaSuccess) e = cudaMemcpy(h, g_prune_stats, sizeof(h), cudaMemcpyDeviceToHost);
-    if (e == cudaSuccess) e = cudaMemset(g_prune_stats, 0, sizeof(h));
-    if (e != cudaSuccess) return fail(SDP_ECUDA, "sdp_col_prune_counts: %s", cudaGetErrorString(e));
-    *steps = (int64_t)h[0];
-    *skipped = (int64_t)h[1];
+    if (e == cudaSuccess) e = cudaMemcpy(h, g_prune_stats + k, sizeof(h), cudaMemcpyDeviceToHost);
+    if (e == cudaSuccess) e = cudaMemset(g_prune_stats + k, 0, sizeof(h));
+    if (e != cudaSuccess) return fail(SDP_ECUDA, what, cudaGetErrorString(e));
+    *a = (int64_t)h[0];
+    *b = (int64_t)h[1];
     return SDP_OK;
 }
+extern "C" int sdp_col_prune_counts(int64_t* steps, int64_t* skipped) {
+    return read_prune_stats(0, steps, skipped, "sdp_col_prune_counts: %s");
+}
+extern "C" int sdp_col_group_counts(int64_t* groups, int64_t* skipped) {
+    return read_prune_stats(2, groups, skipped, "sdp_col_group_counts: %s");
+}
 
-template <int D, int WM, int UB, int PF, int MAXT, bool PRUNE>
+template <int D, int WM, int UB, int PF, int MAXT, bool PRUNE, bool GR = false>
 static int set_column_attrs(size_t shm) {
     static size_t attr_set = 0;          // per instantiation
     if (attr_set >= shm) return SDP_OK;
-    cudaError_t e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE>,
+    cudaError_t e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE, GR>,
                                          cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm);
     if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE>,
+        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE, GR>,
                                  cudaFuncAttributeMaxDynamicSharedMemorySize, (int)shm);
     // the largest shared-memory carve-out (the kernel streams with evict-first loads: 2 % L1 hit
     // rate): k_combine_column_small asks for the same one, so that one of its CTAs can join a
     // resident CTA of this kernel without the SM draining to change its configuration
     if (e == cudaSuccess && tuning().carveout)
-        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE>,
+        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE, GR>,
                                  cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     if (e == cudaSuccess && tuning().carveout)
-        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE>,
+        e = cudaFuncSetAttribute(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE, GR>,
                                  cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return fail(SDP_ECUDA, "cudaFuncSetAttribute: %s", cudaGetErrorString(e));
     attr_set = shm;
     return SDP_OK;
 }
 
-template <int D, int WM, int UB, int PF, int MAXT, bool PRUNE>
+template <int D, int WM, int UB, int PF, int MAXT, bool PRUNE, bool GR = false>
 static void launch_fact_column_kp(const GridT<double>& G, const SdpTables& T, const double* Jprev,
                                   double* part_val, int32_t* part_idx, cudaStream_t st, int threads, size_t shm,
-                                  int64_t pitch, int prepass, double sum_p, unsigned long long* stats) {
+                                  int64_t pitch, int prepass, double sum_p, unsigned long long* stats,
+                                  ColGroups cg) {
     const PVals pv = column_pvals(T);
     const double inv0 = 1.0 / (double)G.stride[0];
     const int dynamic = (T.col_launch_hint & 0xffff) ? !((T.col_launch_hint >> 16) & 1) : tuning().col_dynamic;
     if (T.W == WM)
-        launch_pdl(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE>, dim3((unsigned)T.n_segs), dim3(threads),
-                   shm, st, G, T, Jprev, part_val, part_idx, inv0, pv, pitch, prepass, dynamic, sum_p, stats);
+        launch_pdl(k_sweep_fact_column<D, WM, UB, PF, true, MAXT, PRUNE, GR>, dim3((unsigned)T.n_segs), dim3(threads),
+                   shm, st, G, T, Jprev, part_val, part_idx, inv0, pv, pitch, prepass, dynamic, sum_p, stats, cg);
     else
-        launch_pdl(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE>, dim3((unsigned)T.n_segs), dim3(threads),
-                   shm, st, G, T, Jprev, part_val, part_idx, inv0, pv, pitch, prepass, dynamic, sum_p, stats);
+        launch_pdl(k_sweep_fact_column<D, WM, UB, PF, false, MAXT, PRUNE, GR>, dim3((unsigned)T.n_segs), dim3(threads),
+                   shm, st, G, T, Jprev, part_val, part_idx, inv0, pv, pitch, prepass, dynamic, sum_p, stats, cg);
 }
 
 template <int D, int WM, int UB, int PF, int MAXT>
@@ -2371,15 +2718,25 @@ static int launch_fact_column_k(const GridT<double>& G, const SdpTables& T, cons
         if (rc) return rc;
     }
     const bool prune = tuning().col_prune && column_bound_on(G, T);
-    const size_t shm = (size_t)pitch * 8 + (prune ? (size_t)G.order[0] * 16 : 0);
-    int rc = prune ? set_column_attrs<D, WM, UB, PF, MAXT, true>(shm) : set_column_attrs<D, WM, UB, PF, MAXT, false>(shm);
+    size_t shm = (size_t)pitch * 8 + (prune ? (size_t)G.order[0] * 16 : 0);
+    // group skipping: summaries registered for these tables, and room for the window minima
+    ColGroups cg;
+    memset(&cg, 0, sizeof(cg));
+    // (compiled for the CTA shapes of up to 640 threads: the 85 registers of 768 leave no room)
+    if (MAXT <= 640 && prune && tuning().col_groups && shm + (size_t)G.order[0] * 8 <= SDP_COLUMN_MAX_SMEM_BYTES) {
+        cg = column_groups_find(G, T);
+        if (cg.ent) shm += (size_t)G.order[0] * 8;
+    }
+    constexpr bool GR_OK = MAXT <= 640;
+    int rc = cg.ent ? set_column_attrs<D, WM, UB, PF, MAXT, true, GR_OK>(shm)
+                    : prune ? set_column_attrs<D, WM, UB, PF, MAXT, true>(shm) : set_column_attrs<D, WM, UB, PF, MAXT, false>(shm);
     if (rc) return rc;
     if (prune) {
         unsigned long long* stats = nullptr;
         if (tuning().col_prune_stats) {
             if (!g_prune_stats) {
-                cudaError_t e = cudaMalloc(&g_prune_stats, 2 * sizeof(unsigned long long));
-                if (e == cudaSuccess) e = cudaMemset(g_prune_stats, 0, 2 * sizeof(unsigned long long));
+                cudaError_t e = cudaMalloc(&g_prune_stats, 4 * sizeof(unsigned long long));
+                if (e == cudaSuccess) e = cudaMemset(g_prune_stats, 0, 4 * sizeof(unsigned long long));
                 if (e != cudaSuccess) {
                     g_prune_stats = nullptr;
                     return fail(SDP_ECUDA, "col_prune_stats: %s", cudaGetErrorString(e));
@@ -2390,15 +2747,20 @@ static int launch_fact_column_k(const GridT<double>& G, const SdpTables& T, cons
         const PVals pv = column_pvals(T);
         double sum_p = 0.0;                  // (in w order: tablebuild.column_prune_skip)
         for (int w = 0; w < T.W; ++w) sum_p += pv.v[w];
-        launch_fact_column_kp<D, WM, UB, PF, MAXT, true>(G, T, Jprev, part_val, part_idx, st, threads, shm, pitch,
-                                                         prepass, sum_p, stats);
+        if (cg.ent)
+            launch_fact_column_kp<D, WM, UB, PF, MAXT, true, GR_OK>(G, T, Jprev, part_val, part_idx, st, threads, shm,
+                                                                    pitch, prepass, sum_p, stats, cg);
+        else
+            launch_fact_column_kp<D, WM, UB, PF, MAXT, true>(G, T, Jprev, part_val, part_idx, st, threads, shm, pitch,
+                                                             prepass, sum_p, stats, cg);
     } else {
         launch_fact_column_kp<D, WM, UB, PF, MAXT, false>(G, T, Jprev, part_val, part_idx, st, threads, shm, pitch,
-                                                          prepass, 0.0, nullptr);
+                                                          prepass, 0.0, nullptr, cg);
     }
     note_kernel("%sk_sweep_fact_column<%d,%d,%d,%d,%s,%d%s> [%d CTAs x %d threads]",
                 (prepass && !T.col_table_ready) ? "k_column_table + " : "", D, WM, UB, PF,
-                T.W == WM ? "true" : "false", MAXT, prune ? ",prune" : "", (int)T.n_segs, threads);
+                T.W == WM ? "true" : "false", MAXT, cg.ent ? ",prune,groups" : (prune ? ",prune" : ""),
+                (int)T.n_segs, threads);
     SDP_LAUNCH_CHECK();
     return SDP_OK;
 }

@@ -19,6 +19,7 @@ Reference behaviour the tables reproduce: stodynprog/stodynprog.py:432-463 (cont
 import ctypes
 import os
 import time
+import weakref
 
 import numpy as np
 
@@ -35,6 +36,9 @@ COLUMN_HOIST_DEFAULT = os.environ.get("SDP_COLUMN_HOIST", "1") != "0"
 # against 0.233 ms per sweep for 1/8 of the grid, 0.61 against 0.65 ms for 1/2.  "auto" cuts
 # by columns whenever layout CF applies and every rank gets at least 4 columns.
 SLAB_AXIS_DEFAULT = os.environ.get("SDP_SLAB_AXIS", "auto")
+# layout CF, pruning sweep: controls per group of the group summaries (sdp_column_groups_build,
+# DESIGN.md section 4); 0 builds none.  A multiple of 4, at most 64.
+COLUMN_GROUP_K = int(os.environ.get("SDP_COLUMN_GROUP_K", "8"))
 # solver.column_pairs = "auto": layout CF with two rows per lane (3 shared-memory reads for 2
 # backups instead of 4).  OFF by default: measured on config #5 (profiles/r2_emu_variants_pairs.txt)
 # 1.58-1.67 ms per sweep against 1.15 ms with one row per lane.  The reads saved come back as bank
@@ -305,6 +309,92 @@ def column_prune_skip(g, lam, R0, R1, p, expect, best):
         return bool(0.0 <= lam <= 1.0 and ga <= 2.0 ** 1000 and lb > best)
 
 
+def column_group_skip(gmin, gabs, m_lo, acol, sum_p, best):
+    """Layout CF, group skipping: the decision of the column sweep for one lane and one group of
+    controls (twin of column_group_skip in the device code; DESIGN.md section 4).  `gmin` / `gabs`
+    the least stage cost and a bound of |g| over the lane's live controls of the group, `m_lo` a
+    lower bound of the row bound m(q) over their rows, `acol` the largest A(q) of the column's
+    rows 0..rows-2 (NaN when one is NaN), `sum_p` the sum of the probabilities in w order, `best`
+    the lane's best value so far.  The caller has checked that the group is eligible (every weight
+    in [0, 1], no NaN in g, every row <= rows-2).  True: column_prune_skip holds for every member."""
+    with np.errstate(invalid="ignore", over="ignore"):
+        ga = np.float64(gabs) + np.float64(acol)
+        margin = ga * np.float64(sum_p) * np.float64(2.0 ** -48) + np.float64(2.0 ** -1000)
+        lb = (np.float64(gmin) * np.float64(sum_p) + np.float64(m_lo)) - margin
+        return bool(ga <= 2.0 ** 1000 and lb > best)
+
+
+def column_group_summary(g, lam, q, live, rows):
+    """Layout CF, group skipping: the summary of one (item, group, lane) as the device builds it
+    (k_column_groups): g, lam and the table rows q of the group's K controls of the lane, `live`
+    which of them are live.  Returns (gmin, gabs, qlo, qhi): qlo = 0xffff when no control is live,
+    qhi = 0xffff when the group is not eligible; gabs is rounded up to fp32."""
+    g, lam = np.asarray(g, dtype=np.float64), np.asarray(lam, dtype=np.float64)
+    q, live = np.asarray(q, dtype=np.int64), np.asarray(live, dtype=bool)
+    if not live.any():
+        return 0.0, 0.0, 0xffff, 0
+    g, lam, q = g[live], lam[live], q[live]
+    ok = bool(np.all((lam >= 0.0) & (lam <= 1.0)) and not np.isnan(g).any() and q.min() >= 0 and q.max() <= rows - 2)
+    if not ok:
+        return float(np.fmin.reduce(np.append(g, np.inf))), float("inf"), 0, 0xffff
+    return float(g.min()), float_round_up(np.abs(g).max()), int(q.min()), int(q.max())
+
+
+def float_round_up(x):
+    """the least fp32 value >= x (inf above the largest finite fp32)"""
+    with np.errstate(over="ignore"):
+        f = np.float32(x)
+    if np.isfinite(f) and np.float64(f) < x:
+        f = np.nextafter(f, np.float32(np.inf))
+    return float(f)
+
+
+def window_minima(m, L):
+    """Wm[q] = min m over [q, min(q+L, rows-1)) for q < rows-1 (the last row's bound is the
+    sentinel and takes no part), NaN dropped as fmin does"""
+    m = np.asarray(m, dtype=np.float64)
+    n = len(m) - 1
+    return np.array([np.fmin.reduce(m[q:min(q + L, n)]) for q in range(n)])
+
+
+def group_row_bound(Wm, L, qlo, qhi):
+    """the lower bound of m over [qlo, qhi] the sweep uses, from the window minima (None: the span
+    exceeds 2L and the group is needed)"""
+    if qhi - qlo >= 2 * L:
+        return None
+    return float(np.fmin(Wm[qlo], Wm[max(qlo, qhi - L + 1)]))
+
+
+def build_column_groups(eng, T, K=None):
+    """Layout CF: build and register the group summaries of T's u-part (sdp_column_groups_build),
+    held by T.col_groups; the registration ends with release_column_groups or when T is collected.
+    Every path that rewrites T.cell / T.lam / T.g goes through a table build (sdp_build_tables*),
+    which also drops it."""
+    K = COLUMN_GROUP_K if K is None else K
+    release_column_groups(T)
+    if not K or not T.column or T.pairs:
+        return
+    lib, nb, gid = eng.lib, ctypes.c_int64(0), ctypes.c_int64(0)
+    _cabi.check(lib.sdp_column_groups_bytes(ctypes.byref(T.c_tables), K, eng.stream, ctypes.byref(nb)),
+                "sdp_column_groups_bytes")
+    T.col_groups = _torch().empty(max(int(nb.value), 16), dtype=_torch().uint8, device=eng.device)
+    _cabi.check(lib.sdp_column_groups_build(ctypes.byref(T.grid), ctypes.byref(T.c_tables), K,
+                                            eng._ptr(T.col_groups), int(nb.value), eng.stream, ctypes.byref(gid)),
+                "sdp_column_groups_build")
+    T.col_groups_id = int(gid.value)
+    T.col_groups_fin = weakref.finalize(T, lib.sdp_column_groups_release, int(gid.value))
+
+
+def release_column_groups(T):
+    """end the registration of T's group summaries and free them (before the tables are rewritten)"""
+    fin = getattr(T, "col_groups_fin", None)
+    if fin is not None:
+        fin()
+    T.col_groups_fin = None
+    T.col_groups = None
+    T.col_groups_id = 0
+
+
 def row_aligned(bounds, n_cols):
     """slab boundaries moved to the nearest multiple of n_cols (whole rows of axis 0),
     kept monotone"""
@@ -363,6 +453,9 @@ class SweepTables(object):
         self.item_u_count_host = None
         self.col_table = None      # device fp64 scratch: the column tables of the current sweep
         self.col_bound = None      # device fp64 scratch: their per-row bounds (SdpTables.col_bound)
+        self.col_groups = None     # device bytes: the registered group summaries (build_column_groups)
+        self.col_groups_id = 0
+        self.col_groups_fin = None
         self.run_end = None        # device int64 [n_items]: end of every item's (band, column) run
         self.pairs = False         # layout CF with two rows per lane (SdpTables.col_pairs)
         self.pos_row = self.work_dev = self.work_host = None
@@ -831,6 +924,7 @@ class ShardBuild(object):
         T = reuse if (reuse is not None and reuse.W == plan.W and reuse.d == plan.d
                       and reuse.tiled == self.tiled) else SweepTables()
         self.T = T
+        release_column_groups(T)       # (recycled tables: their entries are about to be rewritten)
         T.grid, T.d, T.W = plan.grid, plan.d, plan.W
         T.tiled = self.tiled
         T.expect = 1 if plan.nb_perturb >= 1 else 0
@@ -1158,6 +1252,8 @@ class ShardBuild(object):
         T.J_out = torch.empty(max(n, 1), dtype=torch.float64, device=dev)
         T.argmin = torch.empty(max(n, 1), dtype=torch.int32, device=dev)
         T.c_tables = fill_c_tables(T)
+        if T.column and plan.eng._cuda:
+            build_column_groups(plan.eng, T)
         # (kept for Engine.recursion_fast: one chunk, one flush, batched evaluation)
         T.build_record = None
         if plan.keep_staging and T.tabulate_mode == "batched" and len(self.flushes) == 1 \
