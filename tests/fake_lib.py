@@ -608,6 +608,137 @@ class FakeLib(object):
         self.launches += n_iter
         return 0
 
+    # -- the exchange over peer memory (SdpPeers): every rank's buffers are plain host memory here.
+    # The epoch / flag / done words are kept as the header says; a wait on a flag that is not yet
+    # published raises instead of spinning (the model runs the ranks one after the other).
+    @staticmethod
+    def _peers(pref):
+        P = pref._obj
+        assert 1 <= P.world <= _cabi.SDP_MAX_PEERS and 0 <= P.rank < P.world
+        assert P.epoch and P.done and all(P.flags[r] for r in range(P.world))
+        return P
+
+    @staticmethod
+    def _publish(P):
+        assert _arr(P.done, 1, ctypes.c_uint32)[0] == 0       # zero between launches
+        ep = _arr(P.epoch, 1, ctypes.c_uint64)
+        ep[0] += 1
+        for q in range(P.world):
+            _arr(P.flags[q], P.world, ctypes.c_uint64)[P.rank] = ep[0]
+
+    @staticmethod
+    def _wait(P, e=None):
+        e = int(_arr(P.epoch, 1, ctypes.c_uint64)[0]) if e is None else e
+        f = _arr(P.flags[P.rank], P.world, ctypes.c_uint64)
+        if not np.all(f >= e):
+            raise AssertionError("rank %d waits for epoch %d on flags %s" % (P.rank, e, list(f)))
+
+    def _store(self, P, dest, J_loc, a_loc):
+        """J_loc / a_loc (local states) -> grid states `dest` of every rank's J (and A) buffer"""
+        n_grid = int(dest.max()) + 1 if len(dest) else 0
+        for q in range(P.world):
+            _arr(P.J[q], n_grid, ctypes.c_double)[dest] = J_loc
+            if P.A[0] and a_loc is not None:
+                _arr(P.A[q], n_grid, ctypes.c_int32)[dest] = a_loc
+
+    def _local_combine(self, tref, part_val, part_idx, argmin_out):
+        T = tref._obj
+        J_loc = np.zeros(T.n_states)
+        if T.n_states:
+            rc = self.sdp_sweep_finalize(tref, part_val, part_idx, ctypes.c_void_p(J_loc.ctypes.data),
+                                         argmin_out, None)
+            assert rc == 0
+        return J_loc, _arr(argmin_out, T.n_states, ctypes.c_int32).copy()
+
+    def sdp_sweep_finalize_p2p(self, tref, part_val, part_idx, argmin_out, pref, state_begin, stream):
+        P = self._peers(pref)
+        assert state_begin >= 0
+        J_loc, a_loc = self._local_combine(tref, part_val, part_idx, argmin_out)
+        self._store(P, state_begin + np.arange(len(J_loc)), J_loc, a_loc)
+        self._publish(P)
+        self.launches += 1
+        return 0
+
+    def sdp_sweep_finalize_p2p_cols(self, tref, part_val, part_idx, argmin_out, pref, glob_cols, col_begin,
+                                    stream):
+        T = tref._obj
+        P = self._peers(pref)
+        assert T.layout == _cabi.LAYOUT_COLUMN_FACTORED and 0 <= col_begin and col_begin + T.n_cols <= glob_cols
+        J_loc, a_loc = self._local_combine(tref, part_val, part_idx, argmin_out)
+        n_rows = T.n_states // T.n_cols if T.n_cols else 0
+        dest = (np.arange(n_rows)[:, None] * glob_cols + col_begin + np.arange(T.n_cols)[None, :]).reshape(-1)
+        self._store(P, dest, J_loc, a_loc)
+        self._publish(P)
+        self.launches += 1
+        return 0
+
+    def sdp_p2p_wait(self, pref, stream):
+        self._wait(self._peers(pref))
+        self.launches += 1
+        return 0
+
+    def sdp_sweep_partials_after(self, gref, tref, J_prev, part_val, part_idx, pref, stream):
+        self._wait(self._peers(pref))
+        return self.sdp_sweep_partials(gref, tref, J_prev, part_val, part_idx, stream)
+
+    def sdp_p2p_broadcast(self, src, offset, n, pref, stream):
+        P = self._peers(pref)
+        assert offset >= 0 and n >= 0
+        if n:
+            piece = _arr(src, offset + n, ctypes.c_double)[offset:].copy()
+            for q in range(P.world):
+                if q != P.rank:
+                    _arr(P.J[q], offset + n, ctypes.c_double)[offset:] = piece
+        self._publish(P)
+        self.launches += 1
+        return 0
+
+    def sdp_p2p_barrier(self, pref, stream):
+        P = self._peers(pref)
+        self._publish(P)
+        self._wait(P)
+        self.launches += 1
+        return 0
+
+    def _policy_backup(self, gref, W, g_per_w, p, cell, lam, lam_plane, g, n, J):
+        """one fixed-policy backup of n states from J, in the kernel's order ([w][n] planes)"""
+        d, smin, smax, orders = _grid(gref)
+        strides = np.concatenate([np.cumprod(orders[::-1])[::-1][1:], [1]]).astype(np.int64)
+        P = _arr(p, W, ctypes.c_double)
+        C = _arr(cell, W * n, ctypes.c_int32).astype(np.int64).reshape(W, n)
+        L = [_arr(lam.value + 8 * k * lam_plane, W * n, ctypes.c_double).reshape(W, n) for k in range(d)]
+        Gv = _arr(g, (W if g_per_w else 1) * n, ctypes.c_double).reshape(-1, n)
+        acc = np.zeros(n)
+        for w in range(W):
+            lam_w = [L[k][w] for k in range(d)]
+
+            def rec(base, k):
+                if k == d:
+                    return J[base]
+                a = rec(base, k + 1)
+                b = rec(base + strides[k], k + 1)
+                return (1 - lam_w[k]) * a + lam_w[k] * b
+            acc = acc + (Gv[w if g_per_w else 0] + rec(C[w], 0)) * P[w]
+        return acc
+
+    def sdp_policy_eval_p2p(self, gref, W, g_per_w, p, cell, lam, lam_plane, g, n_states, state_begin, n_grid,
+                            J_in, pref, ref_cell, ref_lam, ref_g, J_ref_out, stream):
+        P = self._peers(pref)
+        assert 0 <= state_begin and state_begin + n_states <= n_grid
+        J = _arr(J_in, n_grid, ctypes.c_double)
+        acc = self._policy_backup(gref, W, g_per_w, p, cell, lam, lam_plane, g, n_states, J) \
+            if n_states else np.zeros(0)
+        if ref_cell:
+            assert ref_lam and ref_g and J_ref_out
+            # the reference state's entries: [W], [d][W], [W] or [1] (stride 1, lam plane W)
+            ref = self._policy_backup(gref, W, g_per_w, p, ref_cell, ref_lam, W, ref_g, 1, J)[0]
+            _arr(J_ref_out, 1, ctypes.c_double)[0] = ref
+            acc = acc - ref
+        self._store(P, state_begin + np.arange(n_states), acc, None)
+        self._publish(P)
+        self.launches += 1
+        return 0
+
     def sdp_policy_values(self, n, nc, lo, hi, npts, argmin, pol, stream):
         LO = _arr(lo, n * nc, ctypes.c_double).reshape(n, nc)
         HI = _arr(hi, n * nc, ctypes.c_double).reshape(n, nc)

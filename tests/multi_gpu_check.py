@@ -35,7 +35,8 @@ def check_column_layout(sdp, wl, rank):
         J, pol = ora.value_iteration(J)
         want.append((J, pol))
     ok = True
-    # (the cut by columns has not run on GPUs yet: asked for explicitly, scripts/gpu_round2_multi.sh)
+    # (the cut by columns runs when asked for: SDP_CHECK_COLUMN_AXIS=1, as in profiles/r2_multi_gpu_check_n{2,8}.log;
+    # tests/test_peer_exchange.py checks the same exchange with the ranks emulated on one GPU)
     axes = ("rows", "columns") if os.environ.get("SDP_CHECK_COLUMN_AXIS") else ("rows",)
     for axis in axes:
         sv = wl.storage_ar1(sdp, **kw).solver

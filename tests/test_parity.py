@@ -1010,7 +1010,7 @@ def test_column_hoist_is_bit_identical(product, backend, which):
                     J3, pol3 = col2.value_iteration(J0, report_time=False)
                     assert _same_bits(Jr, J3) and np.array_equal(polr, pol3, equal_nan=True), (threads, "pairs")
         finally:
-            lib.sdp_set_option(b"col_threads", 768)
+            lib.sdp_set_option(b"col_threads", 0)          # (the library default)
             lib.sdp_set_option(b"col_ub", 2)
             lib.sdp_set_option(b"col_pf", 2)
             lib.sdp_set_option(b"col_prepass", 3)
