@@ -517,6 +517,50 @@ int sdp_forward_build(const SdpGrid* grid, int32_t W, int32_t g_per_w, const dou
 int sdp_forward_steps(const SdpForwardOp* op, double* mu_a, double* mu_b, int32_t n_steps,
                       double* cost_out, double* resid_out, double* hist, double* scratch, void* stream);
 
+/* Risk-averse backups: the nested mean-CVaR operator.  New feature, no reference counterpart.
+ * For one (state x, control u) let v_w = g + I[J](f(x,u,w)) be the node values of sdp_sweep (same
+ * lerp, same g + v).  Every value is fp64, rounded as written, no FMA:
+ *   E = ((0 + v_0*p_0) + v_1*p_1) + ...                       (w in order: today's expectation)
+ *   C = NaN if any v_w is NaN; otherwise, over the nodes sorted by v descending (ties: lower w
+ *       first; -0 == +0), from cum = acc = 0: skip a node with p_k == 0; stop once cum >= beta;
+ *       r = beta - cum; p_k <= r: acc = acc + v_k*p_k, cum = cum + p_k; else acc = acc + v_k*r and
+ *       stop.  C = acc * inv_beta                           (the CVaR of the upper 1 - alpha tail)
+ *   rho = E*w_mean + C*w_cvar                               (both products first, then the sum)
+ * The argmin over the controls is that of sdp_sweep (lexicographic (value, index), NaN first).
+ * The host computes the constants once: beta = 1 - alpha, inv_beta = 1/beta, w_mean = 1 - weight,
+ * w_cvar = weight (0 <= alpha < 1, 0 <= weight <= 1).  Refused (SDP_EINVAL, nothing launched):
+ * beta outside (0, 1], inv_beta outside [1, DBL_MAX], a weight outside [0, 1], W > SDP_RISK_MAX_W.
+ * A deterministic system (expect == 0) has rho = v_0: the sweep is sdp_sweep_partials'. */
+#define SDP_RISK_MAX_W 16 /* node values and indices of a lane are kept in registers */
+typedef struct SdpRisk {
+    double inv_beta;
+    double beta;
+    double w_mean;
+    double w_cvar;
+} SdpRisk;
+/* Streaming pass of a risk sweep: the partial minima of rho that sdp_sweep_finalize[_p2p|_cols|_p2p_cols]
+ * combine, exactly as after sdp_sweep_partials.  Layout A: kernel k_sweep_risk<d, 9 | 16> (W <= 9 |
+ * W <= 16).  Layout CF with one row per lane (col_pairs == 0): the column-table pre-pass
+ * (sdp_column_table, skipped when col_table_ready) then k_sweep_risk_column<9>, one warp per work
+ * item over the positions seg_begin[0] .. seg_begin[n_segs] of the work list (item_order as for
+ * sdp_sweep_partials), no pruning and no group skipping.  Other layouts and col_pairs == 1 are
+ * refused. */
+int sdp_sweep_risk_partials(const SdpGrid* grid, const SdpTables* tab, const SdpRisk* risk, const double* J_prev,
+                            double* part_val, int32_t* part_idx, void* stream);
+/* sdp_policy_eval / sdp_policy_eval_p2p with the fixed-policy backup rho instead of the
+ * expectation (kernels k_policy_eval_risk<d, 9 | 16, rel> and k_policy_eval_risk_p2p<...>). */
+int sdp_policy_eval_risk(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p,
+                         const int32_t* cell, const double* lam, int64_t lam_plane,
+                         const double* g, int64_t n_states, int64_t state_begin, int64_t n_grid,
+                         double* J_a, double* J_b, int32_t n_iter, int32_t rel_dp,
+                         int64_t ref_index, double* J_ref_hist, const SdpRisk* risk, void* stream);
+int sdp_policy_eval_risk_p2p(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p,
+                             const int32_t* cell, const double* lam, int64_t lam_plane,
+                             const double* g, int64_t n_states, int64_t state_begin, int64_t n_grid,
+                             const double* J_in, const SdpPeers* peers, const int32_t* ref_cell,
+                             const double* ref_lam, const double* ref_g, double* J_ref_out,
+                             const SdpRisk* risk, void* stream);
+
 /* K1''' - sample paths of the chain of a fixed policy (Monte-Carlo trajectories).
  * New feature, no reference counterpart as a kernel: the reference simulates the policy on the host
  * (examples/20 .../storage_control.py:217,246).  The chain is the one of sdp_forward_*, sampled:

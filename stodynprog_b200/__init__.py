@@ -13,9 +13,10 @@ loudly without them - there is no CPU fallback.
 """
 from .sysdesc import SysDescription
 from .solver import DPSolver
+from .risk import MeanCVaR
 from .interp import (MlinInterpolator, MultilinearInterpolator, multilinear_interpolation,
                      mlinspace)
 
 __version__ = "0.1.0"
-__all__ = ["SysDescription", "DPSolver", "MlinInterpolator", "MultilinearInterpolator",
+__all__ = ["SysDescription", "DPSolver", "MeanCVaR", "MlinInterpolator", "MultilinearInterpolator",
            "multilinear_interpolation", "mlinspace"]

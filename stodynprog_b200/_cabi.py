@@ -94,6 +94,17 @@ class SdpPeers(ctypes.Structure):
                 ("A", ctypes.c_void_p * SDP_MAX_PEERS)]
 
 
+RISK_MAX_W = 16   # SDP_RISK_MAX_W: perturbation nodes of the risk kernels
+
+
+class SdpRisk(ctypes.Structure):
+    """host-computed constants of the mean-CVaR backup (sdp_sweep_risk_partials)"""
+    _fields_ = [("inv_beta", ctypes.c_double),
+                ("beta", ctypes.c_double),
+                ("w_mean", ctypes.c_double),
+                ("w_cvar", ctypes.c_double)]
+
+
 class SdpForwardOp(ctypes.Structure):
     """forward (adjoint) operator of a fixed policy: CSR by destination (sdp_forward_*)"""
     _fields_ = [("n", ctypes.c_int64),
@@ -181,6 +192,13 @@ SIGNATURES = {
                                        _vp, _vp, _i32, _i32, _i64, _vp, _vp]),
     "sdp_policy_eval_p2p": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64,
                                            _vp, ctypes.POINTER(SdpPeers), _vp, _vp, _vp, _vp, _vp]),
+    "sdp_sweep_risk_partials": (ctypes.c_int, [_gp, ctypes.POINTER(SdpTables), ctypes.POINTER(SdpRisk), _vp, _vp,
+                                               _vp, _vp]),
+    "sdp_policy_eval_risk": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64,
+                                            _vp, _vp, _i32, _i32, _i64, _vp, ctypes.POINTER(SdpRisk), _vp]),
+    "sdp_policy_eval_risk_p2p": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _vp, _i64, _vp, _i64, _i64, _i64,
+                                                _vp, ctypes.POINTER(SdpPeers), _vp, _vp, _vp, _vp,
+                                                ctypes.POINTER(SdpRisk), _vp]),
     "sdp_forward_sizes": (ctypes.c_int, [_i32, _i32, _i64, _vp, _vp, _vp, _vp]),
     "sdp_forward_build": (ctypes.c_int, [_gp, _i32, _i32, _vp, _vp, _vp, _i64, _vp,
                                          ctypes.POINTER(SdpForwardOp), _vp, _i64, _vp]),

@@ -3957,6 +3957,433 @@ extern "C" int sdp_policy_eval_p2p(const SdpGrid* grid, int32_t W, int32_t g_per
 }
 
 // ---------------------------------------------------------------------------
+// Risk-averse backups: the nested mean-CVaR operator (include/sdp_b200.h, SdpRisk).
+// New feature, no reference counterpart.  rho = E*w_mean + C*w_cvar over the node values
+// v_w = g + I[J](f(x,u,w)) of one (x,u): E the ordered expectation, C the CVaR of the upper
+// tail of mass beta, walked over the nodes sorted by v descending (ties: lower w first).
+// A lane keeps the WM node values of its (x,u) and their indices in registers and sorts them
+// with an odd-even transposition network unrolled at compile time (static register indices:
+// no local memory).  Padding slots hold v = -inf and an index >= W whose probability is 0.
+// ---------------------------------------------------------------------------
+// p_sh: [WM] probabilities in shared memory, 0 beyond W
+template <int WM>
+__device__ __forceinline__ double risk_value(double (&v)[WM], int W, const double* p_sh, const SdpRisk& R) {
+    double E = 0.0;
+    bool nan = false;
+#pragma unroll
+    for (int w = 0; w < WM; ++w) {
+        if (w < W) {
+            E = add_(E, mul_(v[w], p_sh[w]));
+            nan |= (v[w] != v[w]);
+        }
+    }
+    double C;
+    if (nan) {
+        C = CUDART_NAN;
+    } else {
+        int ix[WM];
+#pragma unroll
+        for (int w = 0; w < WM; ++w) {
+            ix[w] = w;
+            if (w >= W) v[w] = -CUDART_INF;
+        }
+#pragma unroll
+        for (int r = 0; r < WM; ++r) {
+#pragma unroll
+            for (int i = (r & 1); i + 1 < WM; i += 2) {
+                const bool sw = (v[i + 1] > v[i]) || (v[i + 1] == v[i] && ix[i + 1] < ix[i]);
+                const double tv = sw ? v[i + 1] : v[i];
+                const double bv = sw ? v[i] : v[i + 1];
+                const int ti = sw ? ix[i + 1] : ix[i];
+                const int bi = sw ? ix[i] : ix[i + 1];
+                v[i] = tv; v[i + 1] = bv; ix[i] = ti; ix[i + 1] = bi;
+            }
+        }
+        double cum = 0.0, acc = 0.0;
+        bool stop = false;
+#pragma unroll
+        for (int k = 0; k < WM; ++k) {
+            const double pk = p_sh[ix[k]];
+            if (!stop && pk != 0.0) {
+                if (cum >= R.beta) {
+                    stop = true;
+                } else {
+                    const double r = sub_(R.beta, cum);
+                    if (pk <= r) {
+                        acc = add_(acc, mul_(v[k], pk));
+                        cum = add_(cum, pk);
+                    } else {
+                        acc = add_(acc, mul_(v[k], r));
+                        stop = true;
+                    }
+                }
+            }
+        }
+        C = mul_(acc, R.inv_beta);
+    }
+    return add_(mul_(E, R.w_mean), mul_(C, R.w_cvar));
+}
+
+template <int WM>
+__device__ __forceinline__ void load_risk_p(double* p_sh, const double* __restrict__ p, int W) {
+    for (int i = threadIdx.x; i < WM; i += blockDim.x) p_sh[i] = i < W ? p[i] : 0.0;
+    __syncthreads();
+}
+
+// Layout A, one control per lane: the k_sweep walk with the node values kept for the risk reduction.
+template <int D, int WM>
+__global__ void __launch_bounds__(256)
+k_sweep_risk(GridT<double> G, SdpTables T, SdpRisk R, const double* __restrict__ Jprev,
+             double* __restrict__ part_val, int32_t* __restrict__ part_idx) {
+    __shared__ double p_sh[WM];
+    load_risk_p<WM>(p_sh, T.p, T.W);
+    const int lane = threadIdx.x & 31;
+    const int64_t item_id = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (item_id >= T.n_items) return;
+    const SdpItem it = T.items[item_id];
+    const int W = T.W;
+    const int64_t pitch = it.Upad;
+    double best_v = CUDART_INF;
+    int best_i = INT_MAX;
+    for (int u = lane; u < it.u_count; u += 32) {
+        const double g0 = T.g_per_w ? 0.0 : __ldcs(T.g + it.g_base + u);
+        double v[WM];
+#pragma unroll
+        for (int w = 0; w < WM; ++w) {
+            v[w] = 0.0;
+            if (w < W) {
+                const int64_t off = it.entry_base + (int64_t)w * pitch + u;
+                double lam[D];
+#pragma unroll
+                for (int k = 0; k < D; ++k) lam[k] = __ldcs(T.lam + (int64_t)k * T.lam_plane + off);
+                const double gw = T.g_per_w ? __ldcs(T.g + it.g_base + (int64_t)w * pitch + u) : g0;
+                v[w] = add_(gw, Lerp<double, D, 0>::eval(Jprev, __ldcs(T.cell + off), G.stride, lam));
+            }
+        }
+        const double rho = risk_value<WM>(v, W, p_sh, R);
+        const int idx = it.u_begin + u;
+        if (better(rho, idx, best_v, best_i)) { best_v = rho; best_i = idx; }
+    }
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        double ov = __shfl_xor_sync(0xffffffffu, best_v, s);
+        int oi = __shfl_xor_sync(0xffffffffu, best_i, s);
+        if (better(ov, oi, best_v, best_i)) { best_v = ov; best_i = oi; }
+    }
+    if (lane == 0) {
+        part_val[item_id] = best_v;
+        part_idx[item_id] = best_i;
+    }
+}
+
+// Layout CF, one row per lane: the column tables of the pre-pass (k_column_table, R[q][w] = the
+// inner interpolation of row q at node w) in global memory, v_w = g + ((1-l)*R[q][w] + l*R[q+1][w])
+// - the nested lerp of layout A, the same bits.  One warp per work item: the positions
+// seg_begin[0] .. seg_begin[n_segs] of the work list (item_order, or the items themselves), so that
+// a view of a range of positions (a piece of columns) sweeps that range only.  No pruning and no
+// group skipping: their bounds are for the expectation.
+__global__ void __launch_bounds__(256)
+k_sweep_risk_column(SdpTables T, SdpRisk R, double inv_stride0, int64_t pitch,
+                    double* __restrict__ part_val, int32_t* __restrict__ part_idx) {
+    constexpr int WM = SDP_FACTORED_MAX_W_REG;
+    __shared__ double p_sh[WM];
+    load_risk_p<WM>(p_sh, T.p, T.W);
+    const int lane = threadIdx.x & 31;
+    const int64_t pos = T.seg_begin[0] + (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    if (pos >= T.seg_begin[T.n_segs]) return;
+    const int64_t item_id = T.item_order ? T.item_order[pos] : pos;
+    const SdpItem it = T.items[item_id];
+    const int W = T.W, P = W | 1;
+    const int Us = T.U[(int64_t)it.state * 32 + lane];          // by position; 0 on padding lanes
+    const double* __restrict__ Rc = T.col_table + (int64_t)it.Upad * pitch;
+    double best_v = CUDART_INF;
+    int best_i = INT_MAX;
+    for (int uu = 0; uu < it.u_count && it.u_begin + uu < Us; ++uu) {
+        const int64_t o = it.entry_base + (int64_t)uu * 32 + lane;
+        const int c = __ldcs(T.cell + o);
+        const double l = __ldcs(T.lam + o), gv = __ldcs(T.g + o);
+        const double oml = sub_(1.0, l);
+        // row q = cell_u / stride0 exactly (cell_u is a multiple of stride0 below 2^31)
+        const double* Ra = Rc + __double2int_rn(__dmul_rn((double)c, inv_stride0)) * P;
+        double v[WM];
+#pragma unroll
+        for (int w = 0; w < WM; ++w)
+            v[w] = w < W ? add_(gv, add_(mul_(oml, __ldg(Ra + w)), mul_(l, __ldg(Ra + P + w)))) : 0.0;
+        const double rho = risk_value<WM>(v, W, p_sh, R);
+        const int idx = it.u_begin + uu;
+        if (better(rho, idx, best_v, best_i)) { best_v = rho; best_i = idx; }
+    }
+    part_val[item_id * 32 + lane] = best_v;
+    part_idx[item_id * 32 + lane] = best_i;
+}
+
+// one fixed-policy risk backup; entry w of the state at index w*stride (as policy_backup)
+template <int D, int WM>
+__device__ __forceinline__ double policy_backup_risk(const GridT<double>& G, int W, int g_per_w,
+                                                     const double* p_sh, const int32_t* __restrict__ cell,
+                                                     const double* __restrict__ lam, int64_t lam_plane,
+                                                     const double* __restrict__ g, int64_t stride,
+                                                     const double* __restrict__ J_in, const SdpRisk& R) {
+    const double g0 = g_per_w ? 0.0 : g[0];
+    double v[WM];
+#pragma unroll
+    for (int w = 0; w < WM; ++w) {
+        v[w] = 0.0;
+        if (w < W) {
+            const int64_t off = (int64_t)w * stride;
+            double l[D];
+#pragma unroll
+            for (int k = 0; k < D; ++k) l[k] = lam[(int64_t)k * lam_plane + off];
+            const double gw = g_per_w ? g[off] : g0;
+            v[w] = add_(gw, Lerp<double, D, 0>::eval(J_in, cell[off], G.stride, l));
+        }
+    }
+    return risk_value<WM>(v, W, p_sh, R);
+}
+
+template <int D, int WM, bool REL>
+__global__ void __launch_bounds__(256)
+k_policy_eval_risk(GridT<double> G, int W, int g_per_w, const double* __restrict__ p,
+                   const int32_t* __restrict__ cell, const double* __restrict__ lam, int64_t lam_plane,
+                   const double* __restrict__ g, int64_t n_states, const double* __restrict__ J_in,
+                   double* __restrict__ J_out, RefState RS, SdpRisk R) {
+    __shared__ double p_sh[WM];
+    __shared__ double ref_sh;
+    load_risk_p<WM>(p_sh, p, W);
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    double acc = 0.0;
+    if (i < n_states)
+        acc = policy_backup_risk<D, WM>(G, W, g_per_w, p_sh, cell + i, lam + i, lam_plane, g + i, n_states, J_in, R);
+    if (REL) {
+        if (threadIdx.x == 0) {
+            ref_sh = policy_backup_risk<D, WM>(G, W, g_per_w, p_sh, RS.cell, RS.lam, RS.lam_plane, RS.g, RS.stride,
+                                               J_in, R);
+            if (blockIdx.x == 0) RS.hist[0] = ref_sh;
+        }
+        __syncthreads();
+        acc = sub_(acc, ref_sh);
+    }
+    if (i < n_states) J_out[i] = acc;
+}
+
+template <int D, int WM, bool REL>
+__global__ void __launch_bounds__(256)
+k_policy_eval_risk_p2p(GridT<double> G, int W, int g_per_w, const double* __restrict__ p,
+                       const int32_t* __restrict__ cell, const double* __restrict__ lam, int64_t lam_plane,
+                       const double* __restrict__ g, int64_t n_states, const double* __restrict__ J_in,
+                       PeersDev P, int64_t state_begin, RefState RS, SdpRisk R) {
+    __shared__ double p_sh[WM];
+    __shared__ double ref_sh;
+    load_risk_p<WM>(p_sh, p, W);
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    double acc = 0.0;
+    if (i < n_states)
+        acc = policy_backup_risk<D, WM>(G, W, g_per_w, p_sh, cell + i, lam + i, lam_plane, g + i, n_states, J_in, R);
+    if (REL) {
+        if (threadIdx.x == 0) {
+            ref_sh = policy_backup_risk<D, WM>(G, W, g_per_w, p_sh, RS.cell, RS.lam, RS.lam_plane, RS.g, RS.stride,
+                                               J_in, R);
+            if (blockIdx.x == 0) RS.hist[0] = ref_sh;
+        }
+        __syncthreads();
+        acc = sub_(acc, ref_sh);
+    }
+    if (i < n_states) {
+#pragma unroll
+        for (int r = 0; r < SDP_MAX_PEERS; ++r)
+            if (r < P.world) P.J[r][state_begin + i] = acc;
+    }
+    publish_epoch(P);
+}
+
+static int check_risk(const SdpRisk* risk, int W, const char* who) {
+    if (!risk) return fail(SDP_EINVAL, "%s: risk is NULL", who);
+    const SdpRisk& R = *risk;
+    if (!(R.beta > 0.0 && R.beta <= 1.0 && R.inv_beta >= 1.0 && R.inv_beta <= 1.7976931348623157e308 &&
+          R.w_mean >= 0.0 && R.w_mean <= 1.0 && R.w_cvar >= 0.0 && R.w_cvar <= 1.0))
+        return fail(SDP_EINVAL, "%s: risk constants out of range (0 < beta <= 1, 1 <= inv_beta < inf, "
+                                "weights in [0, 1])", who);
+    if (W > SDP_RISK_MAX_W) {
+        snprintf(g_err, sizeof g_err, "%s: W = %d perturbation nodes, the risk kernels support at most %d",
+                 who, W, SDP_RISK_MAX_W);
+        return SDP_EINVAL;
+    }
+    return SDP_OK;
+}
+
+extern "C" int sdp_sweep_risk_partials(const SdpGrid* grid, const SdpTables* tab, const SdpRisk* risk,
+                                       const double* J_prev, double* part_val, int32_t* part_idx, void* stream) {
+    GridT<double> G;
+    int rc = make_grid<double>(grid, &G, nullptr);
+    if (rc) return rc;
+    if (!tab) return fail(SDP_EINVAL, "%s", "sdp_sweep_risk_partials: tables is NULL");
+    const SdpTables& T = *tab;
+    rc = check_tables(T, "sdp_sweep_risk_partials");
+    if (rc) return rc;
+    if (T.layout != SDP_LAYOUT_CONTROL_MINOR && !is_column(T))
+        return fail(SDP_EINVAL, "%s", "sdp_sweep_risk_partials: the risk sweep takes layout A or CF tables only");
+    if (is_column(T) && T.col_pairs)
+        return fail(SDP_EINVAL, "%s", "sdp_sweep_risk_partials: layout CF with two rows per lane is not supported");
+    rc = check_risk(risk, T.W, "sdp_sweep_risk_partials");
+    if (rc) return rc;
+    if (is_column(T)) {
+        rc = check_factored_args(grid->d, T.W, T.u_mask, "sdp_sweep_risk_partials");
+        if (!rc) rc = check_column_stream(T, "sdp_sweep_risk_partials");
+        if (rc) return rc;
+        if (SDP_COLUMN_PITCH(G.order[0], T.W) * 8 > SDP_COLUMN_MAX_SMEM_BYTES)
+            return fail(SDP_EINVAL, "%s", "sdp_sweep_risk_partials: the column table does not fit");
+    }
+    if (T.n_states == 0 || T.n_items == 0) return SDP_OK;
+    if (!J_prev || !part_val || !part_idx) return fail(SDP_EINVAL, "%s", "sdp_sweep_risk_partials: NULL pointer");
+    cudaStream_t st = (cudaStream_t)stream;
+    if (is_column(T)) {
+        if (!T.expect)      // deterministic: rho = v_0, today's column sweep
+            return grid->d == 2 ? launch_fact_column<2>(G, T, J_prev, part_val, part_idx, st)
+                                : launch_fact_column<3>(G, T, J_prev, part_val, part_idx, st);
+        if (!T.col_table_ready) {
+            rc = grid->d == 2 ? launch_column_table<2>(G, T, J_prev, st) : launch_column_table<3>(G, T, J_prev, st);
+            if (rc) return rc;
+        }
+        const SdpRisk R = *risk;
+        const unsigned blocks = (unsigned)((T.n_items + 7) / 8);
+        k_sweep_risk_column<<<blocks, 256, 0, st>>>(T, R, 1.0 / (double)G.stride[0],
+                                                    SDP_COLUMN_PITCH(G.order[0], T.W), part_val, part_idx);
+        note_kernel("%s", "k_sweep_risk_column<9>");
+        SDP_LAUNCH_CHECK();
+        return SDP_OK;
+    }
+    if (!T.expect) {
+        // deterministic: rho = v_0, today's backup
+        switch (grid->d) {
+            case 1: return launch_sweep<1>(G, T, J_prev, part_val, part_idx, st);
+            case 2: return launch_sweep<2>(G, T, J_prev, part_val, part_idx, st);
+            case 3: return launch_sweep<3>(G, T, J_prev, part_val, part_idx, st);
+            default: return launch_sweep<4>(G, T, J_prev, part_val, part_idx, st);
+        }
+    }
+    const SdpRisk R = *risk;
+    const int warps = 8;
+    const unsigned blocks = (unsigned)((T.n_items + warps - 1) / warps);
+    const bool small = T.W <= 9;
+#define SDP_RISK_SWEEP(D_)                                                                                      \
+    if (small) k_sweep_risk<D_, 9><<<blocks, warps * 32, 0, st>>>(G, T, R, J_prev, part_val, part_idx);          \
+    else k_sweep_risk<D_, 16><<<blocks, warps * 32, 0, st>>>(G, T, R, J_prev, part_val, part_idx);
+    switch (grid->d) {
+        case 1: SDP_RISK_SWEEP(1) break;
+        case 2: SDP_RISK_SWEEP(2) break;
+        case 3: SDP_RISK_SWEEP(3) break;
+        default: SDP_RISK_SWEEP(4) break;
+    }
+#undef SDP_RISK_SWEEP
+    note_kernel("k_sweep_risk<%d,%d>", grid->d, small ? 9 : 16);
+    SDP_LAUNCH_CHECK();
+    return SDP_OK;
+}
+
+extern "C" int sdp_policy_eval_risk(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p,
+                                    const int32_t* cell, const double* lam, int64_t lam_plane,
+                                    const double* g, int64_t n_states, int64_t state_begin, int64_t n_grid,
+                                    double* J_a, double* J_b, int32_t n_iter, int32_t rel_dp,
+                                    int64_t ref_index, double* J_ref_hist, const SdpRisk* risk, void* stream) {
+    GridT<double> G;
+    int64_t ng = 0;
+    int rc = make_grid<double>(grid, &G, &ng);
+    if (rc) return rc;
+    if (W < 1 || n_states < 0 || n_iter < 0 || n_grid != ng || state_begin < 0 ||
+        state_begin + n_states > n_grid)
+        return fail(SDP_EINVAL, "%s", "sdp_policy_eval_risk: bad sizes");
+    rc = check_risk(risk, W, "sdp_policy_eval_risk");
+    if (rc) return rc;
+    if (n_iter == 0 || n_states == 0) return SDP_OK;
+    if (!p || !cell || !lam || !g || !J_a || !J_b) return fail(SDP_EINVAL, "%s", "sdp_policy_eval_risk: NULL pointer");
+    if (rel_dp && (!J_ref_hist || n_states != n_grid || ref_index < 0 || ref_index >= n_grid))
+        return fail(SDP_EINVAL, "%s", "sdp_policy_eval_risk: rel_dp needs the whole grid in one shard and a J_ref_hist buffer");
+    cudaStream_t st = (cudaStream_t)stream;
+    const unsigned blocks = (unsigned)((n_states + 255) / 256);
+    const SdpRisk R = *risk;
+    const bool small = W <= 9;
+    RefState RS = {nullptr, nullptr, 0, nullptr, 0, nullptr};
+    if (rel_dp) {
+        const int64_t ir = ref_index - state_begin;
+        RS.cell = cell + ir; RS.lam = lam + ir; RS.lam_plane = lam_plane; RS.g = g + ir; RS.stride = n_states;
+    }
+    double* in = J_a;
+    double* out = J_b;
+#define SDP_PE_RISK(D_, WM_, REL_)                                                                              \
+    k_policy_eval_risk<D_, WM_, REL_><<<blocks, 256, 0, st>>>(G, W, g_per_w, p, cell, lam, lam_plane, g, n_states, \
+                                                              in, out + state_begin, RS, R)
+#define SDP_PE_RISK_D(D_)                                                                                       \
+    if (rel_dp) { if (small) SDP_PE_RISK(D_, 9, true); else SDP_PE_RISK(D_, 16, true); }                       \
+    else { if (small) SDP_PE_RISK(D_, 9, false); else SDP_PE_RISK(D_, 16, false); }
+    for (int it = 0; it < n_iter; ++it) {
+        if (rel_dp) RS.hist = J_ref_hist + it;
+        switch (grid->d) {
+            case 1: SDP_PE_RISK_D(1) break;
+            case 2: SDP_PE_RISK_D(2) break;
+            case 3: SDP_PE_RISK_D(3) break;
+            default: SDP_PE_RISK_D(4) break;
+        }
+        SDP_LAUNCH_CHECK();
+        double* t = in; in = out; out = t;
+    }
+#undef SDP_PE_RISK_D
+#undef SDP_PE_RISK
+    note_kernel("k_policy_eval_risk<%d,%d,%d>", grid->d, small ? 9 : 16, rel_dp ? 1 : 0);
+    return SDP_OK;
+}
+
+extern "C" int sdp_policy_eval_risk_p2p(const SdpGrid* grid, int32_t W, int32_t g_per_w, const double* p,
+                                        const int32_t* cell, const double* lam, int64_t lam_plane,
+                                        const double* g, int64_t n_states, int64_t state_begin,
+                                        int64_t n_grid, const double* J_in, const SdpPeers* peers,
+                                        const int32_t* ref_cell, const double* ref_lam,
+                                        const double* ref_g, double* J_ref_out, const SdpRisk* risk,
+                                        void* stream) {
+    GridT<double> G;
+    int64_t ng = 0;
+    int rc = make_grid<double>(grid, &G, &ng);
+    if (rc) return rc;
+    if (W < 1 || n_states < 0 || n_grid != ng || state_begin < 0 || state_begin + n_states > n_grid)
+        return fail(SDP_EINVAL, "%s", "sdp_policy_eval_risk_p2p: bad sizes");
+    rc = check_risk(risk, W, "sdp_policy_eval_risk_p2p");
+    if (rc) return rc;
+    PeersDev P;
+    rc = make_peers(peers, &P, "sdp_policy_eval_risk_p2p");
+    if (rc) return rc;
+    for (int r = 0; r < P.world; ++r)
+        if (!P.J[r]) return fail(SDP_EINVAL, "%s", "sdp_policy_eval_risk_p2p: NULL J buffer");
+    if (!J_in || !p || (n_states > 0 && (!cell || !lam || !g)))
+        return fail(SDP_EINVAL, "%s", "sdp_policy_eval_risk_p2p: NULL pointer");
+    if (ref_cell && (!ref_lam || !ref_g || !J_ref_out))
+        return fail(SDP_EINVAL, "%s", "sdp_policy_eval_risk_p2p: incomplete reference-state arguments");
+    cudaStream_t st = (cudaStream_t)stream;
+    unsigned blocks = (unsigned)((n_states + 255) / 256);
+    if (blocks == 0) blocks = 1;      // the epoch must advance on every rank, even for an empty slab
+    const SdpRisk R = *risk;
+    const bool small = W <= 9;
+    const bool rel = ref_cell != nullptr;
+    RefState RS = {nullptr, nullptr, 0, nullptr, 0, nullptr};
+    if (rel) RS = {ref_cell, ref_lam, (int64_t)W, ref_g, 1, J_ref_out};
+#define SDP_PE_RISK(D_, WM_, REL_)                                                                              \
+    k_policy_eval_risk_p2p<D_, WM_, REL_><<<blocks, 256, 0, st>>>(G, W, g_per_w, p, cell, lam, lam_plane, g,     \
+                                                                  n_states, J_in, P, state_begin, RS, R)
+#define SDP_PE_RISK_D(D_)                                                                                       \
+    if (rel) { if (small) SDP_PE_RISK(D_, 9, true); else SDP_PE_RISK(D_, 16, true); }                          \
+    else { if (small) SDP_PE_RISK(D_, 9, false); else SDP_PE_RISK(D_, 16, false); }
+    switch (grid->d) {
+        case 1: SDP_PE_RISK_D(1) break;
+        case 2: SDP_PE_RISK_D(2) break;
+        case 3: SDP_PE_RISK_D(3) break;
+        default: SDP_PE_RISK_D(4) break;
+    }
+#undef SDP_PE_RISK_D
+#undef SDP_PE_RISK
+    note_kernel("k_policy_eval_risk_p2p<%d,%d,%d>", grid->d, small ? 9 : 16, rel ? 1 : 0);
+    SDP_LAUNCH_CHECK();
+    return SDP_OK;
+}
+
+// ---------------------------------------------------------------------------
 // K1'': forward (adjoint) operator of a fixed policy, mu <- P^T mu (include/sdp_b200.h).
 // New feature: the reference only simulates trajectories (storage_control.py:217,246).
 // Build: CSR by destination from the [w][n] policy-table planes of K1'.  Steps: a gather, one

@@ -440,7 +440,7 @@ class Engine(object):
             self._peer[key] = hs
         return self._peer[key]
 
-    def sweep_shared(self, hs, T, J_next, rel_ref_index=None, want_results=True, while_waiting=None):
+    def sweep_shared(self, hs, T, J_next, rel_ref_index=None, want_results=True, while_waiting=None, risk=None):
         """One sweep with host arrays in and out through the shared page-locked segment `hs`:
         every rank uploads 1/N of J_next and hands it to its peers over NVLink, sweeps its shard
         (the combine kernel stores J AND the argmin into every rank's buffers), maps 1/N of the
@@ -488,7 +488,7 @@ class Engine(object):
         tm.append(time.perf_counter())
         # 3. the sweep; J_new and the argmin are complete on every rank after the flag wait
         ref_out = torch.zeros(1, dtype=torch.float64, device=self.device) if rel_ref_index is not None else None
-        self.sweep(T, J_prev, J_new, rel_ref_index=rel_ref_index, ref_out=ref_out)
+        self.sweep(T, J_prev, J_new, rel_ref_index=rel_ref_index, ref_out=ref_out, risk=risk)
         tm.append(time.perf_counter())
         # 4. 1/N of the results -> the shared slot
         pol = torch.empty((b - a, max(nc, 1)), dtype=torch.float64, device=self.device)
@@ -694,18 +694,19 @@ class Engine(object):
             self._scan_cache = (scan_key, host_full)
         return host_full, mine
 
-    def build_sweep_tables(self, solver, t_k=None, reuse=None):
+    def build_sweep_tables(self, solver, t_k=None, reuse=None, for_risk=False):
         """Tabulate the user's callables over this rank's shard and build the tables on the
         device: `tablebuild.BuildPlan` (scan of the control boxes, cut over the ranks) and
         `tablebuild.ShardBuild` (layout, tabulation with its fall-backs, work list).  `reuse`: a
         SweepTables whose device buffers are recycled when the sizes match (time-dependent
         recursion).  With several ranks and slab_axis "auto" the grid is cut by columns when
         layout CF is expected to apply; if the built tables refuse it (same decision on every
-        rank), the build starts again with slabs of rows."""
+        rank), the build starts again with slabs of rows.  `for_risk`: tables for the risk sweep
+        (layout CF with one row per lane where it applies, else dense layout A)."""
         try:
-            return BuildPlan(self, solver, t_k).run(reuse)
+            return BuildPlan(self, solver, t_k, for_risk=for_risk).run(reuse)
         except _ColumnsNotApplicable:
-            return BuildPlan(self, solver, t_k, forced_axis="rows").run(None)
+            return BuildPlan(self, solver, t_k, forced_axis="rows", for_risk=for_risk).run(None)
 
     COLUMN_SEGS_PER_SM = int(os.environ.get("SDP_COLUMN_SEGS_PER_SM", "1"))
     # share of the tiles at the end of every (band, column) run whose work items are half as long
@@ -820,12 +821,28 @@ class Engine(object):
                                              ctypes.c_void_p(argmin.data_ptr() + 4 * s0), stream)
             _cabi.check(rc, "sdp_sweep_finalize")
 
-    def sweep_local(self, T, J_prev, events=None, J_out=None):
+    def risk_partials(self, T, tab, risk, J_prev, part_val, part_idx, stream=None):
+        """the streaming pass of a risk sweep (sdp_sweep_risk_partials; `risk` an SdpRisk) on the
+        tables view `tab`: the same partial minima the combine passes of sdp_sweep_partials take"""
+        rc = self.lib.sdp_sweep_risk_partials(ctypes.byref(T.grid), ctypes.byref(tab), ctypes.byref(risk),
+                                              self._ptr(J_prev), part_val, part_idx,
+                                              self.stream if stream is None else stream)
+        _cabi.check(rc, "sdp_sweep_risk_partials")
+
+    def sweep_local(self, T, J_prev, events=None, J_out=None, risk=None):
         """Enqueue K1 on this rank's slab.  J_prev: device fp64 [n_grid].
         Results land in `J_out` (default T.J_out) / T.argmin (slab-local).  `events`: optional
         (start, end) torch.cuda.Event pair recorded around the streaming kernel
-        alone (bench roofline)."""
+        alone (bench roofline).  `risk`: an SdpRisk, the risk sweep (layout A tables)."""
         J_out = T.J_out if J_out is None else J_out
+        if risk is not None:
+            if events is not None:
+                events[0].record(self.torch_stream)
+            self.risk_partials(T, T.c_tables, risk, J_prev, self._ptr(T.part_val), self._ptr(T.part_idx))
+            if events is not None:
+                events[1].record(self.torch_stream)
+            self._finalize(T, J_out, T.argmin)
+            return
         if events is None and not T.column:
             rc = self.lib.sdp_sweep(ctypes.byref(T.grid), ctypes.byref(T.c_tables), self._ptr(J_prev),
                                     self._ptr(T.part_val), self._ptr(T.part_idx),
@@ -857,13 +874,14 @@ class Engine(object):
             _cabi.check(rc, "sdp_p2p_wait")
 
     def sweep(self, T, J_prev, J_new, rel_ref_index=None, ref_out=None, resid_out=None,
-              events=None, defer_wait=False, want_argmin=True):
+              events=None, defer_wait=False, want_argmin=True, risk=None):
         """One full Bellman sweep: K1 on the slab, all-gather of the J slab into
         J_new (device fp64 [n_grid]), optional relative-DP shift and optional
         sup-norm residual max|J_new - J_prev| (all-reduced).
         `defer_wait`: the caller's next use of J_new is another sweep (or it calls
         flush_exchange() itself): the arrival of the peers' slabs is then awaited by that
-        sweep's first kernel.
+        sweep's first kernel (a risk sweep waits in a launch of its own).
+        `risk`: an SdpRisk, the risk sweep (layout A tables).
         `want_argmin` False: an intermediate sweep of a device-resident loop, whose policy
         nobody reads - the combine kernel then sends J alone to the peers (the shard's own
         argmin is still written; gather_argmin falls back to collecting those)."""
@@ -881,7 +899,12 @@ class Engine(object):
             # into every rank's J_new over NVLink and publishes the epoch
             if events is not None:
                 events[0].record(self.torch_stream)
-            if pend is not None:
+            if risk is not None:
+                if pend is not None:
+                    rc = self.lib.sdp_p2p_wait(ctypes.byref(pend), self.stream)
+                    _cabi.check(rc, "sdp_p2p_wait")
+                self.risk_partials(T, T.c_tables, risk, J_prev, self._ptr(T.part_val), self._ptr(T.part_idx))
+            elif pend is not None:
                 rc = self.lib.sdp_sweep_partials_after(ctypes.byref(T.grid), ctypes.byref(T.c_tables),
                                                        self._ptr(J_prev), self._ptr(T.part_val),
                                                        self._ptr(T.part_idx), ctypes.byref(pend), self.stream)
@@ -913,9 +936,9 @@ class Engine(object):
         else:
             self._argmin_in_px = False
             if self.coll.world == 1:
-                self.sweep_local(T, J_prev, events, J_out=J_new)     # (one rank: straight into J_new)
+                self.sweep_local(T, J_prev, events, J_out=J_new, risk=risk)     # (one rank: straight into J_new)
             else:
-                self.sweep_local(T, J_prev, events)
+                self.sweep_local(T, J_prev, events, risk=risk)
             if self.coll.world == 1:
                 pass
             elif T.col_bounds is not None:
@@ -1062,7 +1085,7 @@ class Engine(object):
                                         8 * nc * (c1 - c0), n_rows, cs)
             _cabi.check(rc, "sdp_memcpy_2d")
 
-    def sweep_to_host(self, T, J_prev, J_new, while_waiting=None):
+    def sweep_to_host(self, T, J_prev, J_new, while_waiting=None, risk=None):
         """One sweep of a single-rank slab, returning (J, pol) as host arrays in
         page-locked memory.  The slab is swept in a few runs (`_chunk_plan`: ranges of
         states, row bands of layout CF, or - layout CF with one band, the default - pieces
@@ -1071,6 +1094,7 @@ class Engine(object):
         (K3; one launch does both for a piece of columns), a copy stream sends that run's
         J and policy to their place in the host arrays while the following runs still
         compute.  Same kernels on sub-ranges of the same tables: bit-identical to `sweep`.
+        `risk`: an SdpRisk, the risk sweep (layout A tables).
         (stodynprog.py:496-499,517-521: J_k and pol_k are C-order arrays over the grid.)"""
         torch = _torch()
         dev = self.device
@@ -1107,9 +1131,12 @@ class Engine(object):
             if after is not None:
                 st.wait_event(after)       # (the last piece of columns starts after the combine before it)
                 after = None
-            rc = self.lib.sdp_sweep_partials(ctypes.byref(T.grid), ctypes.byref(ch["tab_p"]),
-                                             self._ptr(J_prev), ch["pv"], ch["pi"], sp)
-            _cabi.check(rc, "sdp_sweep_partials")
+            if risk is not None:
+                self.risk_partials(T, ch["tab_p"], risk, J_prev, ch["pv"], ch["pi"], sp)
+            else:
+                rc = self.lib.sdp_sweep_partials(ctypes.byref(T.grid), ctypes.byref(ch["tab_p"]),
+                                                 self._ptr(J_prev), ch["pv"], ch["pi"], sp)
+                _cabi.check(rc, "sdp_sweep_partials")
             mark("run %d swept" % k, st)
             if ch.get("kind") == "cols":
                 # the combine of a piece runs beside the sweep of the next one (small CTAs that fit
@@ -1252,7 +1279,7 @@ class Engine(object):
     # -- time-dependent recursion, fast path ----------------------------------
     RECURSION_MAX_G_BYTES = 8 << 30      # per-instant stage-cost tables kept resident
 
-    def recursion_fast(self, solver, t_ini, t_fin, J_fin, J_out, pol_out):
+    def recursion_fast(self, solver, t_ini, t_fin, J_fin, J_out, pol_out, risk=None):
         """bellman_recursion (stodynprog.py:536-591) for systems whose dynamics and admissible
         controls do not depend on the instant, only the stage cost does - the reference's
         time-dependent examples (examples/01 .../pv_storage_control.py:43-65: the PV production
@@ -1276,7 +1303,7 @@ class Engine(object):
         t_base = t_fin - 1
         solver._keep_staging = True
         try:
-            T = self.build_sweep_tables(solver, t_base)
+            T = self.build_sweep_tables(solver, t_base, for_risk=risk is not None)
         finally:
             solver._keep_staging = False
         rec = getattr(T, "build_record", None)
@@ -1379,10 +1406,16 @@ class Engine(object):
         for k in range(n_T - 1, -1, -1):
             v = _cabi.SdpTables.from_buffer_copy(T.c_tables)
             v.g = g_all.data_ptr() + 8 * k * g_len
-            rc = self.lib.sdp_sweep(ctypes.byref(T.grid), ctypes.byref(v), self._ptr(J_all[k + 1]),
-                                    self._ptr(T.part_val), self._ptr(T.part_idx), self._ptr(J_all[k]),
-                                    self._ptr(arg_all[k]), self.stream)
-            _cabi.check(rc, "sdp_sweep")
+            if risk is not None:
+                self.risk_partials(T, v, risk, J_all[k + 1], self._ptr(T.part_val), self._ptr(T.part_idx))
+                rc = self.lib.sdp_sweep_finalize(ctypes.byref(v), self._ptr(T.part_val), self._ptr(T.part_idx),
+                                                 self._ptr(J_all[k]), self._ptr(arg_all[k]), self.stream)
+                _cabi.check(rc, "sdp_sweep_finalize")
+            else:
+                rc = self.lib.sdp_sweep(ctypes.byref(T.grid), ctypes.byref(v), self._ptr(J_all[k + 1]),
+                                        self._ptr(T.part_val), self._ptr(T.part_idx), self._ptr(J_all[k]),
+                                        self._ptr(arg_all[k]), self.stream)
+                _cabi.check(rc, "sdp_sweep")
             if nc:
                 rc = self.lib.sdp_policy_values(n_grid, nc, self._ptr(T.lo_dev), self._ptr(T.hi_dev),
                                                 self._ptr(T.npts_dev), self._ptr(arg_all[k]),
@@ -1497,20 +1530,23 @@ class Engine(object):
             a = a.astype(float)
         return a.reshape((1,) * (len(full) - a.ndim) + a.shape)
 
-    def policy_eval(self, P, J_a, J_b, n_iter, rel_dp, ref_index, J_ref_hist):
+    def policy_eval(self, P, J_a, J_b, n_iter, rel_dp, ref_index, J_ref_hist, risk=None):
         """n_iter fixed-policy backups, ping-pong between J_a and J_b (device fp64
-        [n_grid]).  Returns the tensor holding the final value function."""
+        [n_grid]).  Returns the tensor holding the final value function.
+        `risk`: an SdpRisk, the risk backups (sdp_policy_eval_risk[_p2p])."""
         n_grid = J_a.numel()
         self.flush_exchange()
+        # (a risk measure: the same entry points with "_risk" and the SdpRisk before the stream)
+        sfx, extra = ("", ()) if risk is None else ("_risk", (ctypes.byref(risk),))
         if self.coll.world == 1:
-            rc = self.lib.sdp_policy_eval(ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.p),
-                                          self._ptr(P.cell), self._ptr(P.lam), P.lam_plane,
-                                          self._ptr(P.g), P.n_states, 0, n_grid,
-                                          self._ptr(J_a), self._ptr(J_b), int(n_iter),
-                                          1 if rel_dp else 0, int(ref_index),
-                                          self._ptr(J_ref_hist) if rel_dp else ctypes.c_void_p(0),
-                                          self.stream)
-            _cabi.check(rc, "sdp_policy_eval")
+            rc = getattr(self.lib, "sdp_policy_eval" + sfx)(ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.p),
+                    self._ptr(P.cell), self._ptr(P.lam), P.lam_plane,
+                    self._ptr(P.g), P.n_states, 0, n_grid,
+                    self._ptr(J_a), self._ptr(J_b), int(n_iter),
+                    1 if rel_dp else 0, int(ref_index),
+                    self._ptr(J_ref_hist) if rel_dp else ctypes.c_void_p(0),
+                    *extra, self.stream)
+            _cabi.check(rc, "sdp_policy_eval" + sfx)
             return J_a if n_iter % 2 == 0 else J_b
         cur, nxt = J_a, J_b
         sb, n = P.state_begin, P.n_states
@@ -1521,25 +1557,25 @@ class Engine(object):
             for k in range(n_iter):
                 k_new = px.index_of(nxt)
                 null = ctypes.c_void_p(0)
-                rc = self.lib.sdp_policy_eval_p2p(
+                rc = getattr(self.lib, "sdp_policy_eval%s_p2p" % sfx)(
                     ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.p), self._ptr(P.cell),
                     self._ptr(P.lam), P.lam_plane, self._ptr(P.g), n, sb, n_grid, self._ptr(cur),
                     ctypes.byref(px.peers[k_new]),
                     self._ptr(P.ref_cell) if rel_dp else null, self._ptr(P.ref_lam) if rel_dp else null,
                     self._ptr(P.ref_g) if rel_dp else null,
-                    ctypes.c_void_p(J_ref_hist.data_ptr() + 8 * k) if rel_dp else null, self.stream)
-                _cabi.check(rc, "sdp_policy_eval_p2p")
+                    ctypes.c_void_p(J_ref_hist.data_ptr() + 8 * k) if rel_dp else null, *extra, self.stream)
+                _cabi.check(rc, "sdp_policy_eval%s_p2p" % sfx)
                 rc = self.lib.sdp_p2p_wait(ctypes.byref(px.peers[k_new]), self.stream)
                 _cabi.check(rc, "sdp_p2p_wait")
                 cur, nxt = nxt, cur
             return cur
         for k in range(n_iter):
-            rc = self.lib.sdp_policy_eval(ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.p),
-                                          self._ptr(P.cell), self._ptr(P.lam), P.lam_plane,
-                                          self._ptr(P.g), n, sb, n_grid,
-                                          self._ptr(cur), self._ptr(nxt), 1, 0, 0,
-                                          ctypes.c_void_p(0), self.stream)
-            _cabi.check(rc, "sdp_policy_eval")
+            rc = getattr(self.lib, "sdp_policy_eval" + sfx)(ctypes.byref(P.grid), P.W, P.g_per_w, self._ptr(P.p),
+                    self._ptr(P.cell), self._ptr(P.lam), P.lam_plane,
+                    self._ptr(P.g), n, sb, n_grid,
+                    self._ptr(cur), self._ptr(nxt), 1, 0, 0,
+                    ctypes.c_void_p(0), *extra, self.stream)
+            _cabi.check(rc, "sdp_policy_eval" + sfx)
             self.coll.all_gather_slabs(nxt[sb:sb + n].clone(), P.bounds, out=nxt)
             if rel_dp:
                 ref_ptr = ctypes.c_void_p(J_ref_hist.data_ptr() + 8 * k)

@@ -29,6 +29,7 @@ import numpy as np
 
 from . import tabulate as tb
 from .interp import MlinInterpolator
+from .risk import check_risk
 
 __all__ = ["DPSolver"]
 
@@ -218,8 +219,23 @@ class DPSolver(object):
             out += [a.tobytes() for a, _, _ in compact]
         return b"".join(out)
 
-    def _cached_tables(self, t_k):
-        return self._table_cache.get(self._cache_key(t_k)) if self.cache_tables else None
+    @staticmethod
+    def _serves_risk(T):
+        """the risk sweep takes layout CF with one row per lane and dense layout A"""
+        return (T.column and not T.pairs) or (not T.column and not T.tiled and not T.u_mask)
+
+    def _table_key(self, t_k, risk=False):
+        """cache key of the tables of a sweep; a risk sweep uses the expectation's tables when they
+        serve it (_serves_risk), else its own, kept beside them"""
+        key = self._cache_key(t_k)
+        if risk:
+            T = self._table_cache.get(key)
+            if T is None or not self._serves_risk(T):
+                key = key + ("risk",)
+        return key
+
+    def _cached_tables(self, t_k, risk=False):
+        return self._table_cache.get(self._table_key(t_k, risk)) if self.cache_tables else None
 
     def _tables_still_valid(self, T, t_k=None):
         """False when the callables no longer give what the cached tables `T` were built from
@@ -227,25 +243,30 @@ class DPSolver(object):
         fp = getattr(T, "probe_fingerprint", None)
         return fp is None or fp == self._probe_fingerprint(t_k)
 
-    def sweep_tables(self, t_k=None, reuse=None, validate=True):
+    def sweep_tables(self, t_k=None, reuse=None, validate=True, risk=False):
         """device tables for the current (sys, grids, control_steps[, t_k]); cached stationary
         tables are re-validated against the callables (`_probe_fingerprint`) unless the caller
-        does that itself while the GPU works (`_sweep_host`)"""
+        does that itself while the GPU works (`_sweep_host`).  `risk`: tables the risk sweep
+        takes (`_table_key`)"""
         if not self.cache_tables:
-            T = self.engine.build_sweep_tables(self, t_k, reuse=reuse)
+            T = self.engine.build_sweep_tables(self, t_k, reuse=reuse, for_risk=risk)
             self.last_tables = T
             return T
-        key = self._cache_key(t_k)
+        key = self._table_key(t_k, risk)
         T = self._table_cache.get(key)
         if T is not None and validate and not self._tables_still_valid(T, t_k):
             self.clear_tables()
+            key = self._table_key(t_k, risk)
             T = None
         if T is None:
-            T = self.engine.build_sweep_tables(self, t_k, reuse=reuse)
+            T = self.engine.build_sweep_tables(self, t_k, reuse=reuse, for_risk=key[-1] == "risk")
             if t_k is None:
-                # stationary tables are reused across sweeps / policy iterations
+                # stationary tables are reused across sweeps / policy iterations; a risk sweep's own
+                # tables are kept beside the expectation's (one entry of each kind)
                 T.probe_fingerprint = self._probe_fingerprint(t_k)
-                self._table_cache = {key: T}
+                own = key[-1] == "risk"
+                self._table_cache = {k: v for k, v in self._table_cache.items() if (k[-1] == "risk") != own}
+                self._table_cache[key] = T
         self.last_tables = T
         return T
 
@@ -254,16 +275,17 @@ class DPSolver(object):
             raise ValueError("host_results must be 'all' or 'root'")
         return self.host_results == "root" and self.engine.coll.world > 1
 
-    def _sweep_host(self, J_next, t_k=None, rel_dp=False, tables=None):
-        """one sweep with host arrays in/out. Returns (J_k, J_ref or None, pol_k, tables)"""
+    def _sweep_host(self, J_next, t_k=None, rel_dp=False, tables=None, risk=None):
+        """one sweep with host arrays in/out. Returns (J_k, J_ref or None, pol_k, tables).
+        `risk`: an SdpRisk"""
         import torch
         eng = self.engine
         state_dims = tuple(len(g) for g in self.state_grid)
         nb_control = len(self.sys.control)
         # cached tables are launched at once and checked against the callables WHILE the GPU
         # sweeps (the host would only wait); a stale cache costs one wasted sweep, then a rebuild
-        cached = tables is None and self._cached_tables(t_k) is not None
-        T = tables if tables is not None else self.sweep_tables(t_k, validate=False)
+        cached = tables is None and self._cached_tables(t_k, risk is not None) is not None
+        T = tables if tables is not None else self.sweep_tables(t_k, validate=False, risk=risk is not None)
         stale = []
 
         def check_cache():
@@ -279,10 +301,11 @@ class DPSolver(object):
             # 1/N of each over every rank's own PCIe link (hostshare.py)
             ref_flat = int(np.ravel_multi_index(self._state_ref_ind, state_dims)) if rel_dp else None
             got = eng.sweep_shared(hs, T, J_next, rel_ref_index=ref_flat,
-                                   want_results=not (root_only and not is_root), while_waiting=check_cache)
+                                   want_results=not (root_only and not is_root), while_waiting=check_cache,
+                                   risk=risk)
             if stale:
                 self.clear_tables()
-                return self._sweep_host(J_next, t_k, rel_dp)
+                return self._sweep_host(J_next, t_k, rel_dp, risk=risk)
             if got is not None:
                 if got[0] is None:
                     return None, None, None, T
@@ -301,29 +324,29 @@ class DPSolver(object):
             eng.upload_J(J_next, J_prev)
         if not rel_dp and eng.can_overlap_results(T):
             # large single-rank sweep: results stream to the host while later runs compute
-            J_k, pol_k = eng.sweep_to_host(T, J_prev, J_new, while_waiting=check_cache)
+            J_k, pol_k = eng.sweep_to_host(T, J_prev, J_new, while_waiting=check_cache, risk=risk)
             if stale:
                 self.clear_tables()
-                return self._sweep_host(J_next, t_k, rel_dp)
+                return self._sweep_host(J_next, t_k, rel_dp, risk=risk)
             return J_k.reshape(state_dims), None, pol_k.reshape(state_dims + (nb_control,)), T
         ref_out = None
         ref_flat = None
         if rel_dp:
             ref_flat = int(np.ravel_multi_index(self._state_ref_ind, state_dims))
             ref_out = torch.zeros(1, dtype=torch.float64, device=eng.device)
-        eng.sweep(T, J_prev, J_new, rel_ref_index=ref_flat, ref_out=ref_out)
+        eng.sweep(T, J_prev, J_new, rel_ref_index=ref_flat, ref_out=ref_out, risk=risk)
         argmin_full = eng.gather_argmin(T)
         if root_only and not is_root:
             check_cache()
             if stale:
                 self.clear_tables()
-                return self._sweep_host(J_next, t_k, rel_dp)
+                return self._sweep_host(J_next, t_k, rel_dp, risk=risk)
             return None, None, None, T           # results travel to rank 0's host only
         pol_dev = eng.policy_values(T, argmin_full)               # K3: indices -> control values
         outs = eng.to_host(J_new, pol_dev, *([ref_out] if rel_dp else []), while_waiting=check_cache)
         if stale:
             self.clear_tables()
-            return self._sweep_host(J_next, t_k, rel_dp)
+            return self._sweep_host(J_next, t_k, rel_dp, risk=risk)
         J_k = outs[0].reshape(state_dims)
         pol_k = outs[1].reshape(state_dims + (nb_control,))
         J_ref = float(outs[2][0]) if rel_dp else None
@@ -332,11 +355,12 @@ class DPSolver(object):
     # ------------------------------------------------------------------
     # solvers
     # ------------------------------------------------------------------
-    def value_iteration(self, J_next, rel_dp=False, report_time=True):
+    def value_iteration(self, J_next, rel_dp=False, report_time=True, risk=None):
         """solve one DP step on the entire state grid, given the cost-to-go
         array `J_next` on that grid.
 
         If rel_dp is True, J_next should be a (J_next, J_ref) tuple.
+        `risk`: None (the expectation) or a `MeanCVaR`, the risk measure of the backup.
 
         Returns (J_k, pol_k); J_k is a tuple (J_diff, J_ref) if `rel_dp`.
         (reference stodynprog.py:466-534)
@@ -356,10 +380,11 @@ class DPSolver(object):
                 # same check and message as interp_on_state (:413-415)
                 raise ValueError('array `A` should be of shape {:s}, not {:s}'.format(
                     str(state_dims), str(J_next.shape)))
+        c_risk = check_risk(risk, self.perturb_proba)
         if report_time:
             print('value iteration...', end='')
         t_k = None
-        J_k, J_ref, pol_k, _ = self._sweep_host(J_next, t_k, rel_dp)
+        J_k, J_ref, pol_k, _ = self._sweep_host(J_next, t_k, rel_dp, risk=c_risk)
         exec_time = (datetime.now() - t_start).total_seconds()
         if report_time:
             print('\rvalue iteration run in {:.2f} s'.format(exec_time))
@@ -367,16 +392,17 @@ class DPSolver(object):
             J_k = J_k, J_ref
         return J_k, pol_k
 
-    def bellman_recursion(self, t_fin, J_fin, t_ini=0, report_time=True):
+    def bellman_recursion(self, t_fin, J_fin, t_ini=0, report_time=True, risk=None):
         """Bellman backward recursion for finite-horizon problems, from `t_fin`
         down to `t_ini` (must be 0).  Supports time-dependent systems: the instant
-        `t_k` is passed first to every callable.
+        `t_k` is passed first to every callable.  `risk`: None or a `MeanCVaR`.
 
         Returns (J, pol) with a leading time axis.  (reference stodynprog.py:536-591)
         """
         t_start = datetime.now()
         state_dims = tuple(len(g) for g in self.state_grid)
         nb_control = len(self.sys.control)
+        c_risk = check_risk(risk, self.perturb_proba)
         print('time-dependent problem: {:s}'.format('no' if self.sys.stationnary else 'yes'))
         assert t_ini == 0  # t_ini > 0 not tested (reference :557)
         J = np.zeros((t_fin - t_ini,) + state_dims)
@@ -389,7 +415,7 @@ class DPSolver(object):
                 str(state_dims), str(J_fin.shape)))
         saved_mode, self.host_results = self.host_results, "all"   # J[k+1] feeds instant k on every rank
         try:
-            self._recursion(t_ini, t_fin, J_fin, J, pol)
+            self._recursion(t_ini, t_fin, J_fin, J, pol, c_risk)
         finally:
             self.host_results = saved_mode
         exec_time = (datetime.now() - t_start).total_seconds()
@@ -397,13 +423,13 @@ class DPSolver(object):
             print('\rvalue iteration run in {:.2f} s'.format(exec_time))
         return J, pol
 
-    def _recursion(self, t_ini, t_fin, J_fin, J, pol):
+    def _recursion(self, t_ini, t_fin, J_fin, J, pol, risk=None):
         # systems whose dynamics and admissible controls ignore the instant (checked, not
         # assumed): one table build, the cost of all instants tabulated up front, the sweeps
         # enqueued back to back (Engine.recursion_fast); anything else: instant by instant
         self.last_recursion = None
         if getattr(self, "recursion_mode", "auto") != "per_instant":
-            info = self.engine.recursion_fast(self, t_ini, t_fin, J_fin, J, pol)
+            info = self.engine.recursion_fast(self, t_ini, t_fin, J_fin, J, pol, risk=risk)
             if info is not None:
                 self.last_tables = info.pop("tables")
                 self.last_recursion = info
@@ -414,14 +440,15 @@ class DPSolver(object):
             k = t_k - t_ini
             J_next = J_fin if t_k == (t_fin - 1) else J[k + 1]
             # tables depend on t_k: rebuilt each step, device buffers recycled
-            tables = self.engine.build_sweep_tables(self, t_k, reuse=tables)
+            tables = self.engine.build_sweep_tables(self, t_k, reuse=tables, for_risk=risk is not None)
             self.last_tables = tables
-            J[k], _, pol[k], _ = self._sweep_host(J_next, t_k, False, tables=tables)
+            J[k], _, pol[k], _ = self._sweep_host(J_next, t_k, False, tables=tables, risk=risk)
 
     def eval_policy(self, pol, n_iter, rel_dp=False, J_zero=None,
-                    report_time=True, J_ref_full=False):
+                    report_time=True, J_ref_full=False, risk=None):
         """evaluate the policy `pol`: cost of each state after `n_iter` steps
-        (the policy-evaluation half of policy iteration).
+        (the policy-evaluation half of policy iteration).  `risk`: None (the
+        expectation) or a `MeanCVaR`, the risk measure of every backup.
 
         With rel_dp the relative DP algorithm is used: after each step the cost
         of the reference state is recorded and subtracted.
@@ -439,6 +466,7 @@ class DPSolver(object):
         ref_ind = self._state_ref_ind
         nb_control = len(self.sys.control)
         assert pol.shape == state_dims + (nb_control,)
+        c_risk = check_risk(risk, self.perturb_proba)
 
         eng = self.engine
         P = eng.build_policy_tables(self, pol)
@@ -449,7 +477,7 @@ class DPSolver(object):
         hist = torch.zeros(max(n_iter, 1), dtype=torch.float64, device=eng.device)
         ref_flat = int(np.ravel_multi_index(ref_ind, state_dims))
         print('\rpolicy evaluation: iter. {:d}/{:d}'.format(max(n_iter - 1, 0), n_iter), end='')
-        J_dev = eng.policy_eval(P, J_a, J_b, n_iter, rel_dp, ref_flat, hist)
+        J_dev = eng.policy_eval(P, J_a, J_b, n_iter, rel_dp, ref_flat, hist, risk=c_risk)
         outs = eng.to_host(J_dev, hist)
         J_pol = outs[0].reshape(state_dims)
         J_ref = outs[1][:n_iter] if rel_dp else None
@@ -463,29 +491,30 @@ class DPSolver(object):
             return J_pol, J_ref
         return J_pol
 
-    def policy_iteration(self, pol_init, n_val, n_pol=1, rel_dp=False):
+    def policy_iteration(self, pol_init, n_val, n_pol=1, rel_dp=False, risk=None):
         """policy iteration: evaluate `pol_init` with `n_val` fixed-policy
         backups, then `n_pol` times (improve with one value iteration, evaluate).
+        `risk`: None or a `MeanCVaR`, used by both halves.
 
         Returns (J_pol, pol); J_pol is a tuple (J_diff, J_ref) if `rel_dp`.
         (reference stodynprog.py:777-812)
         """
         saved_mode, self.host_results = self.host_results, "all"   # every rank needs pol to evaluate it
         try:
-            return self._policy_iteration(pol_init, n_val, n_pol, rel_dp)
+            return self._policy_iteration(pol_init, n_val, n_pol, rel_dp, risk)
         finally:
             self.host_results = saved_mode
 
-    def _policy_iteration(self, pol_init, n_val, n_pol, rel_dp):
+    def _policy_iteration(self, pol_init, n_val, n_pol, rel_dp, risk=None):
         pol = pol_init
-        J_pol = self.eval_policy(pol, n_val, rel_dp)
+        J_pol = self.eval_policy(pol, n_val, rel_dp, risk=risk)
         if rel_dp:
             J_diff, J_ref = J_pol
             print('ref policy cost: {:g}'.format(J_ref))
         for k in range(n_pol):
             print('policy iteration {:d}/{:d}'.format(k + 1, n_pol))
-            _, pol = self.value_iteration(J_pol, rel_dp=rel_dp)
-            J_pol = self.eval_policy(pol, n_val, rel_dp)
+            _, pol = self.value_iteration(J_pol, rel_dp=rel_dp, risk=risk)
+            J_pol = self.eval_policy(pol, n_val, rel_dp, risk=risk)
             if rel_dp:
                 J_ref = J_pol[1]
                 print('ref policy cost: {:g}'.format(J_ref))
@@ -495,16 +524,18 @@ class DPSolver(object):
     # new: device-resident value iteration driven by the sup-norm residual
     # ------------------------------------------------------------------
     def solve_value_iteration(self, J_zero=None, max_iter=100, tol=None, rel_dp=False,
-                              check_every=1):
+                              check_every=1, risk=None):
         """Repeated Bellman sweeps with J kept on the device; stops after
         `max_iter` sweeps or when max|J_k - J_{k+1}| <= tol (all-reduced over the
         ranks).  Not in the reference (users write this loop by hand,
-        doc/example_inventory.py:98-110).  Returns (J, pol, info)."""
+        doc/example_inventory.py:98-110).  `risk`: None (the expectation) or a
+        `MeanCVaR`.  Returns (J, pol, info)."""
         import torch
         eng = self.engine
         state_dims = tuple(len(g) for g in self.state_grid)
         nb_control = len(self.sys.control)
-        T = self.sweep_tables(None)
+        c_risk = check_risk(risk, self.perturb_proba)
+        T = self.sweep_tables(None, risk=c_risk is not None)
         J0 = np.zeros(state_dims) if J_zero is None else np.asarray(J_zero, dtype=float)
         n_grid = int(np.prod(state_dims))
         J_prev, J_new = eng.J_pair(n_grid)
@@ -527,7 +558,7 @@ class DPSolver(object):
             # first kernel; relative DP and the residual read J right away and wait themselves)
             eng.sweep(T, J_prev, J_new, rel_ref_index=ref_flat, ref_out=ref_out,
                       resid_out=resid if tol is not None else None, defer_wait=k + 1 < max_iter,
-                      want_argmin=(tol is not None or k + 1 == max_iter))
+                      want_argmin=(tol is not None or k + 1 == max_iter), risk=c_risk)
             J_prev, J_new = J_new, J_prev
             n_done += 1
             if tol is not None and (k + 1) % check_every == 0:

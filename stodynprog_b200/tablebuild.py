@@ -559,11 +559,14 @@ class BuildPlan(object):
       solver.tabulate       : "auto" | "per_state" | "batched"
       solver.column_hoist, solver.column_pairs, solver.slab_axis, solver.slab_balance,
       solver.host_threads
-    `forced_axis` = "rows": the cut by columns chosen by "auto" was refused by the built tables."""
+    `forced_axis` = "rows": the cut by columns chosen by "auto" was refused by the built tables.
+    `for_risk`: tables for the risk sweep (sdp_sweep_risk_partials), which takes layout CF with one
+    row per lane or dense layout A: where CF does not apply, the tables are dense layout A."""
 
-    def __init__(self, eng, solver, t_k, forced_axis=None):
+    def __init__(self, eng, solver, t_k, forced_axis=None, for_risk=False):
         self.t_start = time.perf_counter()
         self.eng, self.solver, self.t_k = eng, solver, t_k
+        self.for_risk = bool(for_risk)
         self.sys = sys = solver.sys
         self.state_grid = state_grid = [np.asarray(g, dtype=float) for g in solver.state_grid]
         self.d = d = len(state_grid)
@@ -621,7 +624,7 @@ class BuildPlan(object):
         pair_mode = getattr(solver, "column_pairs", "auto")
         if pair_mode not in ("auto", "on", "off"):
             raise ValueError("column_pairs must be 'auto', 'on' or 'off'")
-        self.pairs = bool(self.col_candidate
+        self.pairs = bool(self.col_candidate and not self.for_risk
                           and (pair_mode == "on" or (pair_mode == "auto" and COLUMN_PAIRS_DEFAULT))
                           and 8 * _cabi.column_pitch(n_rows0, W, pairs=True) <= _cabi.COLUMN_MAX_SMEM_BYTES)
         # several ranks: slabs of whole rows of axis 0 ("rows"), or - layout CF only - whole
@@ -854,6 +857,8 @@ class ShardBuild(object):
                              "that does not depend on axis 0, and order[0]*(W|1)*8 bytes of "
                              "shared memory")
         self.column = column
+        if plan.for_risk and not column:
+            self.tiled, self.u_mask = False, 0       # the risk sweep's other layout: dense A
 
     def positions(self, col):
         """(n_eff, U_eff, host_eff, flat_eff, valid, bands): the shard's states in table order -
@@ -1066,6 +1071,9 @@ class ShardBuild(object):
         batched = mode in ("auto", "batched")
         L = None
         while L is None:
+            if plan.for_risk and not (column and u_mask == 1):
+                self.tiled = T.tiled = False         # (CF refused: dense layout A for the risk sweep)
+                u_mask, column = 0, False
             try:
                 col = column and u_mask == 1
                 built = self.tabulate(g_per_w, batched, u_mask, col)
